@@ -21,7 +21,7 @@ extern "C" {
 
 #define OTSLAM_OK 0
 #define OTSLAM_ERR_INVALID (-1)   /* bad argument */
-#define OTSLAM_ERR_FORMAT (-2)    /* "[ScalableTSDFVolume::Integrate] Unsupported image format." */
+#define OTSLAM_ERR_FORMAT (-2)    /* "[ScalableTSDFVolume::Integrate] Unsupported image format."; malformed checkpoint file */
 #define OTSLAM_ERR_CUDA (-3)      /* CUDA runtime / no device */
 #define OTSLAM_ERR_NOMEM (-4)     /* device memory exhausted */
 #define OTSLAM_ERR_OVERFLOW (-5)  /* per-voxel frame-count limit (65535) or key range exceeded */
@@ -136,6 +136,28 @@ int otslam_volume_num_blocks(otslam_volume* v, int64_t* n_blocks);
 int otslam_volume_export_blocks(otslam_volume* v, int32_t* keys, float* tsdf, float* weight, float* color);
 /* sum of all voxel weights (== number of voxel updates since reset) and voxels with weight > 0 */
 int otslam_volume_stats(otslam_volume* v, int64_t* n_blocks, uint64_t* weight_sum, uint64_t* n_observed);
+
+/* ---- checkpoints (file format version 1, DESIGN.md §4): a volume's voxel records written verbatim, so that a loaded
+ *      volume continues integrating bit for bit as if it had never been saved.
+ * save writes the blocks this volume is responsible for: all blocks of a plain volume; the OWNED blocks of a slab rank
+ * (halo-imported pieces and halo = 1 neighbour blocks are left out, so the part files of N ranks partition the volume);
+ * the selected object of an arena, with the object's key offset removed.  The file is written under a temporary name,
+ * synced and renamed.
+ * load adds a file's blocks to a volume (which may hold blocks already): voxel_length / sdf_trunc / color_type must equal
+ * the volume's bit for bit; a slab rank keeps what its spec keeps (owned blocks, plus the +1 neighbours when halo = 1), so
+ * loading every part file of N ranks into M ranks reshards the volume; an arena loads into the selected object
+ * (|kx| >= 2^17: OTSLAM_ERR_OVERFLOW).  The frame count becomes max(volume's, file's).  Every check (header, size, key order
+ * and duplicates, keys already present, checksums, record validity) runs before anything is inserted: on any error the
+ * volume is unchanged.  Malformed files: OTSLAM_ERR_FORMAT.  *n_loaded (nullable) = blocks added. */
+int otslam_volume_save(otslam_volume* v, const char* path);
+int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded);
+/* header of a checkpoint, validated on the host (no GPU needed); outputs nullable */
+int otslam_checkpoint_info(const char* path, double* voxel_length, double* sdf_trunc, int32_t* color_type, int64_t* frames,
+                           int64_t* n_blocks);
+/* this thread's last save / load: [0] device ms of its kernels (save: gather + checksum; load: key filter + verify +
+ * insert), [1] device ms of its host<->device copies, [2] ms spent in file reads / writes / fsync (summed over the I/O
+ * thread's calls), [3] wall ms of the whole call */
+int otslam_checkpoint_profile(double out[4]);
 
 /* ---- halo exchange for slab.halo == 0 (the path's only inter-GPU exchange of voxel data besides the final
  *      gather): export the low-side boundary pieces (256 voxel records of 16 bytes each, opaque) of every

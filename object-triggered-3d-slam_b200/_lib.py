@@ -55,7 +55,11 @@ _SIGS = {
     "otslam_volume_num_blocks": (_i, [_vp, C.POINTER(_i64)]),
     "otslam_volume_export_blocks": (_i, [_vp, _vp, _vp, _vp, _vp]),
     "otslam_volume_stats": (_i, [_vp, C.POINTER(_i64), C.POINTER(_u64), C.POINTER(_u64)]),
-    "otslam_volume_halo_export": (_i, [_vp, C.POINTER(_i64), _vp, _vp, _vp]),
+    "otslam_volume_save": (_i, [_vp, C.c_char_p]),
+    "otslam_volume_load": (_i, [_vp, C.c_char_p, C.POINTER(_i64)]),
+    "otslam_checkpoint_info": (_i, [C.c_char_p, C.POINTER(_d), C.POINTER(_d), C.POINTER(C.c_int32), C.POINTER(_i64), C.POINTER(_i64)]),
+    "otslam_checkpoint_profile": (_i, [_vp]),
+    "otslam_volume_halo_export":(_i, [_vp, C.POINTER(_i64), _vp, _vp, _vp]),
     "otslam_volume_halo_import": (_i, [_vp, _i64, _vp, _vp]),
     "otslam_volume_halo_pack": (_i, [_vp, C.POINTER(_i64), _vp]),
     "otslam_volume_halo_fetch": (_i, [_vp, _vp, _vp]),

@@ -179,12 +179,6 @@ __global__ void __launch_bounds__(256) tri_area_kernel(const double* __restrict_
 // ---- sequential-order accumulation (surface area, area CDF, outlier-filter statistics): ordered_sum.cu
 int device_ordered_sum(double* d_x, int64_t n, int mode, const double* d_div, double mean, double* d_out, cudaStream_t s);
 
-__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
-    x += 0x9E3779B97F4A7C15ull;
-    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
-    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
-    return x ^ (x >> 31);
-}
 __device__ __forceinline__ double u01(uint64_t seed, uint64_t ctr) {
     return __dmul_rn((double)(splitmix64(seed * 0xD1342543DE82EF95ull + ctr) >> 11), 1.0 / 9007199254740992.0);
 }

@@ -77,6 +77,13 @@ __host__ __device__ inline uint32_t hash_key(uint64_t k) {
     k ^= k >> 33;
     return (uint32_t)k;
 }
+// splitmix64 finaliser: the mesh sampler's counter-based RNG (cloud.cu) and the checkpoint checksums (checkpoint.cu)
+__host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
+    x += 0x9E3779B97F4A7C15ull;
+    x = (x ^ (x >> 30)) * 0xBF58476D1CE4E5B9ull;
+    x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
+    return x ^ (x >> 31);
+}
 
 // ---- multi-object arenas (config 3: multi_reconstruct_rgbd_filter.py, several objects, each "its own volume"): the
 // objects share ONE block hash / pool / per-batch work list, so that one integration launch covers the union of their

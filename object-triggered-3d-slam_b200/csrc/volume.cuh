@@ -124,6 +124,9 @@ int volume_sorted_blocks_device(otslam_volume* v, const uint64_t** d_keys, const
 int volume_selected_blocks_device(otslam_volume* v, const uint64_t** d_keys, const int32_t** d_slots, int* n, int* x_off);
 // the same downloaded to the host (export_blocks)
 int volume_sorted_blocks(otslam_volume* v, std::vector<uint64_t>& keys, std::vector<int32_t>& slots);
+// volume.cu, used by checkpoint.cu: 4x larger block hash (both streams drained first); pool chunks for blocks_needed slots
+int grow_hash(otslam_volume* v);
+int ensure_pool(otslam_volume* v, int64_t blocks_needed);
 // knn.cu: stable LSD radix sort of (u64 key, i32 value) pairs by the low `bits` bits; result in (kb, vb), (ka, va) clobbered
 int device_sort_pairs(uint64_t* ka, int32_t* va, uint64_t* kb, int32_t* vb, int64_t n, int bits, cudaStream_t s);
 }

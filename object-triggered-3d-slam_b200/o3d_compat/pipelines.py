@@ -1,11 +1,12 @@
 """o3d.pipelines.integration: ScalableTSDFVolume on the GPU (reconstruct_rgbd.py:79-83,107,112)."""
 import enum
+import os
 import types
 
 import numpy as np
 
 from .. import _lib
-from ..volume import TSDFVolume
+from ..volume import TSDFVolume, checkpoint_info
 from . import geometry
 
 _FMT = "[ScalableTSDFVolume::Integrate] Unsupported image format."
@@ -84,6 +85,22 @@ class ScalableTSDFVolume:
             raise RuntimeError(_FMT)
         self._vol.integrate_batch(depths, colors if self.color_type == TSDFVolumeColorType.RGB8 else None,
                                   intrinsic.fxfycxcy(), extrinsics, depth_scale, depth_trunc)
+
+    # -- checkpoint extension (the names of Open3D's tensor VoxelBlockGrid; the file format is this library's own) ----
+    def save(self, file_name):
+        """Write the volume's voxel state to `file_name`; ScalableTSDFVolume.load continues from it bit for bit."""
+        self._vol.save(file_name)
+
+    @staticmethod
+    def load(file_name, device=0):
+        """A new volume holding a checkpoint (or, given a list, the part files of a sharded volume), with the voxel
+        parameters stored in the file."""
+        first = file_name if isinstance(file_name, (str, bytes, os.PathLike)) else file_name[0]
+        info = checkpoint_info(first)
+        color = TSDFVolumeColorType.RGB8 if info["color"] else TSDFVolumeColorType.NoColor
+        vol = ScalableTSDFVolume(info["voxel_length"], info["sdf_trunc"], color, device=device)
+        vol._vol.load(file_name)
+        return vol
 
 
 integration = types.SimpleNamespace(ScalableTSDFVolume=ScalableTSDFVolume, TSDFVolumeColorType=TSDFVolumeColorType)

@@ -4,11 +4,29 @@ Mirrors o3d.pipelines.integration.ScalableTSDFVolume as used at
 /root/reference/3d_model/reconstruct_rgbd.py:79-83,107,112.
 """
 import ctypes as C
+import os
 import weakref
 
 import numpy as np
 
 from . import _lib
+
+
+def checkpoint_info(path):
+    """Header of a checkpoint written by TSDFVolume.save, validated on the host (no GPU needed)."""
+    vl, tr = C.c_double(0), C.c_double(0)
+    ct = C.c_int32(0)
+    frames, nb = C.c_int64(0), C.c_int64(0)
+    _lib.check(_lib.lib.otslam_checkpoint_info(os.fsencode(path), C.byref(vl), C.byref(tr), C.byref(ct), C.byref(frames), C.byref(nb)))
+    return {"voxel_length": vl.value, "sdf_trunc": tr.value, "color": ct.value == _lib.COLOR_RGB8, "frames": frames.value,
+            "n_blocks": nb.value}
+
+
+def checkpoint_profile():
+    """Timings of this thread's last save / load: device ms of kernels and of copies, ms in file I/O, wall ms."""
+    out = np.zeros(4, np.float64)
+    _lib.check(_lib.lib.otslam_checkpoint_profile(_lib.ptr(out)))
+    return {"kernel_ms": float(out[0]), "copy_ms": float(out[1]), "file_ms": float(out[2]), "wall_ms": float(out[3])}
 
 
 class TSDFVolume:
@@ -187,6 +205,23 @@ class TSDFVolume:
         nb, ws, no = C.c_int64(0), C.c_uint64(0), C.c_uint64(0)
         _lib.check(_lib.lib.otslam_volume_stats(self._h, C.byref(nb), C.byref(ws), C.byref(no)))
         return {"n_blocks": nb.value, "weight_sum": ws.value, "n_observed": no.value}
+
+    # ---- checkpoints (otslam_volume_save / _load; format in DESIGN.md §4) ---------------------------------------------
+    def save(self, path):
+        """Write this volume's blocks to `path` (a slab rank: its owned blocks; an arena: the selected object)."""
+        _lib.check(_lib.lib.otslam_volume_save(self._h, os.fsencode(path)))
+
+    def load(self, paths):
+        """Add the blocks of one checkpoint file or of several part files (e.g. every rank's part of a sharded volume);
+        a slab rank keeps the blocks its spec keeps.  Each file is checked completely before any of its blocks is
+        inserted: a bad file raises and leaves the volume as it was.  Returns the number of blocks added."""
+        self._detach_resident_mesh()
+        total = 0
+        for p in [paths] if isinstance(paths, (str, bytes, os.PathLike)) else paths:
+            n = C.c_int64(0)
+            _lib.check(_lib.lib.otslam_volume_load(self._h, os.fsencode(p), C.byref(n)))
+            total += n.value
+        return total
 
     def halo_export(self):
         """(keys [n,4] i32 = block key + piece kind, dest rank [n] i32, pieces [n,4096] u8) for the slab halo exchange."""
