@@ -197,6 +197,20 @@ int otslam_volume_points_copy(otslam_volume* v, double* points, double* colors, 
  * TSDF at every point of the last extraction (Open3D GetNormalAt / GetTSDFAt); normals [n][3], host or device */
 int otslam_volume_points_normals(otslam_volume* v, double* normals);
 
+/* ---- ray casting: render the volume from n camera poses (the ray-cast half of a KinectFusion-style system; interface
+ *      after Open3D's tensor VoxelBlockGrid.ray_cast, arithmetic in DESIGN.md §4 "Ray casting").  Pixel (u, v) of view i
+ *      follows the ray that integration projects onto (u, v), from the camera centre of inverse4(extrinsics[i]); depth is
+ *      the camera z of the first front-face (+ -> -) zero crossing of two consecutive observed samples with
+ *      depth_min <= t < depth_max.  Outputs (each nullable, host or device pointer): depth [n][H][W] f32 metres, vertex and
+ *      normal [n][H][W][3] f32 world (normal = GetNormalAt at the vertex, as extract_point_cloud's), color [n][H][W][3] u8
+ *      (trilinear over the observed voxels, renormalised; 0 for a NoColor volume); 0 where a ray hits nothing.
+ *      *n_hits (nullable) = pixels with a hit.  An arena renders its selected object only; slab-sharded volumes are refused
+ *      (load the part files into one volume).  The volume is read only: no result, block list or epoch changes.  Bad
+ *      arguments give OTSLAM_ERR_INVALID before any CUDA call.  otslam_last_op_device_ms() = device ms of the render. */
+int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, const double intr[4],
+                          const double* extrinsics, double depth_min, double depth_max, float* depth, float* vertex,
+                          float* normal, uint8_t* color, int64_t* n_hits);
+
 /* ---- stateless image / cloud operators.  Every pointer argument may be a HOST pointer or a DEVICE pointer of `device`
  *      (unified addressing; the copies inside become device-to-device): a caller that keeps its clouds in HBM between
  *      operators (otslam_b200/cloud.py: DeviceCloud) never crosses PCIe.  Device inputs must be complete (producer stream

@@ -102,6 +102,13 @@ class ScalableTSDFVolume:
         vol._vol.load(file_name)
         return vol
 
+    # -- ray-casting extension (named after Open3D's tensor VoxelBlockGrid.ray_cast) ---------------------------------------
+    def ray_cast(self, intrinsic, extrinsic, depth_min=0.1, depth_max=3.0):
+        """Render the volume from one camera (a PinholeCameraIntrinsic and a world->camera 4x4 extrinsic): a dict of
+        NumPy arrays depth [H,W] f32 metres, vertex / normal [H,W,3] f32 world, color [H,W,3] u8 (0 where nothing is hit).
+        depth_max defaults to the reference's depth_trunc of 3.0."""
+        return self._vol.ray_cast(intrinsic.fxfycxcy(), extrinsic, intrinsic.width, intrinsic.height, depth_min, depth_max)
+
 
 integration = types.SimpleNamespace(ScalableTSDFVolume=ScalableTSDFVolume, TSDFVolumeColorType=TSDFVolumeColorType)
 

@@ -133,8 +133,9 @@ def _checker(P, base, cell=0.08):
     return base.to(P.dtype) * shade[..., None]
 
 
-def render(prims, T_wo, intr=REF_INTRINSICS, device="cpu", max_range=5.0, floor=True):
-    """Ray-cast one frame. Returns (depth_u16 [H,W], rgb_u8 [H,W,3]) torch tensors on `device`."""
+def render(prims, T_wo, intr=REF_INTRINSICS, device="cpu", max_range=5.0, floor=True, depth_m=False):
+    """Ray-cast one frame. Returns (depth_u16 [H,W], rgb_u8 [H,W,3]) torch tensors on `device`; depth_m=True returns the
+    unrounded f64 depth in metres instead of the millimetre image (0 where nothing is hit)."""
     W, H, fx, fy, cx, cy = intr
     dt = torch.float64
     T = torch.as_tensor(T_wo, dtype=dt, device=device)
@@ -194,6 +195,8 @@ def render(prims, T_wo, intr=REF_INTRINSICS, device="cpu", max_range=5.0, floor=
     hit = torch.isfinite(best_t) & (best_t <= max_range)          # scanner_node.cpp:277-278
     P = O + best_t.nan_to_num(posinf=0.0)[..., None] * D
     rgb = torch.where(hit[..., None], _checker(P, best_c), torch.zeros_like(best_c))
+    if depth_m:
+        return torch.where(hit, best_t, torch.zeros_like(best_t)), rgb.round().clamp(0, 255).to(torch.uint8)
     depth = torch.where(hit, torch.round(best_t * 1000.0), torch.zeros_like(best_t))
     depth = depth.clamp(0, 65535).to(torch.int32).to(torch.uint16) if hasattr(torch, "uint16") else depth
     return depth, rgb.round().clamp(0, 255).to(torch.uint8)

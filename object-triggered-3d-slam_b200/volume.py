@@ -313,6 +313,52 @@ class TSDFVolume:
             _lib.check(_lib.lib.otslam_volume_points_normals(self._h, _lib.ptr(nrm)))
         return pts, cols, ek, nrm
 
+    # ---- ray casting (otslam_volume_raycast; arithmetic in DESIGN.md §4 "Ray casting") --------------------------------
+    RAY_CAST_ATTRIBUTES = ("depth", "color", "normal", "vertex")
+
+    def _ray_cast(self, intr, extrinsics, width, height, depth_min, depth_max, attributes, alloc):
+        attributes = tuple(attributes)
+        bad = [a for a in attributes if a not in self.RAY_CAST_ATTRIBUTES]
+        if bad:
+            raise ValueError(f"unknown ray-cast attributes {bad}; choose from {self.RAY_CAST_ATTRIBUTES}")
+        e = np.ascontiguousarray(extrinsics, np.float64)
+        single = e.shape == (4, 4)
+        e = e.reshape(-1, 16)
+        n, H, W = len(e), int(height), int(width)
+        shapes = {"depth": ((n, H, W), "f4"), "vertex": ((n, H, W, 3), "f4"), "normal": ((n, H, W, 3), "f4"),
+                  "color": ((n, H, W, 3), "u1")}
+        out = {a: alloc(*shapes[a]) for a in attributes}
+        hits = C.c_int64(0)
+        _lib.check(_lib.lib.otslam_volume_raycast(self._h, n, W, H, _lib.ptr(self._intr(intr)), _lib.ptr(e), float(depth_min),
+                                                  float(depth_max), _lib.ptr(out.get("depth")), _lib.ptr(out.get("vertex")),
+                                                  _lib.ptr(out.get("normal")), _lib.ptr(out.get("color")), C.byref(hits)))
+        if single:
+            out = {k: a[0] for k, a in out.items()}
+        return out, hits.value
+
+    def ray_cast(self, intr, extrinsics, width, height, depth_min=0.1, depth_max=3.0,
+                 attributes=("depth", "color", "normal", "vertex")):
+        """Render the volume from camera poses (after Open3D's VoxelBlockGrid.ray_cast).  intr = (fx, fy, cx, cy);
+        extrinsics = one world->camera 4x4 (unbatched results) or [n,4,4].  Returns a dict of NumPy arrays: depth [n,H,W]
+        f32 metres (camera z), vertex / normal [n,H,W,3] f32 world, color [n,H,W,3] u8; 0 where a ray hits nothing.  The
+        volume is only read."""
+        out, _ = self._ray_cast(intr, extrinsics, width, height, depth_min, depth_max, attributes,
+                                lambda shape, dt: np.empty(shape, dt))
+        return out
+
+    def ray_cast_tensors(self, intr, extrinsics, width, height, depth_min=0.1, depth_max=3.0,
+                         attributes=("depth", "color", "normal", "vertex")):
+        """ray_cast() with the maps rendered straight into torch CUDA tensors on this volume's GPU (no host copy).  The
+        tensors are complete when this returns."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        dts = {"f4": torch.float32, "u1": torch.uint8}
+        self.wait_stream(torch.cuda.current_stream(dev).cuda_stream)   # the outputs may reuse memory torch still uses
+        out, _ = self._ray_cast(intr, extrinsics, width, height, depth_min, depth_max, attributes,
+                                lambda shape, dt: torch.empty(shape, dtype=dts[dt], device=dev))
+        return out
+
+
 
 
 class ArenaView:
