@@ -211,6 +211,24 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
                           const double* extrinsics, double depth_min, double depth_max, float* depth, float* vertex,
                           float* normal, uint8_t* color, int64_t* n_hits);
 
+/* ---- frame-to-model tracking: refine the world->camera poses of n depth frames against the volume by projective
+ *      point-to-plane ICP on its ray-cast model (interface after Open3D's tensor SLAM Model.track_frame_to_model,
+ *      arithmetic in DESIGN.md §4 "Frame-to-model tracking").  Each frame is tracked independently against the volume as
+ *      it is: its model (vertex and normal maps over [depth_min, depth_max)) is rendered once at init_extrinsics[i], and
+ *      its pixels (depth = raw / depth_scale, valid when > 0 and < depth_max) are associated projectively into that view
+ *      and gated by depth_diff metres.  depth [n][H][W] u16 in `memory` (OTSLAM_MEM_HOST or OTSLAM_MEM_DEVICE, as
+ *      integrate_batch); init_extrinsics [n][16] on the host.  Host outputs (all but extrinsics_out nullable):
+ *      extrinsics_out [n][16] refined world->camera; status [n] 0 = converged, 1 = reached max_iterations (1..100),
+ *      2 = fewer than 64 inliers, 3 = degenerate system (2 and 3 keep the last pose); iterations [n]; fitness [n] =
+ *      inliers / valid pixels and inlier_rmse [n] = point-to-plane RMS over the inliers, both at the returned pose.  An
+ *      arena tracks against its selected object; slab-sharded volumes are refused (load the part files into one volume).
+ *      The volume is read only.  Bad arguments give OTSLAM_ERR_INVALID before any CUDA call.
+ *      otslam_last_op_device_ms() = device ms of the whole call. */
+int otslam_volume_track(otslam_volume* v, int n_frames, const uint16_t* depth, int width, int height, const double intr[4],
+                        const double* init_extrinsics, double depth_scale, double depth_min, double depth_max,
+                        double depth_diff, int max_iterations, double* extrinsics_out, int32_t* status,
+                        int32_t* iterations, double* fitness, double* inlier_rmse, int memory);
+
 /* ---- stateless image / cloud operators.  Every pointer argument may be a HOST pointer or a DEVICE pointer of `device`
  *      (unified addressing; the copies inside become device-to-device): a caller that keeps its clouds in HBM between
  *      operators (otslam_b200/cloud.py: DeviceCloud) never crosses PCIe.  Device inputs must be complete (producer stream

@@ -10,11 +10,12 @@
 //                   in registers, so the hash is probed only when a ray enters a new block (about every 16 samples).
 //                   Normal (FP64 GetNormalAt) and trilinear colour run at the hit only.
 // Host outputs are rendered into two bounded device staging buffers, chunk by chunk; the copy of chunk k (copy stream)
-// overlaps the render of chunk k + 1.  Device outputs are written in place.
+// overlaps the render of chunk k + 1.  Device outputs are written in place.  raycast_launch (raycast.cuh) is the one launch
+// path, shared with the frame-to-model tracker (track.cu), which renders its model maps with it.
 #include <cmath>
 #include <vector>
 
-#include "volume_lookup.cuh"
+#include "raycast.cuh"
 
 namespace otslam {
 
@@ -23,29 +24,6 @@ constexpr int kViewsPerChunk = 32;
 constexpr size_t kStagingBytes = 256ull << 20;  // per staging buffer (two of them) for host outputs
 constexpr int kTileW = 16, kTileH = 8;
 constexpr double kMaxWindowVoxels = 4194304.0;  // 2^22: depth_max * max|d_c| / vl, keeps one-voxel steps >= 2 ulp(t)
-
-struct RayView {
-    float R[9];      // rows 0..2, cols 0..2 of camera_pose = inverse4(extrinsic), cast to f32
-    float o[3];      // camera centre (column 3 of camera_pose), f32
-};
-
-struct RayArgs {
-    ExtractCtx c;
-    const RayView* views;   // [chunk]
-    int W, H;
-    float cx, cy, ifx, ify; // ifx = 1.0f / (float)fx, as the integration's multiplier table (SURVEY A.2)
-    float vl, ktr;          // (float)voxel_length, (float)(k * sdf_trunc)
-    float dmin, dmax;
-    int cap;                // iterations per ray (host: raycast_cap)
-    int arena;              // multi-object arena: a block whose true x lies outside [-2^17, 2^17) is absent
-    int color;              // volume keeps colour
-    double gap;             // 0.99 voxel (GetNormalAt)
-    float* depth;           // outputs of this chunk, [chunk][H][W](...) or null
-    float* vertex;
-    float* normal;
-    uint8_t* rgb;
-    unsigned long long* hits;
-};
 
 // slot of block (bx, by, bz) (true x), -1 if absent or outside the selected object's window
 __device__ __forceinline__ int block_slot(const RayArgs& a, int bx, int by, int bz) {
@@ -255,6 +233,58 @@ struct EventPair {
     ~EventPair() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
 };
 
+bool ray_view(const double* e, RayView* out) {
+    double pose[16];
+    if (!finite_all(e, 16) || !inverse4(e, pose)) return false;
+    for (int r = 0; r < 3; ++r) {
+        for (int c = 0; c < 3; ++c) out->R[3 * r + c] = (float)pose[4 * r + c];
+        out->o[r] = (float)pose[4 * r + 3];
+    }
+    return true;
+}
+
+int ray_args(const otslam_volume* v, int width, int height, const double intr[4], double depth_min, double depth_max,
+             const char* op, RayArgs* out) {
+    const std::string p(op);
+    if (!v) return set_error(OTSLAM_ERR_INVALID, p + ": null volume");
+    if (v->slab.n_ranks > 1)
+        return set_error(OTSLAM_ERR_INVALID, p + ": slab-sharded volumes are not ray cast; load every rank's part file into one "
+                                                 "volume (otslam_volume_load) and ray cast that");
+    if (v->n_objects > 0 && v->sel_obj < 0) return set_error(OTSLAM_ERR_INVALID, "multi-object arena: otslam_volume_select_object first");
+    RayArgs a{};
+    a.W = width; a.H = height;
+    a.cx = (float)intr[2]; a.cy = (float)intr[3];
+    a.ifx = 1.0f / (float)intr[0]; a.ify = 1.0f / (float)intr[1];
+    a.vl = (float)v->voxel_length;
+    a.ktr = (float)((double)kStepFactor * v->sdf_trunc);
+    a.dmin = (float)depth_min; a.dmax = (float)depth_max;
+    float max_len = 0.f;
+    for (int u : {0, width - 1})
+        for (int vv : {0, height - 1}) max_len = std::max(max_len, ray_len(u, vv, a.cx, a.cy, a.ifx, a.ify));
+    if (!(depth_max * max_len / v->voxel_length <= kMaxWindowVoxels))
+        return set_error(OTSLAM_ERR_INVALID, p + ": depth_max * max|d_c| / voxel_length exceeds 2^22");
+    a.cap = (int)raycast_cap(depth_min, depth_max, max_len, v->voxel_length);
+    a.arena = v->n_objects > 0;
+    a.color = v->color_type == OTSLAM_COLOR_RGB8;
+    a.gap = 0.99 * v->voxel_length;
+    a.c.keys = v->d_keys; a.c.vals = v->d_vals; a.c.cap_mask = v->cap - 1; a.c.chunks = v->d_chunks;
+    a.c.bkeys = nullptr; a.c.bslots = nullptr; a.c.n = 0; a.c.slab = v->slab;
+    a.c.vl = v->voxel_length; a.c.half = 0.5 * v->voxel_length; a.c.unit = v->unit_length;
+    a.c.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0;
+    *out = a;
+    return OTSLAM_OK;
+}
+
+int raycast_launch(RayArgs a, const RayView* d_views, int n_views, float* depth, float* vertex, float* normal, uint8_t* rgb,
+                   cudaStream_t s) {
+    a.views = d_views;
+    a.depth = depth; a.vertex = vertex; a.normal = normal; a.rgb = rgb;
+    const dim3 grid((unsigned)((a.W + kTileW - 1) / kTileW), (unsigned)((a.H + kTileH - 1) / kTileH), (unsigned)n_views);
+    raycast_kernel<<<grid, kTileW * kTileH, 0, s>>>(a);
+    OT_LAUNCHED();
+    return OTSLAM_OK;
+}
+
 }  // namespace otslam
 
 using namespace otslam;
@@ -277,40 +307,11 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
     const int64_t px = (int64_t)width * height;
     if (n_views > 0 && px > INT64_MAX / 12 / n_views) return set_error(OTSLAM_ERR_INVALID, "raycast: output size overflows int64");
     std::vector<RayView> views((size_t)n_views);
-    for (int i = 0; i < n_views; ++i) {
-        const double* e = extrinsics + 16 * (size_t)i;
-        double pose[16];
-        if (!finite_all(e, 16) || !inverse4(e, pose)) return set_error(OTSLAM_ERR_INVALID, "raycast: extrinsic is not finite or is singular");
-        for (int r = 0; r < 3; ++r) {
-            for (int c = 0; c < 3; ++c) views[i].R[3 * r + c] = (float)pose[4 * r + c];
-            views[i].o[r] = (float)pose[4 * r + 3];
-        }
-    }
-    if (!v) return set_error(OTSLAM_ERR_INVALID, "raycast: null volume");
-    if (v->slab.n_ranks > 1)
-        return set_error(OTSLAM_ERR_INVALID, "raycast: slab-sharded volumes are not ray cast; load every rank's part file into one "
-                                             "volume (otslam_volume_load) and ray cast that");
-    if (v->n_objects > 0 && v->sel_obj < 0) return set_error(OTSLAM_ERR_INVALID, "multi-object arena: otslam_volume_select_object first");
+    for (int i = 0; i < n_views; ++i)
+        if (!ray_view(extrinsics + 16 * (size_t)i, &views[i]))
+            return set_error(OTSLAM_ERR_INVALID, "raycast: extrinsic is not finite or is singular");
     RayArgs a{};
-    a.W = width; a.H = height;
-    a.cx = (float)intr[2]; a.cy = (float)intr[3];
-    a.ifx = 1.0f / (float)intr[0]; a.ify = 1.0f / (float)intr[1];
-    a.vl = (float)v->voxel_length;
-    a.ktr = (float)((double)kStepFactor * v->sdf_trunc);
-    a.dmin = (float)depth_min; a.dmax = (float)depth_max;
-    float max_len = 0.f;
-    for (int u : {0, width - 1})
-        for (int vv : {0, height - 1}) max_len = std::max(max_len, ray_len(u, vv, a.cx, a.cy, a.ifx, a.ify));
-    if (!(depth_max * max_len / v->voxel_length <= kMaxWindowVoxels))
-        return set_error(OTSLAM_ERR_INVALID, "raycast: depth_max * max|d_c| / voxel_length exceeds 2^22");
-    a.cap = (int)raycast_cap(depth_min, depth_max, max_len, v->voxel_length);
-    a.arena = v->n_objects > 0;
-    a.color = v->color_type == OTSLAM_COLOR_RGB8;
-    a.gap = 0.99 * v->voxel_length;
-    a.c.keys = v->d_keys; a.c.vals = v->d_vals; a.c.cap_mask = v->cap - 1; a.c.chunks = v->d_chunks;
-    a.c.bkeys = nullptr; a.c.bslots = nullptr; a.c.n = 0; a.c.slab = v->slab;
-    a.c.vl = v->voxel_length; a.c.half = 0.5 * v->voxel_length; a.c.unit = v->unit_length;
-    a.c.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0;
+    OT_TRY(ray_args(v, width, height, intr, depth_min, depth_max, "raycast", &a));
     if (n_views == 0) return OTSLAM_OK;
 
     OT_TRY(use_device(v->device));
@@ -359,11 +360,7 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
                 if (host[j]) { dst[j] = stage + off; off += elem[j] * (size_t)px * nv; }
                 else dst[j] = (uint8_t*)outs[j] + elem[j] * (size_t)px * first;
             }
-            a.views = d_views.p + first;
-            a.depth = (float*)dst[0]; a.vertex = (float*)dst[1]; a.normal = (float*)dst[2]; a.rgb = dst[3];
-            const dim3 grid((unsigned)((width + kTileW - 1) / kTileW), (unsigned)((height + kTileH - 1) / kTileH), (unsigned)nv);
-            raycast_kernel<<<grid, kTileW * kTileH, 0, s>>>(a);
-            OT_LAUNCHED();
+            OT_TRY(raycast_launch(a, d_views.p + first, nv, (float*)dst[0], (float*)dst[1], (float*)dst[2], dst[3], s));
             if (host_bytes_per_view) {
                 OT_CUDA(cudaEventRecord(rendered.e[buf], s));
                 OT_CUDA(cudaStreamWaitEvent(cs, rendered.e[buf], 0));

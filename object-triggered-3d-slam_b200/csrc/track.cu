@@ -1,0 +1,358 @@
+// track.cu -- frame-to-model camera tracking on sm_100a: projective point-to-plane ICP of raw u16 depth frames against
+// vertex and normal maps ray cast from the volume (the model for the interface is Open3D's tensor SLAM
+// Model.track_frame_to_model).  The arithmetic is DESIGN.md §4 "Frame-to-model tracking" and is restated on the CPU by
+// tests/models/track_model.cpp; the two agree bit for bit.  All FP64 arithmetic is explicit round-to-nearest, no FMA.
+//
+//   raycast_launch      (raycast.cu) the model: vertex and normal maps of each frame at its initial pose E0, once
+//   track_assoc_kernel  one thread per source pixel, a 16x8 pixel tile per CTA, one grid z slice per frame: back-project
+//                       with the current pose T, project into E0, gate, and form the 30 terms of the pixel; the CTA sums
+//                       its 128 pixels by a fixed pairwise tree and writes one partial per tile
+//   track_solve_kernel  one CTA per frame: sums the tile partials by a fixed pairwise tree (in place, in global memory),
+//                       then one thread solves the 6x6 system and updates the frame's pose and status
+// The iterations are queued with no host round trip; a converged or failed frame's later CTAs exit on its device flag.
+#include <cmath>
+#include <vector>
+
+#include "raycast.cuh"
+
+namespace otslam {
+
+constexpr int kTrackChunk = 32;                     // frames whose maps are rendered at once
+constexpr size_t kTrackMapBytes = 512ull << 20;     // bound of the chunk's vertex + normal maps
+constexpr int kTileW = 16, kTileH = 8, kTilePx = kTileW * kTileH;
+constexpr int kTerms = 30;                          // 21 JtJ (upper triangle, row-major), 6 Jtr, r^2, inliers, valid pixels
+constexpr int kSolveThreads = 256;
+constexpr double kMinInliers = 64.0;
+constexpr double kPivotRel = 1e-10;
+constexpr double kConverged = 1e-6;                 // max |xi_i| (radians, metres) of a converged step
+constexpr double kStalled = 1e-5;                   // ... or a step this small that is not smaller than the one before
+
+struct TrackFrame {
+    double T[16];        // current camera pose (camera -> world)
+    double E[16];        // its extrinsic, inverse4(T); the returned pose
+    double E0[16];       // initial extrinsic: the view of the model maps
+    double fitness, rmse;
+    double last_step;    // max |xi_i| of the previous step (infinity before the first)
+    int status, iters, active;
+};
+
+struct TrackArgs {
+    const uint16_t* depth;   // [chunk][H][W]
+    const float* vertex;     // [chunk][H][W][3] model maps at E0
+    const float* normal;
+    TrackFrame* frames;      // [chunk]
+    double* partials;        // [chunk][kTerms][P]
+    int W, H, tiles_x, n_tiles, P;
+    float scale;             // (float)depth_scale
+    double dmax, ddiff2;     // depth_max, depth_diff * depth_diff
+    double fx, fy, cx, cy;
+};
+
+__device__ __forceinline__ double dm(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ double da(double a, double b) { return __dadd_rn(a, b); }
+__device__ __forceinline__ double ds(double a, double b) { return __dsub_rn(a, b); }
+
+// the shared cofactor inverse (inverse4 in volume.cu), restated with explicit round-to-nearest operations
+__device__ bool inverse4_rn(const double* m, double* o) {
+    const double a00 = m[0], a01 = m[1], a02 = m[2], a03 = m[3], a10 = m[4], a11 = m[5], a12 = m[6], a13 = m[7],
+                 a20 = m[8], a21 = m[9], a22 = m[10], a23 = m[11], a30 = m[12], a31 = m[13], a32 = m[14], a33 = m[15];
+    const double s0 = ds(dm(a00, a11), dm(a01, a10)), s1 = ds(dm(a00, a12), dm(a02, a10)), s2 = ds(dm(a00, a13), dm(a03, a10)),
+                 s3 = ds(dm(a01, a12), dm(a02, a11)), s4 = ds(dm(a01, a13), dm(a03, a11)), s5 = ds(dm(a02, a13), dm(a03, a12)),
+                 c0 = ds(dm(a20, a31), dm(a21, a30)), c1 = ds(dm(a20, a32), dm(a22, a30)), c2 = ds(dm(a20, a33), dm(a23, a30)),
+                 c3 = ds(dm(a21, a32), dm(a22, a31)), c4 = ds(dm(a21, a33), dm(a23, a31)), c5 = ds(dm(a22, a33), dm(a23, a32));
+    const double det = da(ds(da(da(ds(dm(s0, c5), dm(s1, c4)), dm(s2, c3)), dm(s3, c2)), dm(s4, c1)), dm(s5, c0));
+    if (det == 0.0 || !isfinite(det)) return false;
+    const double id = __ddiv_rn(1.0, det);
+    o[0] = dm(da(ds(dm(a11, c5), dm(a12, c4)), dm(a13, c3)), id);
+    o[1] = dm(ds(ds(dm(a02, c4), dm(a01, c5)), dm(a03, c3)), id);
+    o[2] = dm(da(ds(dm(a31, s5), dm(a32, s4)), dm(a33, s3)), id);
+    o[3] = dm(ds(ds(dm(a22, s4), dm(a21, s5)), dm(a23, s3)), id);
+    o[4] = dm(ds(ds(dm(a12, c2), dm(a10, c5)), dm(a13, c1)), id);
+    o[5] = dm(da(ds(dm(a00, c5), dm(a02, c2)), dm(a03, c1)), id);
+    o[6] = dm(ds(ds(dm(a32, s2), dm(a30, s5)), dm(a33, s1)), id);
+    o[7] = dm(da(ds(dm(a20, s5), dm(a22, s2)), dm(a23, s1)), id);
+    o[8] = dm(da(ds(dm(a10, c4), dm(a11, c2)), dm(a13, c0)), id);
+    o[9] = dm(ds(ds(dm(a01, c2), dm(a00, c4)), dm(a03, c0)), id);
+    o[10] = dm(da(ds(dm(a30, s4), dm(a31, s2)), dm(a33, s0)), id);
+    o[11] = dm(ds(ds(dm(a21, s2), dm(a20, s4)), dm(a23, s0)), id);
+    o[12] = dm(ds(ds(dm(a11, c1), dm(a10, c3)), dm(a12, c0)), id);
+    o[13] = dm(da(ds(dm(a00, c3), dm(a01, c1)), dm(a02, c0)), id);
+    o[14] = dm(ds(ds(dm(a31, s1), dm(a30, s3)), dm(a32, s0)), id);
+    o[15] = dm(da(ds(dm(a20, s3), dm(a21, s1)), dm(a22, s0)), id);
+    return true;
+}
+
+// rows 0..2 of M p, in the integration's product order ((M0 x + M1 y) + M2 z) + M3
+__device__ __forceinline__ void affine(const double* M, const double p[3], double out[3]) {
+#pragma unroll
+    for (int r = 0; r < 3; ++r) out[r] = da(da(da(dm(M[4 * r], p[0]), dm(M[4 * r + 1], p[1])), dm(M[4 * r + 2], p[2])), M[4 * r + 3]);
+}
+
+// report = 0: one Gauss-Newton iteration's association (frames no longer active exit); report = 1: the final pass
+__global__ void __launch_bounds__(kTilePx) track_assoc_kernel(const TrackArgs a, int report) {
+    __shared__ double sm[kTerms][kTilePx];
+    const TrackFrame& f = a.frames[blockIdx.z];
+    if (!report && !f.active) return;
+    const int lane = threadIdx.x;
+    const int u = blockIdx.x * kTileW + (lane % kTileW), v = blockIdx.y * kTileH + (lane / kTileW);
+    double t[kTerms];
+#pragma unroll
+    for (int k = 0; k < kTerms; ++k) t[k] = 0.0;
+    if (u < a.W && v < a.H) {
+        const size_t px = (size_t)a.W * a.H;
+        const float d = __fdiv_rn((float)a.depth[blockIdx.z * px + (size_t)v * a.W + u], a.scale);
+        if (d > 0.f && (double)d < a.dmax) {
+            t[29] = 1.0;
+            const double z = (double)d;
+            const double pc[3] = {dm(__ddiv_rn(ds((double)u, a.cx), a.fx), z), dm(__ddiv_rn(ds((double)v, a.cy), a.fy), z), z};
+            double p[3], q[3];
+            affine(f.T, pc, p);
+            affine(f.E0, p, q);
+            if (q[2] > 0.0) {
+                const double uf = floor(da(da(__ddiv_rn(dm(a.fx, q[0]), q[2]), a.cx), 0.5));
+                const double vf = floor(da(da(__ddiv_rn(dm(a.fy, q[1]), q[2]), a.cy), 0.5));
+                if (uf >= 0.0 && uf < (double)a.W && vf >= 0.0 && vf < (double)a.H) {
+                    const size_t m = 3 * (blockIdx.z * px + (size_t)vf * a.W + (size_t)uf);
+                    const double N[3] = {(double)a.normal[m], (double)a.normal[m + 1], (double)a.normal[m + 2]};
+                    if (N[0] != 0.0 || N[1] != 0.0 || N[2] != 0.0) {
+                        const double e[3] = {ds(p[0], (double)a.vertex[m]), ds(p[1], (double)a.vertex[m + 1]),
+                                             ds(p[2], (double)a.vertex[m + 2])};
+                        if (da(da(dm(e[0], e[0]), dm(e[1], e[1])), dm(e[2], e[2])) <= a.ddiff2) {
+                            const double r = da(da(dm(N[0], e[0]), dm(N[1], e[1])), dm(N[2], e[2]));
+                            const double J[6] = {ds(dm(p[1], N[2]), dm(p[2], N[1])), ds(dm(p[2], N[0]), dm(p[0], N[2])),
+                                                 ds(dm(p[0], N[1]), dm(p[1], N[0])), N[0], N[1], N[2]};
+                            int k = 0;
+#pragma unroll
+                            for (int i = 0; i < 6; ++i)
+#pragma unroll
+                                for (int j = i; j < 6; ++j) t[k++] = dm(J[i], J[j]);
+#pragma unroll
+                            for (int i = 0; i < 6; ++i) t[21 + i] = dm(J[i], r);
+                            t[27] = dm(r, r);
+                            t[28] = 1.0;
+                        }
+                    }
+                }
+            }
+        }
+    }
+#pragma unroll
+    for (int k = 0; k < kTerms; ++k) sm[k][lane] = t[k];
+    // fixed pairwise tree: lane i += lane i + 64, then i + 32, ... (absent pixels hold 0)
+    for (int s = kTilePx / 2; s > 0; s >>= 1) {
+        __syncthreads();
+        for (int j = lane; j < kTerms * s; j += kTilePx) {
+            const int k = j / s, i = j - k * s;
+            sm[k][i] = da(sm[k][i], sm[k][i + s]);
+        }
+    }
+    __syncthreads();
+    if (lane < kTerms) a.partials[((size_t)blockIdx.z * kTerms + lane) * a.P + blockIdx.y * a.tiles_x + blockIdx.x] = sm[lane][0];
+}
+
+// Cholesky solve of A xi = -b (A from the 21 upper-triangle sums); false when a pivot is <= kPivotRel * max diag(A)
+__device__ bool solve6(const double* S, double xi[6]) {
+    double A[6][6], L[6][6], y[6];
+    int k = 0;
+    for (int i = 0; i < 6; ++i)
+        for (int j = i; j < 6; ++j) { A[i][j] = S[k]; A[j][i] = S[k]; ++k; }
+    double maxd = A[0][0];
+    for (int i = 1; i < 6; ++i)
+        if (A[i][i] > maxd) maxd = A[i][i];
+    const double thr = dm(kPivotRel, maxd);
+    for (int j = 0; j < 6; ++j) {
+        double s = A[j][j];
+        for (int c = 0; c < j; ++c) s = ds(s, dm(L[j][c], L[j][c]));
+        if (!(s > thr)) return false;
+        L[j][j] = __dsqrt_rn(s);
+        for (int i = j + 1; i < 6; ++i) {
+            double w = A[i][j];
+            for (int c = 0; c < j; ++c) w = ds(w, dm(L[i][c], L[j][c]));
+            L[i][j] = __ddiv_rn(w, L[j][j]);
+        }
+    }
+    for (int i = 0; i < 6; ++i) {
+        double w = S[21 + i];
+        for (int c = 0; c < i; ++c) w = ds(w, dm(L[i][c], y[c]));
+        y[i] = __ddiv_rn(w, L[i][i]);
+    }
+    for (int i = 5; i >= 0; --i) {
+        double w = y[i];
+        for (int c = i + 1; c < 6; ++c) w = ds(w, dm(L[c][i], xi[c]));
+        xi[i] = __ddiv_rn(w, L[i][i]);
+    }
+    for (int i = 0; i < 6; ++i) xi[i] = -xi[i];
+    return true;
+}
+
+__global__ void __launch_bounds__(kSolveThreads) track_solve_kernel(const TrackArgs a, int it, int max_it, int report) {
+    TrackFrame& f = a.frames[blockIdx.x];
+    if (!report && !f.active) return;
+    double* buf = a.partials + (size_t)blockIdx.x * kTerms * a.P;
+    // fixed pairwise tree over the tile partials padded to P = 2^k: i += i + P/2, then i + P/4, ...
+    for (int h = a.P / 2; h > 0; h >>= 1) {
+        for (int j = threadIdx.x; j < kTerms * h; j += kSolveThreads) {
+            const int k = j / h, i = j - k * h;
+            const double x = i < a.n_tiles ? buf[(size_t)k * a.P + i] : 0.0;
+            const double y = i + h < a.n_tiles ? buf[(size_t)k * a.P + i + h] : 0.0;
+            buf[(size_t)k * a.P + i] = da(x, y);
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x != 0) return;
+    double S[kTerms];
+    for (int k = 0; k < kTerms; ++k) S[k] = buf[(size_t)k * a.P];
+    if (report) {
+        f.fitness = S[29] > 0.0 ? __ddiv_rn(S[28], S[29]) : 0.0;
+        f.rmse = S[28] > 0.0 ? __dsqrt_rn(__ddiv_rn(S[27], S[28])) : 0.0;
+        return;
+    }
+    f.iters = it + 1;
+    if (S[28] < kMinInliers) { f.status = 2; f.active = 0; return; }
+    double xi[6];
+    if (!solve6(S, xi)) { f.status = 3; f.active = 0; return; }
+    // Cayley rotation: a = w / 2, dR = I + 2 / (1 + |a|^2) ([a]x + [a]x^2); dT = [dR | t]; T <- dT T; E = inverse4(T)
+    const double h[3] = {dm(0.5, xi[0]), dm(0.5, xi[1]), dm(0.5, xi[2])};
+    const double n2 = da(da(dm(h[0], h[0]), dm(h[1], h[1])), dm(h[2], h[2]));
+    const double c = __ddiv_rn(2.0, da(1.0, n2));
+    const double K[9] = {0.0, -h[2], h[1], h[2], 0.0, -h[0], -h[1], h[0], 0.0};
+    double D[16];
+    for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 3; ++j) {
+            double k2 = dm(h[i], h[j]);
+            if (i == j) k2 = ds(k2, n2);
+            D[4 * i + j] = da(i == j ? 1.0 : 0.0, dm(c, da(K[3 * i + j], k2)));
+        }
+        D[4 * i + 3] = xi[3 + i];
+    }
+    D[12] = 0.0; D[13] = 0.0; D[14] = 0.0; D[15] = 1.0;
+    double T[16], E[16];
+    for (int r = 0; r < 4; ++r)
+        for (int cc = 0; cc < 4; ++cc)
+            T[4 * r + cc] = da(da(da(dm(D[4 * r], f.T[cc]), dm(D[4 * r + 1], f.T[4 + cc])), dm(D[4 * r + 2], f.T[8 + cc])),
+                               dm(D[4 * r + 3], f.T[12 + cc]));
+    if (!inverse4_rn(T, E)) { f.status = 3; f.active = 0; return; }
+    for (int k = 0; k < 16; ++k) { f.T[k] = T[k]; f.E[k] = E[k]; }
+    double step = 0.0;
+    for (int k = 0; k < 6; ++k)
+        if (fabs(xi[k]) > step) step = fabs(xi[k]);
+    // A step that stops shrinking near the association's resolution is a 2-cycle of pixel associations flipping at
+    // depth edges (DESIGN §4): converged too.
+    const bool stalled = step <= kStalled && step >= f.last_step;
+    f.last_step = step;
+    if (step <= kConverged || stalled) { f.status = 0; f.active = 0; }
+    else if (it + 1 >= max_it) { f.status = 1; f.active = 0; }
+}
+
+static bool finite_all(const double* p, int n) {
+    for (int i = 0; i < n; ++i)
+        if (!std::isfinite(p[i])) return false;
+    return true;
+}
+
+}  // namespace otslam
+
+using namespace otslam;
+
+extern "C" {
+
+int otslam_volume_track(otslam_volume* v, int n_frames, const uint16_t* depth, int width, int height, const double intr[4],
+                        const double* init_extrinsics, double depth_scale, double depth_min, double depth_max, double depth_diff,
+                        int max_iterations, double* extrinsics_out, int32_t* status, int32_t* iterations, double* fitness,
+                        double* inlier_rmse, int memory) {
+    // ---- every argument is checked before any CUDA call
+    if (n_frames < 0) return set_error(OTSLAM_ERR_INVALID, "track: n_frames < 0");
+    if (width <= 0 || height <= 0) return set_error(OTSLAM_ERR_INVALID, "track: width and height must be > 0");
+    if (!intr) return set_error(OTSLAM_ERR_INVALID, "track: null intrinsics");
+    if (!finite_all(intr, 4) || !(intr[0] > 0.0) || !(intr[1] > 0.0))
+        return set_error(OTSLAM_ERR_INVALID, "track: fx and fy must be finite and > 0, cx and cy finite");
+    if (!std::isfinite(depth_min) || !std::isfinite(depth_max) || !(depth_min > 0.0) || !(depth_min < depth_max))
+        return set_error(OTSLAM_ERR_INVALID, "track: need finite 0 < depth_min < depth_max");
+    if (!std::isfinite(depth_scale) || !(depth_scale > 0.0)) return set_error(OTSLAM_ERR_INVALID, "track: depth_scale must be finite and > 0");
+    if (!std::isfinite(depth_diff) || !(depth_diff > 0.0)) return set_error(OTSLAM_ERR_INVALID, "track: depth_diff must be finite and > 0");
+    if (max_iterations < 1 || max_iterations > 100) return set_error(OTSLAM_ERR_INVALID, "track: max_iterations must be in 1..100");
+    if (memory != OTSLAM_MEM_HOST && memory != OTSLAM_MEM_DEVICE) return set_error(OTSLAM_ERR_INVALID, "track: bad memory kind");
+    if (n_frames > 0 && (!depth || !init_extrinsics || !extrinsics_out))
+        return set_error(OTSLAM_ERR_INVALID, "track: null depth, init_extrinsics or extrinsics_out");
+    const int64_t px = (int64_t)width * height;
+    std::vector<TrackFrame> frames((size_t)n_frames);
+    std::vector<RayView> views((size_t)n_frames);
+    for (int i = 0; i < n_frames; ++i) {
+        const double* e = init_extrinsics + 16 * (size_t)i;
+        TrackFrame& f = frames[i];
+        f = TrackFrame{};
+        if (!ray_view(e, &views[i]) || !inverse4(e, f.T))
+            return set_error(OTSLAM_ERR_INVALID, "track: initial extrinsic is not finite or is singular");
+        for (int k = 0; k < 16; ++k) f.E[k] = f.E0[k] = e[k];
+        f.last_step = INFINITY;
+        f.status = 1; f.active = 1;
+    }
+    RayArgs ra{};
+    OT_TRY(ray_args(v, width, height, intr, depth_min, depth_max, "track", &ra));
+    if (n_frames == 0) return OTSLAM_OK;
+
+    OT_TRY(use_device(v->device));
+    cudaStream_t s = v->stream;
+    const int chunk = (int)std::min<size_t>(std::min(kTrackChunk, n_frames), std::max<size_t>(1, kTrackMapBytes / (24 * (size_t)px)));
+    TrackArgs a{};
+    a.W = width; a.H = height;
+    a.tiles_x = (width + kTileW - 1) / kTileW;
+    a.n_tiles = a.tiles_x * ((height + kTileH - 1) / kTileH);
+    a.P = 1;
+    while (a.P < a.n_tiles) a.P *= 2;
+    a.scale = (float)depth_scale;
+    a.dmax = depth_max; a.ddiff2 = depth_diff * depth_diff;
+    a.fx = intr[0]; a.fy = intr[1]; a.cx = intr[2]; a.cy = intr[3];
+    DevBuf<RayView> d_views;
+    DevBuf<TrackFrame> d_frames;
+    DevBuf<float> d_maps;
+    DevBuf<double> d_partials;
+    DevBuf<uint16_t> d_depth;
+    DevBuf<unsigned long long> d_hits;
+    OT_CUDA(d_views.alloc((size_t)n_frames)); OT_CUDA(d_frames.alloc((size_t)n_frames)); OT_CUDA(d_hits.alloc(1));
+    OT_CUDA(d_maps.alloc(6 * (size_t)px * chunk));
+    OT_CUDA(d_partials.alloc((size_t)kTerms * a.P * chunk));
+    if (memory == OTSLAM_MEM_HOST) OT_CUDA(d_depth.alloc((size_t)px * chunk));
+    ra.hits = d_hits.p;
+    a.vertex = d_maps.p;
+    a.normal = d_maps.p + 3 * (size_t)px * chunk;
+    a.partials = d_partials.p;
+    {
+        OpTimer timer(s);
+        OT_CUDA(cudaMemcpyAsync(d_views.p, views.data(), sizeof(RayView) * views.size(), cudaMemcpyHostToDevice, s));
+        OT_CUDA(cudaMemcpyAsync(d_frames.p, frames.data(), sizeof(TrackFrame) * frames.size(), cudaMemcpyHostToDevice, s));
+        for (int first = 0; first < n_frames; first += chunk) {
+            const int nf = std::min(chunk, n_frames - first);
+            if (memory == OTSLAM_MEM_HOST) {
+                OT_CUDA(cudaMemcpyAsync(d_depth.p, depth + (size_t)px * first, 2 * (size_t)px * nf, cudaMemcpyHostToDevice, s));
+                a.depth = d_depth.p;
+            } else {
+                a.depth = depth + (size_t)px * first;
+            }
+            a.frames = d_frames.p + first;
+            OT_TRY(raycast_launch(ra, d_views.p + first, nf, nullptr, d_maps.p, d_maps.p + 3 * (size_t)px * chunk, nullptr, s));
+            const dim3 grid((unsigned)a.tiles_x, (unsigned)((height + kTileH - 1) / kTileH), (unsigned)nf);
+            for (int it = 0; it <= max_iterations; ++it) {
+                const int report = it == max_iterations;   // the last pass reports fitness and RMSE at the returned pose
+                track_assoc_kernel<<<grid, kTilePx, 0, s>>>(a, report);
+                OT_LAUNCHED();
+                track_solve_kernel<<<nf, kSolveThreads, 0, s>>>(a, it, max_iterations, report);
+                OT_LAUNCHED();
+            }
+        }
+        OT_CUDA(cudaMemcpyAsync(frames.data(), d_frames.p, sizeof(TrackFrame) * frames.size(), cudaMemcpyDeviceToHost, s));
+        timer.stop();
+    }
+    OT_CUDA(cudaStreamSynchronize(s));
+    for (int i = 0; i < n_frames; ++i) {
+        const TrackFrame& f = frames[i];
+        for (int k = 0; k < 16; ++k) extrinsics_out[16 * (size_t)i + k] = f.E[k];
+        if (status) status[i] = f.status;
+        if (iterations) iterations[i] = f.iters;
+        if (fitness) fitness[i] = f.fitness;
+        if (inlier_rmse) inlier_rmse[i] = f.rmse;
+    }
+    return OTSLAM_OK;
+}
+
+}  // extern "C"

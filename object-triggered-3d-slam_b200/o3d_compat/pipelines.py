@@ -109,6 +109,30 @@ class ScalableTSDFVolume:
         depth_max defaults to the reference's depth_trunc of 3.0."""
         return self._vol.ray_cast(intrinsic.fxfycxcy(), extrinsic, intrinsic.width, intrinsic.height, depth_min, depth_max)
 
+    # -- tracking extension (named after Open3D's tensor SLAM Model.track_frame_to_model) -------------------------------
+    def track_frame_to_model(self, image, intrinsic, extrinsic, depth_min=0.1, depth_max=3.0, depth_diff=0.07,
+                             max_iterations=20):
+        """Refine the pose of one frame (an RGBDImage with raw u16 depth; its depth scale is used) against the volume by
+        point-to-plane ICP on its ray-cast model, starting from `extrinsic` (world->camera 4x4).  Unlike Open3D, whose
+        result holds a camera-to-camera correction, OdometryResult.transformation IS the refined world->camera extrinsic:
+        what integrate() takes.  The volume is only read."""
+        if image._depth_raw is None or not image._depth_is_raw_u16:
+            raise RuntimeError("track_frame_to_model needs an RGBDImage made from raw u16 depth")
+        r = self._vol.track(image._depth_raw, intrinsic.fxfycxcy(), extrinsic, image._depth_scale, depth_min, depth_max,
+                            depth_diff, max_iterations)
+        return OdometryResult(r["extrinsic"], float(r["fitness"]), float(r["inlier_rmse"]), int(r["status"]) == 0)
+
+
+class OdometryResult:
+    """Result of ScalableTSDFVolume.track_frame_to_model: the refined world->camera extrinsic, fitness (inliers / valid
+    pixels), inlier_rmse (metres) and whether the iteration converged."""
+
+    def __init__(self, transformation, fitness, inlier_rmse, converged):
+        self.transformation, self.fitness, self.inlier_rmse, self.converged = transformation, fitness, inlier_rmse, converged
+
+    def __repr__(self):
+        return f"OdometryResult with fitness={self.fitness:e}, inlier_rmse={self.inlier_rmse:e}, converged={self.converged}"
+
 
 integration = types.SimpleNamespace(ScalableTSDFVolume=ScalableTSDFVolume, TSDFVolumeColorType=TSDFVolumeColorType)
 

@@ -358,6 +358,39 @@ class TSDFVolume:
                                 lambda shape, dt: torch.empty(shape, dtype=dts[dt], device=dev))
         return out
 
+    # ---- frame-to-model tracking (otslam_volume_track; DESIGN.md §4 "Frame-to-model tracking") ---------------------------
+    def track(self, depth, intr, init_extrinsics, depth_scale=1000.0, depth_min=0.1, depth_max=3.0, depth_diff=0.07,
+              max_iterations=20):
+        """Refine the world->camera poses of raw u16 depth frames against this volume by point-to-plane ICP on its
+        ray-cast model (after Open3D's tensor SLAM Model.track_frame_to_model).  depth: a NumPy array or a CUDA torch
+        tensor, [n,H,W] or [H,W]; intr = (fx, fy, cx, cy); init_extrinsics [n,4,4] or one 4x4.  Each frame is tracked
+        independently against the volume as it is; the volume is only read.  Returns a dict: extrinsic [n,4,4] (refined),
+        status [n] (0 converged, 1 reached max_iterations, 2 fewer than 64 inliers, 3 degenerate; 2 and 3 keep the last
+        pose), iterations [n], fitness [n] (inliers / valid pixels) and inlier_rmse [n] (metres); unbatched for one
+        [H,W] frame."""
+        on_dev = hasattr(depth, "is_cuda") and depth.is_cuda
+        if on_dev:
+            assert depth.is_contiguous() and depth.element_size() == 2
+        else:
+            depth = np.ascontiguousarray(depth, np.uint16)
+        single = depth.ndim == 2
+        if single:
+            depth = depth[None]
+        n, H, W = int(depth.shape[0]), int(depth.shape[1]), int(depth.shape[2])
+        e = np.ascontiguousarray(init_extrinsics, np.float64).reshape(n, 16)
+        out = {"extrinsic": np.empty((n, 4, 4)), "status": np.empty(n, np.int32), "iterations": np.empty(n, np.int32),
+               "fitness": np.empty(n), "inlier_rmse": np.empty(n)}
+        if on_dev:
+            self._after_torch_stream(depth)
+        _lib.check(_lib.lib.otslam_volume_track(
+            self._h, n, _lib.ptr(depth), W, H, _lib.ptr(self._intr(intr)), _lib.ptr(e), float(depth_scale), float(depth_min),
+            float(depth_max), float(depth_diff), int(max_iterations), _lib.ptr(out["extrinsic"]), _lib.ptr(out["status"]),
+            _lib.ptr(out["iterations"]), _lib.ptr(out["fitness"]), _lib.ptr(out["inlier_rmse"]),
+            _lib.MEM_DEVICE if on_dev else _lib.MEM_HOST))
+        if single:
+            out = {k: a[0] for k, a in out.items()}
+        return out
+
 
 
 
