@@ -190,7 +190,7 @@ int device_sort_pairs(uint64_t* ka_in, int32_t* va_in, uint64_t* kb_out, int32_t
         std::swap(ka, kb);
         std::swap(va, vb);
     }
-    if (ka != kb_out) {   // odd number of passes leaves the result in the input buffers
+    if (ka != kb_out) {   // an even number of passes leaves the result in the input buffers
         OT_CUDA(cudaMemcpyAsync(kb_out, ka, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
         OT_CUDA(cudaMemcpyAsync(vb_out, va, (size_t)n * 4, cudaMemcpyDeviceToDevice, s));
     }

@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 from scipy.spatial import cKDTree
 
+import cloud_ref
 from conftest import canon_mesh, lexorder
 from oracle import oracle
 
@@ -202,6 +203,10 @@ def test_point_cloud_distance_vs_ckdtree(mesh):
     pa, pb = o3d.geometry.PointCloud(a), o3d.geometry.PointCloud(b)
     d_ab = pa.compute_point_cloud_distance(pb)
     d_ba = pb.compute_point_cloud_distance(pa)
+    # exact FP64 in the (dx^2 + dy^2) + dz^2 order: bit-exact against the reference (brute force on a sample ties it down)
+    ref_ab, ref_ba = cloud_ref.nn_distance_large(a, b), cloud_ref.nn_distance_large(b, a)
+    assert (ref_ab[:2000] == cloud_ref.nn_distance(a[:2000], b)).all() and (ref_ba[:2000] == cloud_ref.nn_distance(b[:2000], a)).all()
+    assert (d_ab == ref_ab).all() and (d_ba == ref_ba).all()
     assert np.allclose(d_ab, cKDTree(b).query(a)[0], rtol=1e-12, atol=1e-15)
     assert np.allclose(d_ba, cKDTree(a).query(b)[0], rtol=1e-12, atol=1e-15)
     assert (pa.compute_point_cloud_distance(pa) == 0).all()
