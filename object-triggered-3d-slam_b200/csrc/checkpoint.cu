@@ -193,8 +193,7 @@ struct FilterArgs {
     const int32_t* keys;        // [n][3] as in the file
     int n, x_off, arena;
     SlabSpec slab;
-    const uint64_t* hkeys;
-    uint32_t cap_mask;
+    HashTable table;
     int* flag;
     uint64_t* packed;
     int* bad;
@@ -212,13 +211,7 @@ __global__ void __launch_bounds__(256) ckpt_filter_kernel(FilterArgs a) {
     const int sx = x + a.x_off;
     if (!slab_keeps(a.slab, sx, y, z)) return;
     const uint64_t k = pack_key(sx, y, z);
-    uint32_t h = hash_key(k) & a.cap_mask;
-    for (uint32_t probe = 0; probe <= a.cap_mask; ++probe) {
-        const uint64_t e = a.hkeys[h];
-        if (e == k) { atomicOr(a.bad, kBadPresent); break; }
-        if (e == kEmptyKey) break;
-        h = (h + 1) & a.cap_mask;
-    }
+    if (hash_find(a.table, k) >= 0) atomicOr(a.bad, kBadPresent);
     a.flag[i] = 1;
     a.packed[i] = k;
 }
@@ -259,20 +252,9 @@ __global__ void __launch_bounds__(256) ckpt_verify_kernel(uint4* const* chunks, 
 }
 
 // load: keys known to be absent and distinct; kept block j gets pool slot first_slot + j (its records are already there)
-__global__ void __launch_bounds__(256) ckpt_insert_kernel(const uint64_t* __restrict__ kept_keys, int m, int first_slot, uint64_t* keys,
-                                                          int32_t* vals, uint32_t cap_mask) {
+__global__ void __launch_bounds__(256) ckpt_insert_kernel(const uint64_t* __restrict__ kept_keys, int m, int first_slot, HashTable t) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= m) return;
-    const uint64_t k = kept_keys[j];
-    uint32_t h = hash_key(k) & cap_mask;
-    for (;;) {
-        if (atomicCAS(reinterpret_cast<unsigned long long*>(keys + h), (unsigned long long)kEmptyKey, (unsigned long long)k) ==
-            (unsigned long long)kEmptyKey) {
-            vals[h] = first_slot + j;
-            return;
-        }
-        h = (h + 1) & cap_mask;
-    }
+    if (j < m) hash_insert_absent(t, kept_keys[j], first_slot + j);
 }
 
 // =============================================================================================
@@ -472,7 +454,7 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
         OT_CUDA(cudaMemsetAsync(bad.p, 0, 4, s));
         FilterArgs fa;
         fa.keys = keys3.p; fa.n = n; fa.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0; fa.arena = v->n_objects > 0;
-        fa.slab = v->slab; fa.hkeys = v->d_keys; fa.cap_mask = v->cap - 1; fa.flag = flag.p; fa.packed = packed.p; fa.bad = bad.p;
+        fa.slab = v->slab; fa.table = volume_hash(v); fa.flag = flag.p; fa.packed = packed.p; fa.bad = bad.p;
         ckpt_filter_kernel<<<(n + 255) / 256, 256, 0, s>>>(fa);
         OT_LAUNCHED();
         OT_TRY(device_exclusive_scan(flag.p, pos.p, n, s));
@@ -560,15 +542,11 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
                 return rc;
             }
             // every check passed: insert
-            while ((uint64_t)((int64_t)base + m) * 2 > v->cap) {
-                OT_CUDA(cudaStreamSynchronize(v->pre_stream));
-                OT_CUDA(cudaStreamSynchronize(s));
-                OT_TRY(grow_hash(v));
-            }
+            OT_TRY(reserve_hash(v, (int64_t)base + m));
             cudaEvent_t ei[2];
             OT_CUDA(cudaEventCreate(&ei[0])); OT_CUDA(cudaEventCreate(&ei[1]));
             OT_CUDA(cudaEventRecord(ei[0], s));
-            ckpt_insert_kernel<<<(m + 255) / 256, 256, 0, s>>>(kept_keys.p, m, base, v->d_keys, v->d_vals, v->cap - 1);
+            ckpt_insert_kernel<<<(m + 255) / 256, 256, 0, s>>>(kept_keys.p, m, base, volume_hash(v));
             OT_LAUNCHED();
             OT_CUDA(cudaEventRecord(ei[1], s));
             const int pool = base + m;

@@ -53,12 +53,9 @@ __device__ __forceinline__ void load_neighbours(const ExtractCtx& c, uint64_t ke
     if (threadIdx.x < 8) {
         const int j = threadIdx.x;
         int kx, ky, kz;
-        unpack_key(key, kx, ky, kz);
+        unpack_key(key, kx, ky, kz);                               // stored x: the arena offset included
         int s = slot;
-        if (j) {
-            const int nx = kx + (j & 1), ny = ky + ((j >> 1) & 1), nz = kz + ((j >> 2) & 1);
-            s = key_in_range(nx, ny, nz) ? find_slot(c, pack_key(nx, ny, nz)) : -1;
-        }
+        if (j) s = block_slot(c, kx - c.x_off + (j & 1), ky + ((j >> 1) & 1), kz + ((j >> 2) & 1));
         nslot[j] = s;
     }
 }
@@ -529,7 +526,7 @@ static int make_ctx(otslam_volume* v, ExtractCtx& c) {
     int x_off = 0;
     OT_TRY(volume_selected_blocks_device(v, &dk, &ds, &n, &x_off));
     c.x_off = x_off;
-    c.keys = v->d_keys; c.vals = v->d_vals; c.cap_mask = v->cap - 1; c.chunks = v->d_chunks;
+    c.table = volume_hash(v); c.chunks = v->d_chunks;
     c.bkeys = dk; c.bslots = ds; c.n = n; c.slab = v->slab;
     c.vl = v->voxel_length; c.half = 0.5 * v->voxel_length; c.unit = v->unit_length;
     return OTSLAM_OK;

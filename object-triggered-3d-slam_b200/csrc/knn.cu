@@ -289,26 +289,16 @@ __global__ void __launch_bounds__(128) voxel_mean_kernel(const double* __restric
 
 // ---- k-NN grid hash: cell key -> segment id
 __global__ void __launch_bounds__(256) cell_hash_build_kernel(const uint64_t* __restrict__ sorted_keys, const int32_t* __restrict__ seg_start,
-                                                              int64_t n_seg, uint64_t* hkeys, int32_t* hvals, uint32_t cap_mask) {
+                                                              int64_t n_seg, HashTable t) {
     const int64_t m = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (m >= n_seg) return;
-    const uint64_t key = sorted_keys[seg_start[m]];
-    uint32_t h = hash_key(key) & cap_mask;
-    for (;;) {
-        const unsigned long long old = atomicCAS(reinterpret_cast<unsigned long long*>(hkeys + h), (unsigned long long)kEmptyKey,
-                                                 (unsigned long long)key);
-        if (old == (unsigned long long)kEmptyKey) { hvals[h] = (int32_t)m; return; }
-        h = (h + 1) & cap_mask;
-    }
+    if (m < n_seg) hash_insert_absent(t, sorted_keys[seg_start[m]], (int32_t)m);
 }
 
 // one level of the search structure: points bucketed by uniform-grid cell (sorted by cell key), cell -> bucket hash
 struct KnnGrid {
     const int32_t* idx;         // sorted position -> original index
     const int32_t* seg_start;   // [n_seg+1]
-    const uint64_t* hkeys;
-    const int32_t* hvals;
-    uint32_t cap_mask;
+    HashTable cells;            // cell key -> segment id
     double mn[3], cell;
     int dim[3];
     KeyLayout L;
@@ -415,14 +405,7 @@ __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double*
                 }
                 const int x = c[0] + dx, y = c[1] + dy, z = c[2] + dz;
                 if (x >= 0 && x < g.dim[0] && y >= 0 && y < g.dim[1] && z >= 0 && z < g.dim[2]) {
-                    const uint64_t key = layout_key(g.L, x, y, z);
-                    uint32_t h = hash_key(key) & g.cap_mask;
-                    for (;;) {
-                        const uint64_t hk = g.hkeys[h];
-                        if (hk == key) { seg = g.hvals[h]; break; }
-                        if (hk == kEmptyKey) break;
-                        h = (h + 1) & g.cap_mask;
-                    }
+                    seg = hash_find(g.cells, layout_key(g.L, x, y, z));
                 }
             }
             unsigned have = __ballot_sync(0xffffffffu, seg >= 0);
@@ -605,12 +588,13 @@ static int build_grid(const double* d_pts, int64_t n, const double mn[3], const 
     OT_TRY(sort_pairs(b.k0, b.i0, b.k1, b.i1, n, g.L.bits));
     OT_TRY(find_segments(b.k1.p, n, b.seg, &b.n_seg));
     uint32_t cap = 1024;
-    while ((int64_t)cap < 2 * b.n_seg) cap <<= 1;
+    while (!hash_fits(b.n_seg, cap)) cap <<= 1;
     OT_CUDA(b.hk.alloc(cap)); OT_CUDA(b.hv.alloc(cap));
     OT_CUDA(cudaMemset(b.hk.p, 0xFF, (size_t)cap * 8));
-    cell_hash_build_kernel<<<(unsigned)((b.n_seg + 255) / 256), 256>>>(b.k1.p, b.seg.p, b.n_seg, b.hk.p, b.hv.p, cap - 1);
+    g.cells = {b.hk.p, b.hv.p, cap - 1};
+    cell_hash_build_kernel<<<(unsigned)((b.n_seg + 255) / 256), 256>>>(b.k1.p, b.seg.p, b.n_seg, g.cells);
     OT_LAUNCHED();
-    g.idx = b.i1.p; g.seg_start = b.seg.p; g.hkeys = b.hk.p; g.hvals = b.hv.p; g.cap_mask = cap - 1;
+    g.idx = b.i1.p; g.seg_start = b.seg.p;
     return OTSLAM_OK;
 }
 
@@ -825,15 +809,7 @@ __global__ void __launch_bounds__(128) nn_within_kernel(KnnGrid g, const double*
             for (int dx = -1; dx <= 1; ++dx) {
                 const int x = c[0] + dx, y = c[1] + dy, z = c[2] + dz;
                 if (x < 0 || x >= g.dim[0] || y < 0 || y >= g.dim[1] || z < 0 || z >= g.dim[2]) continue;
-                const uint64_t key = layout_key(g.L, x, y, z);
-                uint32_t h = hash_key(key) & g.cap_mask;
-                int seg = -1;
-                for (;;) {
-                    const uint64_t hk = g.hkeys[h];
-                    if (hk == key) { seg = g.hvals[h]; break; }
-                    if (hk == kEmptyKey) break;
-                    h = (h + 1) & g.cap_mask;
-                }
+                const int seg = hash_find(g.cells, layout_key(g.L, x, y, z));
                 if (seg < 0) continue;
                 for (int j = g.seg_start[seg]; j < g.seg_start[seg + 1]; ++j) {
                     const int pi = g.idx[j];

@@ -28,8 +28,7 @@ constexpr double kMaxWindowVoxels = 4194304.0;  // 2^22: depth_max * max|d_c| / 
 // slot of block (bx, by, bz) (true x), -1 if absent or outside the selected object's window
 __device__ __forceinline__ int block_slot(const RayArgs& a, int bx, int by, int bz) {
     if (a.arena && (bx < -kObjHalf || bx >= kObjHalf)) return -1;
-    if (!key_in_range(bx + a.c.x_off, by, bz)) return -1;
-    return find_slot(a.c, pack_key(bx + a.c.x_off, by, bz));
+    return block_slot(a.c, bx, by, bz);
 }
 
 // trilinear colour at a world point over the observed corners only, renormalised; voxel colour = exact sum / count
@@ -109,7 +108,7 @@ __global__ void __launch_bounds__(kTileW * kTileH) raycast_kernel(const RayArgs 
                 const bool ok = !(a.arena && (b[0] < -kObjHalf || b[0] >= kObjHalf)) && key_in_range(b[0] + a.c.x_off, b[1], b[2]);
                 if (ok) {
                     const uint64_t key = pack_key(b[0] + a.c.x_off, b[1], b[2]);
-                    if (key != cur_key) { cur_key = key; cur_slot = find_slot(a.c, key); }
+                    if (key != cur_key) { cur_key = key; cur_slot = hash_find(a.c.table, key); }
                     slot = cur_slot;
                 }
                 if (slot < 0) {
@@ -267,7 +266,7 @@ int ray_args(const otslam_volume* v, int width, int height, const double intr[4]
     a.arena = v->n_objects > 0;
     a.color = v->color_type == OTSLAM_COLOR_RGB8;
     a.gap = 0.99 * v->voxel_length;
-    a.c.keys = v->d_keys; a.c.vals = v->d_vals; a.c.cap_mask = v->cap - 1; a.c.chunks = v->d_chunks;
+    a.c.table = volume_hash(v); a.c.chunks = v->d_chunks;
     a.c.bkeys = nullptr; a.c.bslots = nullptr; a.c.n = 0; a.c.slab = v->slab;
     a.c.vl = v->voxel_length; a.c.half = 0.5 * v->voxel_length; a.c.unit = v->unit_length;
     a.c.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0;

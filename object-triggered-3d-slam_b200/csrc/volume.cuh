@@ -2,7 +2,7 @@
 #pragma once
 #include <vector>
 
-#include "common.cuh"
+#include "hash_table.cuh"
 
 namespace otslam {
 
@@ -55,7 +55,7 @@ struct otslam_volume {
     int64_t obj_frames[otslam::kMaxObjects] = {};   // frames integrated per object (the 65535 limit is per voxel)
     int64_t frames_integrated = 0;
 
-    // block hash: open addressing, entry index is the handle used by the per-batch work list
+    // block hash (hash_table.cuh; volume_hash() below): the entry index is the handle used by the per-batch work list
     uint32_t cap = 0;
     uint64_t* d_keys = nullptr;
     int32_t* d_vals = nullptr;     // entry -> pool slot
@@ -124,8 +124,11 @@ int volume_sorted_blocks_device(otslam_volume* v, const uint64_t** d_keys, const
 int volume_selected_blocks_device(otslam_volume* v, const uint64_t** d_keys, const int32_t** d_slots, int* n, int* x_off);
 // the same downloaded to the host (export_blocks)
 int volume_sorted_blocks(otslam_volume* v, std::vector<uint64_t>& keys, std::vector<int32_t>& slots);
-// volume.cu, used by checkpoint.cu: 4x larger block hash (both streams drained first); pool chunks for blocks_needed slots
-int grow_hash(otslam_volume* v);
+// the volume's block hash as the kernels take it
+inline HashTable volume_hash(const otslam_volume* v) { return {v->d_keys, v->d_vals, v->cap - 1}; }
+// volume.cu, used by checkpoint.cu: grow the block hash until it holds n_entries (drains both streams first when it must
+// grow); pool chunks for blocks_needed slots
+int reserve_hash(otslam_volume* v, int64_t n_entries);
 int ensure_pool(otslam_volume* v, int64_t blocks_needed);
 // knn.cu: stable LSD radix sort of (u64 key, i32 value) pairs by the low `bits` bits; result in (kb, vb), (ka, va) clobbered
 int device_sort_pairs(uint64_t* ka, int32_t* va, uint64_t* kb, int32_t* vb, int64_t n, int bits, cudaStream_t s);

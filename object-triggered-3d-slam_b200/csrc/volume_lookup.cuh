@@ -1,14 +1,13 @@
-// volume_lookup.cuh -- read-only voxel lookups through the block hash, shared by extraction (extract.cu) and ray casting
-// (raycast.cu): the probe, and Open3D's GetTSDFAt (trilinear TSDF at a world point, the basis of GetNormalAt).
+// volume_lookup.cuh -- read-only voxel lookups through the block hash (hash_table.cuh), shared by extraction (extract.cu)
+// and ray casting (raycast.cu): the range-checked block lookup, and Open3D's GetTSDFAt (trilinear TSDF at a world point,
+// the basis of GetNormalAt).
 #pragma once
 #include "volume.cuh"
 
 namespace otslam {
 
 struct ExtractCtx {
-    const uint64_t* keys;     // hash
-    const int32_t* vals;
-    uint32_t cap_mask;
+    HashTable table;          // the volume's block hash
     uint4* const* chunks;
     const uint64_t* bkeys;    // [n] sorted block keys (extraction only)
     const int32_t* bslots;    // [n] their pool slots
@@ -18,15 +17,10 @@ struct ExtractCtx {
     int x_off;                // multi-object arena: x-key offset of the selected object (stored key - x_off = true block x)
 };
 
-__device__ __forceinline__ int find_slot(const ExtractCtx& c, uint64_t key) {
-    uint32_t h = hash_key(key) & c.cap_mask;
-    for (uint32_t probe = 0; probe <= c.cap_mask; ++probe) {
-        const uint64_t k = c.keys[h];
-        if (k == key) return c.vals[h];
-        if (k == kEmptyKey) return -1;
-        h = (h + 1) & c.cap_mask;
-    }
-    return -1;
+// pool slot of block (bx, by, bz) (true x: the arena offset is added here), -1 if absent or outside the key range
+__device__ __forceinline__ int block_slot(const ExtractCtx& c, int bx, int by, int bz) {
+    if (!key_in_range(bx + c.x_off, by, bz)) return -1;
+    return hash_find(c.table, pack_key(bx + c.x_off, by, bz));
 }
 
 // ---- ScalableTSDFVolume::GetTSDFAt: trilinear interpolation of the TSDF at a world point (FP64).  Voxels of absent blocks
@@ -40,7 +34,7 @@ __device__ inline double tsdf_at(const ExtractCtx& c, const double p[3]) {
         index0[i] = (int)floor(__ddiv_rn(pl, c.unit));
         pg[i] = __ddiv_rn(__dsub_rn(pl, __dmul_rn((double)index0[i], c.unit)), c.vl);
     }
-    if (!key_in_range(index0[0] + c.x_off, index0[1], index0[2]) || find_slot(c, pack_key(index0[0] + c.x_off, index0[1], index0[2])) < 0) return 0.0;
+    if (block_slot(c, index0[0], index0[1], index0[2]) < 0) return 0.0;
 #pragma unroll
     for (int i = 0; i < 3; ++i) {
         idx0[i] = min(max((int)floor(pg[i]), 0), kRes - 1);
@@ -54,7 +48,7 @@ __device__ inline double tsdf_at(const ExtractCtx& c, const double p[3]) {
 #pragma unroll
         for (int j = 0; j < 3; ++j)
             if (v[j] >= kRes) { v[j] -= kRes; b[j] += 1; }
-        const int s = key_in_range(b[0] + c.x_off, b[1], b[2]) ? find_slot(c, pack_key(b[0] + c.x_off, b[1], b[2])) : -1;
+        const int s = block_slot(c, b[0], b[1], b[2]);
         f[q] = s >= 0 ? (double)__uint_as_float(block_ptr(c.chunks, s)[rec_index(v[0], v[1], v[2])].x) : 0.0;
     }
     const double o0 = __dsub_rn(1.0, r[0]), o1 = __dsub_rn(1.0, r[1]), o2 = __dsub_rn(1.0, r[2]);
