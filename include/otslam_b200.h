@@ -228,6 +228,20 @@ int otslam_volume_track(otslam_volume* v, int n_frames, const uint16_t* depth, i
                         const double* init_extrinsics, double depth_scale, double depth_min, double depth_max,
                         double depth_diff, int max_iterations, double* extrinsics_out, int32_t* status,
                         int32_t* iterations, double* fitness, double* inlier_rmse, int memory);
+/* ---- coarse-to-fine frame-to-model tracking: otslam_volume_track over a depth pyramid of n_levels (1..4) levels, index
+ *      = level, 0 = full resolution.  Level l + 1 halves level l (an odd last column or row dropped; intrinsics fx / 2,
+ *      fy / 2, (cx - 0.5) / 2, (cy - 0.5) / 2); a coarse pixel averages the valid depths of its 2x2 block that lie within
+ *      4 voxels of the block's nearest.  Each level has its own model render at init_extrinsics[i], its own gate
+ *      depth_diff[l] (metres, finite and > 0) and its own max_iterations[l] (1..100).  Levels run from the coarsest to 0,
+ *      each from the pose the coarser level returned, whatever its status.  status is level 0's; iterations are summed
+ *      over the levels; fitness and inlier_rmse are level 0's at the returned pose.  With more than one level the
+ *      coarsest must be at least 16x8 pixels.  n_levels = 1 is otslam_volume_track, bit for bit.  Other arguments,
+ *      outputs and checks as otslam_volume_track. */
+int otslam_volume_track_pyramid(otslam_volume* v, int n_frames, const uint16_t* depth, int width, int height,
+                                const double intr[4], const double* init_extrinsics, double depth_scale,
+                                double depth_min, double depth_max, int n_levels, const double* depth_diff,
+                                const int32_t* max_iterations, double* extrinsics_out, int32_t* status,
+                                int32_t* iterations, double* fitness, double* inlier_rmse, int memory);
 
 /* ---- stateless image / cloud operators.  Every pointer argument may be a HOST pointer or a DEVICE pointer of `device`
  *      (unified addressing; the copies inside become device-to-device): a caller that keeps its clouds in HBM between

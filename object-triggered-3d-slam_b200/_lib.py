@@ -72,6 +72,7 @@ _SIGS = {
     "otslam_volume_points_normals": (_i, [_vp, _vp]),
     "otslam_volume_raycast": (_i, [_vp, _i, _i, _i, _vp, _vp, _d, _d, _vp, _vp, _vp, _vp, C.POINTER(_i64)]),
     "otslam_volume_track": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _d, _d, _d, _d, _i, _vp, _vp, _vp, _vp, _vp, _i]),
+    "otslam_volume_track_pyramid": (_i, [_vp, _i, _vp, _i, _i, _vp, _vp, _d, _d, _d, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i]),
     "otslam_depth_convert": (_i, [_vp, _i64, _d, _d, _vp, _i]),
     "otslam_backproject_rgbd": (_i, [_vp, _vp, _i, _i, _vp, _vp, _vp, _vp, C.POINTER(_i64), _i]),
     "otslam_mesh_vertex_normals": (_i, [_vp, _i64, _vp, _i64, _vp, _i]),

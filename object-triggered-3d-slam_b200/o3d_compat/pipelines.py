@@ -115,7 +115,8 @@ class ScalableTSDFVolume:
         """Refine the pose of one frame (an RGBDImage with raw u16 depth; its depth scale is used) against the volume by
         point-to-plane ICP on its ray-cast model, starting from `extrinsic` (world->camera 4x4).  Unlike Open3D, whose
         result holds a camera-to-camera correction, OdometryResult.transformation IS the refined world->camera extrinsic:
-        what integrate() takes.  The volume is only read."""
+        what integrate() takes.  depth_diff and max_iterations may be per-level sequences (coarse-to-fine tracking over a
+        depth pyramid, as TSDFVolume.track; volume.TRACK_PYRAMID is the recommended setting).  The volume is only read."""
         if image._depth_raw is None or not image._depth_is_raw_u16:
             raise RuntimeError("track_frame_to_model needs an RGBDImage made from raw u16 depth")
         r = self._vol.track(image._depth_raw, intrinsic.fxfycxcy(), extrinsic, image._depth_scale, depth_min, depth_max,

@@ -29,6 +29,11 @@ def checkpoint_profile():
     return {"kernel_ms": float(out[0]), "copy_ms": float(out[1]), "file_ms": float(out[2]), "wall_ms": float(out[3])}
 
 
+# Recommended coarse-to-fine setting of TSDFVolume.track (index = pyramid level, 0 = full resolution), chosen from
+# tools/track_bench.py on a B200 (DESIGN.md §4 "Frame-to-model tracking"): vol.track(..., **TRACK_PYRAMID).
+TRACK_PYRAMID = {"depth_diff": (0.07, 0.1, 0.2, 0.4), "max_iterations": (20, 10, 10, 10)}
+
+
 class TSDFVolume:
     def __init__(self, voxel_length, sdf_trunc, color=True, device=0, slab=None):
         self.voxel_length, self.sdf_trunc, self.device = float(voxel_length), float(sdf_trunc), int(device)
@@ -367,7 +372,15 @@ class TSDFVolume:
         independently against the volume as it is; the volume is only read.  Returns a dict: extrinsic [n,4,4] (refined),
         status [n] (0 converged, 1 reached max_iterations, 2 fewer than 64 inliers, 3 degenerate; 2 and 3 keep the last
         pose), iterations [n], fitness [n] (inliers / valid pixels) and inlier_rmse [n] (metres); unbatched for one
-        [H,W] frame."""
+        [H,W] frame.
+
+        depth_diff and max_iterations may each be a sequence of per-level values (index = level, 0 = full resolution):
+        the frames are then tracked coarse to fine over a depth pyramid of that many levels (1..4), and a scalar beside a
+        sequence applies to every level.  status is then level 0's and iterations the sum over the levels.
+        TRACK_PYRAMID is the recommended setting for starts a few centimetres and degrees off."""
+        levels = {len(x) for x in (depth_diff, max_iterations) if np.ndim(x) > 0}
+        if len(levels) > 1:
+            raise ValueError(f"depth_diff and max_iterations give different level counts {sorted(levels)}")
         on_dev = hasattr(depth, "is_cuda") and depth.is_cuda
         if on_dev:
             assert depth.is_contiguous() and depth.element_size() == 2
@@ -382,11 +395,18 @@ class TSDFVolume:
                "fitness": np.empty(n), "inlier_rmse": np.empty(n)}
         if on_dev:
             self._after_torch_stream(depth)
-        _lib.check(_lib.lib.otslam_volume_track(
-            self._h, n, _lib.ptr(depth), W, H, _lib.ptr(self._intr(intr)), _lib.ptr(e), float(depth_scale), float(depth_min),
-            float(depth_max), float(depth_diff), int(max_iterations), _lib.ptr(out["extrinsic"]), _lib.ptr(out["status"]),
-            _lib.ptr(out["iterations"]), _lib.ptr(out["fitness"]), _lib.ptr(out["inlier_rmse"]),
-            _lib.MEM_DEVICE if on_dev else _lib.MEM_HOST))
+        outs = (_lib.ptr(out["extrinsic"]), _lib.ptr(out["status"]), _lib.ptr(out["iterations"]), _lib.ptr(out["fitness"]),
+                _lib.ptr(out["inlier_rmse"]), _lib.MEM_DEVICE if on_dev else _lib.MEM_HOST)
+        k = self._intr(intr)                # kept alive across the call: only its address goes into `head`
+        head = (self._h, n, _lib.ptr(depth), W, H, _lib.ptr(k), _lib.ptr(e), float(depth_scale), float(depth_min),
+                float(depth_max))
+        if levels:
+            L = levels.pop()
+            dd = np.ascontiguousarray(np.broadcast_to(np.asarray(depth_diff, np.float64), (L,)))
+            mi = np.ascontiguousarray(np.broadcast_to(np.asarray(max_iterations, np.int32), (L,)))
+            _lib.check(_lib.lib.otslam_volume_track_pyramid(*head, L, _lib.ptr(dd), _lib.ptr(mi), *outs))
+        else:
+            _lib.check(_lib.lib.otslam_volume_track(*head, float(depth_diff), int(max_iterations), *outs))
         if single:
             out = {k: a[0] for k, a in out.items()}
         return out

@@ -1,12 +1,14 @@
-"""Frame-to-model tracking timings and pose errors on one GPU.  Prints one JSON line.
+"""Frame-to-model tracking timings and pose errors on one GPU, single-scale and coarse to fine.  Prints one JSON line.
 
 Legs: configs[1] (1000 frames of the chair+table sequence, 640x480, 5 mm) and the HD geometry of configs[3] (2000 frames of
 the large room, 1280x720, 2 mm).  Per leg the volume is integrated from HBM at the true poses, then every captured frame
 (a CUDA tensor) is tracked against it in batches of 32, from initial poses moved by 1-3 cm and turned by 1-2 degrees in
-seeded random directions.  One batch warms up first.  Reported: frames/s from the device time of the calls
-(otslam_last_op_device_ms, summed) and from wall time; the share of device time that the model render takes (the same
-poses ray cast separately into CUDA tensors with vertex and normal only: the tracker's render); mean iterations, status
-counts, and median and maximum translation and rotation error against the true poses.
+seeded random directions, twice from the same starts: single-scale (the defaults of TSDFVolume.track) and with
+volume.TRACK_PYRAMID.  One batch of each warms up first.  Reported per run: frames/s from the device time of the calls
+(otslam_last_op_device_ms, summed) and from wall time; mean iterations; status counts; and the median, 95th percentile and
+maximum translation and rotation error against the true poses, for each status separately.  Single-scale runs also report
+the share of device time that the model render takes (the same poses ray cast separately into CUDA tensors with vertex
+and normal only: the tracker's render).
 """
 import argparse
 import json
@@ -56,10 +58,47 @@ def starts(extrinsics, seed):
     return np.stack(out)
 
 
-def leg(name, scene, frames, intr, voxel):
+def stats(x):
+    import numpy as np
+    return {"median": float(np.median(x)), "p95": float(np.percentile(x, 95)), "max": float(x.max())} if len(x) else None
+
+
+def run(vol, d, k, init, ext, W, H, render, **kw):
+    """track every frame in batches from `init` with TSDFVolume.track(**kw); timings, status counts and errors by status"""
     import numpy as np
     import torch
-    from otslam_b200 import _lib, synth
+    from otslam_b200 import _lib
+    frames = len(init)
+    vol.track(d[:BATCH], k, init[:BATCH], **kw)                     # warm-up
+    torch.cuda.synchronize()
+    dev_ms, wall, render_ms = 0.0, 0.0, 0.0
+    res = {x: [] for x in ("extrinsic", "status", "iterations")}
+    for first in range(0, frames, BATCH):
+        t0 = time.perf_counter()
+        r = vol.track(d[first:first + BATCH], k, init[first:first + BATCH], **kw)   # returns with the results on the host
+        wall += time.perf_counter() - t0
+        dev_ms += _lib.last_op_device_ms()
+        for x in res:
+            res[x].append(r[x])
+        if render:
+            vol.ray_cast_tensors(k, init[first:first + BATCH], W, H, attributes=("vertex", "normal"))
+            render_ms += _lib.last_op_device_ms()
+    res = {x: np.concatenate(v) for x, v in res.items()}
+    err = np.array([pose_error(x, t) for x, t in zip(res["extrinsic"], ext)])
+    out = {"frames_per_s_device": frames / (dev_ms * 1e-3), "frames_per_s_wall": frames / wall,
+           "mean_iterations": float(res["iterations"].mean()),
+           "status_counts": {str(s): int((res["status"] == s).sum()) for s in range(4)},
+           "error_by_status": {str(s): {"translation_mm": stats(err[res["status"] == s, 0] * 1e3),
+                                        "rotation_deg": stats(err[res["status"] == s, 1])}
+                               for s in range(4) if (res["status"] == s).any()}}
+    if render:
+        out["render_share_of_device_time"] = render_ms / dev_ms
+    return out
+
+
+def leg(name, scene, frames, intr, voxel, settings):
+    import torch
+    from otslam_b200 import synth
     from otslam_b200.volume import TSDFVolume
     seq = synth.make_sequence(scene, frames, intr=intr, device="cuda:0")
     d, c, ext, k = seq.depth, seq.rgb, seq.extrinsic, seq.fxfycxcy
@@ -68,29 +107,12 @@ def leg(name, scene, frames, intr, voxel):
     vol.integrate_batch(d, c, k, ext)
     torch.cuda.synchronize()
     init = starts(ext, 11)
-    vol.track(d[:BATCH], k, init[:BATCH])                          # warm-up
-    vol.ray_cast_tensors(k, init[:BATCH], W, H, attributes=("vertex", "normal"))
-    torch.cuda.synchronize()
-    dev_ms, wall, render_ms = 0.0, 0.0, 0.0
-    res = {x: [] for x in ("extrinsic", "status", "iterations")}
-    for first in range(0, frames, BATCH):
-        t0 = time.perf_counter()
-        r = vol.track(d[first:first + BATCH], k, init[first:first + BATCH])   # returns with the results on the host
-        wall += time.perf_counter() - t0
-        dev_ms += _lib.last_op_device_ms()
-        for x in res:
-            res[x].append(r[x])
-        vol.ray_cast_tensors(k, init[first:first + BATCH], W, H, attributes=("vertex", "normal"))
-        render_ms += _lib.last_op_device_ms()
-    res = {x: np.concatenate(v) for x, v in res.items()}
-    err = np.array([pose_error(x, t) for x, t in zip(res["extrinsic"], ext)])
+    vol.ray_cast_tensors(k, init[:BATCH], W, H, attributes=("vertex", "normal"))     # warm-up of the separate render
+    out = {"workload": name, "frames": frames, "width": W, "height": H, "voxel_mm": voxel * 1000}
+    for label, kw in settings.items():
+        out[label] = run(vol, d, k, init, ext, W, H, not kw, **kw)
     vol.close()
-    return {"workload": name, "frames": frames, "width": W, "height": H, "voxel_mm": voxel * 1000,
-            "frames_per_s_device": frames / (dev_ms * 1e-3), "frames_per_s_wall": frames / wall,
-            "render_share_of_device_time": render_ms / dev_ms, "mean_iterations": float(res["iterations"].mean()),
-            "status_counts": {str(s): int((res["status"] == s).sum()) for s in range(4)},
-            "translation_error_mm": {"median": float(np.median(err[:, 0]) * 1e3), "max": float(err[:, 0].max() * 1e3)},
-            "rotation_error_deg": {"median": float(np.median(err[:, 1])), "max": float(err[:, 1].max())}}
+    return out
 
 
 def main():
@@ -102,13 +124,17 @@ def main():
     if not torch.cuda.is_available():
         sys.exit("track_bench needs a CUDA device")
     from otslam_b200 import synth
+    from otslam_b200.volume import TRACK_PYRAMID
     from raycast_bench import gpu_details
     res = gpu_details()
     res["batch_frames"] = BATCH
     res["initial_error"] = "1-3 cm, 1-2 degrees, seeded directions"
-    res["legs"] = [leg("configs[1] chair+table 640x480", "chair_table", a.frames, synth.REF_INTRINSICS, 0.005)]
+    settings = {"single_scale": {}, "pyramid": dict(TRACK_PYRAMID)}
+    res["pyramid"] = settings["pyramid"]
+    res["legs"] = [leg("configs[1] chair+table 640x480", "chair_table", a.frames, synth.REF_INTRINSICS, 0.005, settings)]
     if a.hd_frames > 0:
-        res["legs"].append(leg("configs[3] geometry: large room 1280x720", "room", a.hd_frames, synth.HD_INTRINSICS, 0.002))
+        res["legs"].append(leg("configs[3] geometry: large room 1280x720", "room", a.hd_frames, synth.HD_INTRINSICS, 0.002,
+                               settings))
     print(json.dumps(res))
 
 
