@@ -89,7 +89,8 @@ __host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
 // objects share ONE block hash / pool / per-batch work list, so that one integration launch covers the union of their
 // touched blocks.  The object id lives in the block key: object o (0..7) owns the x-key window
 // [o * 2^18 - 2^20 + 0, +2^18), i.e. its true block coordinate kx in [-2^17, 2^17) is stored as kx + obj_key_offset(o).
-// Blocks of different objects are never neighbours, and sorting by key groups the blocks by object.
+// Sorting by key groups the blocks by object.  The stored key one past an object's last block (true kx = 2^17 - 1) is the
+// next object's first block (true kx = -2^17): readers go through block_slot() (volume_lookup.cuh), which checks the window.
 constexpr int kObjShift = 18;
 constexpr int kMaxObjects = 8;
 constexpr int kObjHalf = 1 << (kObjShift - 1);            // |true kx| limit inside an arena

@@ -25,12 +25,6 @@ constexpr size_t kStagingBytes = 256ull << 20;  // per staging buffer (two of th
 constexpr int kTileW = 16, kTileH = 8;
 constexpr double kMaxWindowVoxels = 4194304.0;  // 2^22: depth_max * max|d_c| / vl, keeps one-voxel steps >= 2 ulp(t)
 
-// slot of block (bx, by, bz) (true x), -1 if absent or outside the selected object's window
-__device__ __forceinline__ int block_slot(const RayArgs& a, int bx, int by, int bz) {
-    if (a.arena && (bx < -kObjHalf || bx >= kObjHalf)) return -1;
-    return block_slot(a.c, bx, by, bz);
-}
-
 // trilinear colour at a world point over the observed corners only, renormalised; voxel colour = exact sum / count
 __device__ __forceinline__ void color_at(const RayArgs& a, const double p[3], uint8_t out[3]) {
     int g0[3];
@@ -46,7 +40,7 @@ __device__ __forceinline__ void color_at(const RayArgs& a, const double p[3], ui
     for (int q = 0; q < 8; ++q) {
         const int sx = q & 1, sy = (q >> 1) & 1, sz = q >> 2;
         const int g[3] = {g0[0] + sx, g0[1] + sy, g0[2] + sz};
-        const int s = block_slot(a, g[0] >> 4, g[1] >> 4, g[2] >> 4);
+        const int s = block_slot(a.c, g[0] >> 4, g[1] >> 4, g[2] >> 4);
         if (s < 0) continue;
         const uint4 rec = __ldg(block_ptr(a.c.chunks, s) + rec_index(g[0] & 15, g[1] & 15, g[2] & 15));
         const uint32_t w = rec_weight(rec);
@@ -104,13 +98,11 @@ __global__ void __launch_bounds__(kTileW * kTileH) raycast_kernel(const RayArgs 
             } else {
                 const int g[3] = {(int)q[0], (int)q[1], (int)q[2]};
                 const int b[3] = {g[0] >> 4, g[1] >> 4, g[2] >> 4};
-                int slot = -1;
-                const bool ok = !(a.arena && (b[0] < -kObjHalf || b[0] >= kObjHalf)) && key_in_range(b[0] + a.c.x_off, b[1], b[2]);
-                if (ok) {
-                    const uint64_t key = pack_key(b[0] + a.c.x_off, b[1], b[2]);
-                    if (key != cur_key) { cur_key = key; cur_slot = hash_find(a.c.table, key); }
-                    slot = cur_slot;
-                }
+                // |q| < 2^24 keeps every b within [-2^20, 2^20), where the packed key tells blocks apart even when the arena
+                // offset takes x outside the key range (block_slot then finds the block absent)
+                const uint64_t key = pack_key(b[0] + a.c.x_off, b[1], b[2]);
+                if (key != cur_key) { cur_key = key; cur_slot = block_slot(a.c, b[0], b[1], b[2]); }
+                const int slot = cur_slot;
                 if (slot < 0) {
                     // absent block: to where the ray leaves it (the nearest exit plane), at least one voxel
                     have_prev = false;
@@ -263,13 +255,13 @@ int ray_args(const otslam_volume* v, int width, int height, const double intr[4]
     if (!(depth_max * max_len / v->voxel_length <= kMaxWindowVoxels))
         return set_error(OTSLAM_ERR_INVALID, p + ": depth_max * max|d_c| / voxel_length exceeds 2^22");
     a.cap = (int)raycast_cap(depth_min, depth_max, max_len, v->voxel_length);
-    a.arena = v->n_objects > 0;
     a.color = v->color_type == OTSLAM_COLOR_RGB8;
     a.gap = 0.99 * v->voxel_length;
     a.c.table = volume_hash(v); a.c.chunks = v->d_chunks;
     a.c.bkeys = nullptr; a.c.bslots = nullptr; a.c.n = 0; a.c.slab = v->slab;
     a.c.vl = v->voxel_length; a.c.half = 0.5 * v->voxel_length; a.c.unit = v->unit_length;
     a.c.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0;
+    a.c.arena = v->n_objects > 0;
     *out = a;
     return OTSLAM_OK;
 }

@@ -18,7 +18,6 @@ struct RayArgs {
     float vl, ktr;          // (float)voxel_length, (float)(k * sdf_trunc)
     float dmin, dmax;
     int cap;                // iterations per ray (host: raycast_cap)
-    int arena;              // multi-object arena: a block whose true x lies outside [-2^17, 2^17) is absent
     int color;              // volume keeps colour
     double gap;             // 0.99 voxel (GetNormalAt)
     float* depth;           // outputs of this chunk, [chunk][H][W](...) or null

@@ -15,11 +15,13 @@ struct ExtractCtx {
     SlabSpec slab;
     double vl, half, unit;    // voxel length, half of it, block edge length
     int x_off;                // multi-object arena: x-key offset of the selected object (stored key - x_off = true block x)
+    bool arena;               // multi-object arena: a block whose true x lies outside [-2^17, 2^17) is absent
 };
 
-// pool slot of block (bx, by, bz) (true x: the arena offset is added here), -1 if absent or outside the key range
+// pool slot of block (bx, by, bz) (true x: the arena offset is added here), -1 if absent, outside the key range or outside
+// the selected arena object's window (the stored key one past an object's last block is the next object's first block)
 __device__ __forceinline__ int block_slot(const ExtractCtx& c, int bx, int by, int bz) {
-    if (!key_in_range(bx + c.x_off, by, bz)) return -1;
+    if ((c.arena && (bx < -kObjHalf || bx >= kObjHalf)) || !key_in_range(bx + c.x_off, by, bz)) return -1;
     return hash_find(c.table, pack_key(bx + c.x_off, by, bz));
 }
 

@@ -364,6 +364,22 @@ int oracle_volume_halo_import(void* h, int64_t n, const int32_t* keys, const flo
     }
     return 0;
 }
+// Whole blocks as export_blocks gives them (keys [n][3], tsdf / weight [n][4096], colour [n][4096][3] on the 0..255 scale;
+// voxel index x*256 + y*16 + z): a block already present is overwritten.  Extraction, point normals and the ray-cast and
+// tracking models then have a CPU reference for any block set, including keys no camera would reach.
+int oracle_volume_import_blocks(void* h, int64_t n, const int32_t* keys, const float* tsdf, const float* weight, const double* color) {
+    Volume* v = (Volume*)h;
+    for (int64_t i = 0; i < n; ++i) {
+        Key k{keys[3 * i], keys[3 * i + 1], keys[3 * i + 2]};
+        auto it = v->blocks.find(k);
+        if (it == v->blocks.end()) it = v->blocks.emplace(k, new Block(k)).first;
+        Block* b = it->second;
+        memcpy(b->tsdf.data(), tsdf + i * NVOX, NVOX * sizeof(float));
+        memcpy(b->weight.data(), weight + i * NVOX, NVOX * sizeof(float));
+        memcpy(b->color.data(), color + i * 3 * NVOX, 3 * NVOX * sizeof(double));
+    }
+    return 0;
+}
 void oracle_volume_destroy(void* h) { delete (Volume*)h; }
 void oracle_volume_reset(void* h) {
     Volume* v = (Volume*)h;

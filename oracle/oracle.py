@@ -144,6 +144,16 @@ class Volume:
         k = np.ascontiguousarray(keys, np.int32)
         lib().oracle_volume_halo_import(self.h, C.c_int64(n), _p(k), _p(tsdf), _p(w), _p(col))
 
+    def import_blocks(self, keys, tsdf, weight, color):
+        """Add whole blocks in export_blocks' form (keys [n,3] i32, tsdf / weight [n,4096] f32, colour [n,4096,3] f64 on the
+        0..255 scale); a block already present is overwritten."""
+        k = np.ascontiguousarray(keys, np.int32).reshape(-1, 3)
+        n = len(k)
+        t = np.ascontiguousarray(tsdf, np.float32).reshape(n, 4096)
+        w = np.ascontiguousarray(weight, np.float32).reshape(n, 4096)
+        c = np.ascontiguousarray(color, np.float64).reshape(n, 4096, 3)
+        lib().oracle_volume_import_blocks(self.h, C.c_int64(n), _p(k), _p(t), _p(w), _p(c))
+
     def extract_triangle_mesh(self):
         nv, nf = C.c_int64(0), C.c_int64(0)
         m = C.c_void_p(lib().oracle_volume_extract_mesh(self.h, C.byref(nv), C.byref(nf)))

@@ -30,8 +30,9 @@ def word_sum(words):
 
 
 def pack_key(x, y, z):
-    b = 1 << 20
-    return ((x + b) << 42) | ((y + b) << 21) | (z + b)
+    """the library's pack_key, also for keys outside the range (each biased field taken as uint32, shifted, mod 2^64)"""
+    b, m = 1 << 20, (1 << 32) - 1
+    return ((((x + b) & m) << 42) | (((y + b) & m) << 21) | ((z + b) & m)) & ((1 << 64) - 1)
 
 
 def block_checksum(records, key):
