@@ -7,6 +7,10 @@
 namespace otslam {
 
 constexpr int kMaxBatch = 32;   // frames fused per block residency (one bit each in the entry mask)
+// integration kernel's brick cull (tests/cull_ref.py models it): max-depth tile edge in pixels, and the most tiles one
+// (brick, frame) test reads; a footprint over more tiles is not tested.  Chosen by tools/study_culling_bricks.py.
+constexpr int kCullTile = 4;
+constexpr int kCullMaxTiles = 36;
 
 // per-frame constants consumed by the allocation (FP64 pose) and integration (FP32 extrinsic) kernels
 struct FrameDev {
@@ -79,7 +83,9 @@ struct otslam_volume {
     uint16_t* d_raw_depth[otslam::kNB] = {};
     uint8_t* d_raw_rgb[otslam::kNB] = {};
     uint2* d_packed[otslam::kNB] = {};
-    size_t raw_frames_cap = 0, raw_px_cap = 0, packed_cap = 0, packed_px = 0;
+    float* d_tiles[otslam::kNB] = {};      // max-depth tiles of the packed frames (integration kernel's brick cull)
+    bool cull = true;                      // OTSLAM_K4_CULL=0 turns the brick cull off (results are the same)
+    size_t raw_frames_cap = 0, raw_px_cap = 0, packed_cap = 0, packed_px = 0, tiles_cap = 0;
     size_t raw_depth_bytes_per_px = 2;
     cudaEvent_t ev_copied[otslam::kNB] = {}, ev_raw_free[otslam::kNB] = {};
     otslam::FrameDev* d_frames[otslam::kNB] = {};
