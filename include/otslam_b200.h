@@ -284,6 +284,41 @@ int otslam_cloud_nn_distance(const double* source, int64_t n_source, const doubl
  * o3d_compat/pipelines.py. */
 int otslam_cloud_nn_within(const double* source, int64_t n_source, const double* target, int64_t n_target, double radius,
                            int32_t* out_index, double* out_dist2, int device);
+/* PointCloud.estimate_normals(KDTreeSearchParamHybrid(radius, max_nn)) (radius = +inf: KDTreeSearchParamKNN(max_nn)), for
+ * clouds that come without normals (a ground-truth scan, a cloud read from PLY).  Arithmetic in DESIGN.md §4 "Normals and
+ * point-to-plane registration":
+ *   neighbours of point i = the min(max_nn, m) points with the smallest squared distance among the m points with
+ *     d2 < radius^2, point i itself included (d2 = 0); d2 = (dx^2 + dy^2) + dz^2 in FP64, the list ordered by (d2, index)
+ *     ascending, so that the set and the summation order do not depend on the search structure (lattices, duplicated and
+ *     identical points included);
+ *   covariance = Open3D's ComputeCovariance: the nine cumulants x, y, z, xx, xy, xz, yy, yz, zz summed in neighbour order,
+ *     divided by the count, C = E[x x^T] - mu mu^T; C = I with fewer than 3 neighbours;
+ *   normal = the unit eigenvector of C's smallest eigenvalue by a cyclic Jacobi (+ - * / sqrt only, C scaled by its largest
+ *     |entry|; among equal eigenvalues the highest index, so C = I gives (0, 0, 1)); a zero vector becomes the prior
+ *     normal, or (0, 0, 1) without priors;
+ *   sign: with prior_normals (nullable; a cloud's existing normals) flipped when n . prior < 0; without, flipped so that
+ *     the largest-magnitude component (the first of equal ones) is positive.
+ * out_normals [n][3].  1 <= max_nn <= 128, radius > 0 (finite, or +inf), n < 2^31, non-null points and out_normals:
+ * otherwise OTSLAM_ERR_INVALID before any CUDA call.  otslam_last_op_device_ms() = device ms of search and kernel. */
+int otslam_cloud_estimate_normals(const double* points, int64_t n, const double* prior_normals, double radius, int max_nn,
+                                  double* out_normals, int device);
+/* o3d.pipelines.registration.registration_icp(source, target, max_distance, init,
+ * TransformationEstimationPointToPlane(), ICPConvergenceCriteria(relative_fitness, relative_rmse, max_iteration)) in one
+ * call: Open3D's RegistrationICP loop, correspondences by otslam_cloud_nn_within's rule (nearest target strictly within
+ * max_distance, ties to the lower index) on a grid of the target built once.  The source is moved by init, evaluated, then
+ * each iteration solves J^T J x = -J^T r (r = n . (s - t), J = [s x n, n], n = the target's normal; FP64 sums by fixed
+ * trees, the tracking's Cholesky and degeneracy rule), turns x into R = Rz(x2) Ry(x1) Rx(x0), t = x[3..5] (identity when
+ * the solve fails or nothing corresponds), sets T <- update * T, moves the source by the update and evaluates again; it stops
+ * after max_iteration (>= 0) iterations or when |d fitness| < relative_fitness and |d rmse| < relative_rmse.
+ * fitness = inliers / n_source, inlier_rmse = sqrt(sum d2 / inliers) (0 without inliers), both at the returned transform;
+ * corr_index [n_source] (nullable) = each source point's target index or -1 from the last evaluation.  source, target,
+ * target_normals and corr_index may be device pointers; init, transform_out [16] and the scalar outputs (nullable) are host
+ * pointers.  n_source = 0 returns init with 0 iterations.  Bad arguments give OTSLAM_ERR_INVALID before any CUDA call.
+ * otslam_last_op_device_ms() = device ms from the grid build to the last evaluation. */
+int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, const double* target, const double* target_normals,
+                                    int64_t n_target, double max_distance, const double init[16], double relative_fitness,
+                                    double relative_rmse, int max_iteration, double transform_out[16], double* fitness,
+                                    double* inlier_rmse, int32_t* iterations, int32_t* corr_index, int device);
 /* create_map_cloud's pixel loop (fusion/hybrid_map.py:45-55); out sized w*h*3 (or NULL to count) */
 int otslam_grid_to_points(const uint8_t* gray, int width, int height, double resolution, double origin_x,
                           double origin_y, int threshold, double* out_points, int64_t* n_out, int device);

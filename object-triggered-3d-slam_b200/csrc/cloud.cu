@@ -511,6 +511,18 @@ int otslam_grid_to_points(const uint8_t* gray, int width, int height, double res
     return OTSLAM_OK;
 }
 
+// p' = (T * [p, 1]).xyz / w on device buffers (otslam_cloud_transform's arithmetic), queued on stream s; the cloud ICP
+// moves its source by each update with it
+int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s) {
+    if (n <= 0) return OTSLAM_OK;
+    RigidArgs a;
+    for (int i = 0; i < 16; ++i) a.m[i] = T[i];
+    a.mode = 0;
+    rigid_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_in, nullptr, n, a, d_out, nullptr);
+    OT_LAUNCHED();
+    return OTSLAM_OK;
+}
+
 static int rigid_apply(const double* points, const double* normals, int64_t n, const RigidArgs& a, double* out_points, double* out_normals,
                        int device) {
     if (n < 0 || (n && (!points || !out_points))) return set_error(OTSLAM_ERR_INVALID, "bad arguments");

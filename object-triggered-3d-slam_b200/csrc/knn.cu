@@ -17,6 +17,7 @@
 #include <cstdlib>
 #include <vector>
 
+#include "icp_solve.h"
 #include "volume.cuh"
 
 namespace otslam {
@@ -349,11 +350,35 @@ __device__ __forceinline__ void warp_argmax(const double* best, int cnt, int lan
     vmax = v; pmax = p;
 }
 
-// ring search on one level; true when the k best are final (ring termination or whole grid covered),
-// false when `last_ring` was scanned without reaching that point
+// (d2, index) order of the normal estimation's neighbour lists
+__device__ __forceinline__ bool pair_less(double d, int i, double e, int j) { return d < e || (d == e && i < j); }
+
+// the largest (d2, index) of the list: its value, index and position
+__device__ __forceinline__ void warp_argmax_idx(const double* best, const int* bidx, int cnt, int lane, double& vmax, int& imax,
+                                                int& pmax) {
+    double v = -1.0;
+    int i = -1, p = 0;
+    for (int e = lane; e < cnt; e += 32)
+        if (pair_less(v, i, best[e], bidx[e])) { v = best[e]; i = bidx[e]; p = e; }
+    for (int o = 16; o; o >>= 1) {
+        const double ov = __shfl_xor_sync(0xffffffffu, v, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, i, o);
+        const int op = __shfl_xor_sync(0xffffffffu, p, o);
+        if (pair_less(v, i, ov, oi)) { v = ov; i = oi; p = op; }
+    }
+    vmax = v; imax = i; pmax = p;
+}
+
+// The k best of a query on one level of the search structure.  kIdx = false (statistical outlier removal, nearest
+// distance): the k smallest squared distances, a newcomer inserted after its equals.  kIdx = true (normal estimation):
+// the k smallest (d2, index) pairs among the points with d2 < r2, the index carried beside each distance (reg_idx in
+// registers for k <= 32, bidx in shared memory up to 128), and the ring walk also ends once the scanned box reaches
+// beyond the radius.  True when the k best are final (ring termination, radius reached or whole grid covered), false
+// when `last_ring` was scanned without reaching that point.
+template <bool kIdx>
 __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double* __restrict__ pts, const double (&q)[3], int k,
-                                                 int last_ring, int lane, double* best, double& reg_best, int& found, double& thr,
-                                                 int& pos) {
+                                                 int last_ring, int lane, double* best, int* bidx, double& reg_best, int& reg_idx,
+                                                 int& found, double& thr, int& thr_idx, int& pos, double r2) {
     int c[3];
 #pragma unroll
     for (int ax = 0; ax < 3; ++ax) {
@@ -362,7 +387,7 @@ __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double*
     }
     const int maxring = max(g.dim[0], max(g.dim[1], g.dim[2]));
     for (int ring = 0; ring <= maxring; ++ring) {
-        if (found >= k && ring >= 1) {
+        if ((found >= k || (kIdx && r2 < INFINITY)) && ring >= 1) {
             // distance from q to the nearest face of the already scanned box that still has grid behind it
             double reach = 1e300;
 #pragma unroll
@@ -372,7 +397,9 @@ __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double*
             }
             if (reach == 1e300) return true;           // the box covers the whole grid
             reach -= 1e-9 * g.cell;                    // conservative against rounding of the cell boundaries
-            if (reach > 0.0 && reach * reach > thr) return true;
+            // strictly beyond the k-th: an unscanned point cannot tie with it (kIdx: a tie with a lower index would enter)
+            if (found >= k && reach > 0.0 && reach * reach > thr) return true;
+            if (kIdx && reach > 0.0 && reach * reach >= r2) return true;
         }
         if (ring > last_ring) return false;
         // enumerate the shell cells of this ring, 32 at a time (one hash lookup per lane)
@@ -417,15 +444,17 @@ __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double*
                 for (int j0 = b; j0 < e; j0 += 32) {
                     const int j = j0 + lane;
                     double d2 = 0.0;
+                    int pidx = 0;
                     bool cand = false;
                     if (j < e) {
-                        const size_t pi = (size_t)g.idx[j];
+                        pidx = g.idx[j];
+                        const size_t pi = (size_t)pidx;
                         const double dx = __dsub_rn(q[0], pts[3 * pi]), dy = __dsub_rn(q[1], pts[3 * pi + 1]),
                                      dz = __dsub_rn(q[2], pts[3 * pi + 2]);
                         d2 = __dadd_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)), __dmul_rn(dz, dz));
-                        cand = true;
+                        cand = !kIdx || d2 < r2;
                     }
-                    unsigned todo = __ballot_sync(0xffffffffu, cand && (found < k || d2 < thr));
+                    unsigned todo = __ballot_sync(0xffffffffu, cand && (found < k || (kIdx ? pair_less(d2, pidx, thr, thr_idx) : d2 < thr)));
                     if (k <= 32) {
                         // k best kept sorted ascending, one per lane (lanes >= found hold +inf): an insert is a
                         // ballot (rank of the newcomer), one shuffle (shift the tail up) and a select
@@ -433,21 +462,46 @@ __device__ __forceinline__ bool knn_search_level(const KnnGrid& g, const double*
                             const int L = __ffs(todo) - 1;
                             todo &= todo - 1;
                             const double d = __shfl_sync(0xffffffffu, d2, L);
-                            if (found == k && !(d < thr)) continue;                      // warp-uniform
-                            const int rank = __popc(__ballot_sync(0xffffffffu, reg_best <= d));   // ties: after its equals
-                            const double up = __shfl_up_sync(0xffffffffu, reg_best, 1);
-                            if (lane == rank) reg_best = d;
-                            else if (lane > rank) reg_best = up;
-                            if (found < k) ++found;
-                            if (lane >= k) reg_best = INFINITY;
-                            if (found == k) thr = __shfl_sync(0xffffffffu, reg_best, k - 1);
+                            if (kIdx) {
+                                const int di = __shfl_sync(0xffffffffu, pidx, L);
+                                if (found == k && !pair_less(d, di, thr, thr_idx)) continue;             // warp-uniform
+                                const int rank = __popc(__ballot_sync(0xffffffffu, pair_less(reg_best, reg_idx, d, di)));
+                                const double up = __shfl_up_sync(0xffffffffu, reg_best, 1);
+                                const int upi = __shfl_up_sync(0xffffffffu, reg_idx, 1);
+                                if (lane == rank) { reg_best = d; reg_idx = di; }
+                                else if (lane > rank) { reg_best = up; reg_idx = upi; }
+                                if (found < k) ++found;
+                                if (lane >= k) { reg_best = INFINITY; reg_idx = 0x7fffffff; }
+                                if (found == k) { thr = __shfl_sync(0xffffffffu, reg_best, k - 1); thr_idx = __shfl_sync(0xffffffffu, reg_idx, k - 1); }
+                            } else {
+                                if (found == k && !(d < thr)) continue;                      // warp-uniform
+                                const int rank = __popc(__ballot_sync(0xffffffffu, reg_best <= d));   // ties: after its equals
+                                const double up = __shfl_up_sync(0xffffffffu, reg_best, 1);
+                                if (lane == rank) reg_best = d;
+                                else if (lane > rank) reg_best = up;
+                                if (found < k) ++found;
+                                if (lane >= k) reg_best = INFINITY;
+                                if (found == k) thr = __shfl_sync(0xffffffffu, reg_best, k - 1);
+                            }
                         }
                     } else {
                         while (todo) {
                             const int L = __ffs(todo) - 1;
                             todo &= todo - 1;
                             const double d = __shfl_sync(0xffffffffu, d2, L);
-                            if (found < k) {
+                            if (kIdx) {
+                                const int di = __shfl_sync(0xffffffffu, pidx, L);
+                                if (found < k) {
+                                    if (lane == 0) { best[found] = d; bidx[found] = di; }
+                                    ++found;
+                                    __syncwarp();
+                                    if (found == k) warp_argmax_idx(best, bidx, k, lane, thr, thr_idx, pos);
+                                } else if (pair_less(d, di, thr, thr_idx)) {
+                                    if (lane == 0) { best[pos] = d; bidx[pos] = di; }
+                                    __syncwarp();
+                                    warp_argmax_idx(best, bidx, k, lane, thr, thr_idx, pos);
+                                }
+                            } else if (found < k) {
                                 if (lane == 0) best[found] = d;
                                 ++found;
                                 __syncwarp();
@@ -481,6 +535,7 @@ __global__ void __launch_bounds__(kKnnWarps * 32) knn_mean_dist_kernel(KnnArgs a
     double thr = 0.0;   // current k-th best (valid when found == k)
     int pos = 0;
     double reg_best = INFINITY;                    // k <= 32: the sorted k best, one per lane
+    int reg_idx = 0, thr_idx = 0;                  // unused without the index (kIdx = false)
     // one copy of the search code for the three levels (three inlined copies thrashed the instruction cache:
     // ncu showed no_instruction stalls of 2 warps per issue slot)
     bool done = false;
@@ -489,7 +544,8 @@ __global__ void __launch_bounds__(kKnnWarps * 32) knn_mean_dist_kernel(KnnArgs a
         const int last = level == 0 ? a.fine_rings : (level == 1 ? a.coarse_rings : 0x3fffffff);
         found = 0; thr = 0.0; pos = 0; reg_best = INFINITY;    // a coarser level's buckets contain the finer level's finds again
         __syncwarp();
-        done = knn_search_level(a.lv[level], a.pts, q, k, last, lane, best, reg_best, found, thr, pos);
+        done = knn_search_level<false>(a.lv[level], a.pts, q, k, last, lane, best, nullptr, reg_best, reg_idx, found, thr, thr_idx, pos,
+                                       INFINITY);
     }
     if (k <= 32 && lane < found) best[lane] = reg_best;
     __syncwarp();
@@ -510,6 +566,144 @@ __global__ void __launch_bounds__(kKnnWarps * 32) knn_mean_dist_kernel(KnnArgs a
         if (a.mode == 1) a.dbar[qi] = found > 0 ? __dsqrt_rn(sorted[0]) : -1.0;
         else a.dbar[qi] = found > 0 ? __ddiv_rn(s, (double)found) : -1.0;
     }
+}
+
+// ---- normal estimation (PointCloud.estimate_normals, DESIGN.md §4 "Normals and point-to-plane registration")
+constexpr int kJacobiSweeps = 16;
+
+// one Jacobi rotation of the symmetric A zeroing A[p][q]; V accumulates the rotations (its columns are the eigenvectors)
+__device__ __forceinline__ void jacobi_rotate(double (&A)[3][3], double (&V)[3][3], int p, int q) {
+    const double apq = A[p][q];
+    if (apq == 0.0) return;
+    const int r = 3 - p - q;
+    const double theta = __ddiv_rn(__dsub_rn(A[q][q], A[p][p]), __dmul_rn(2.0, apq));
+    double t;
+    if (fabs(theta) > 1e150) t = __ddiv_rn(0.5, theta);      // theta^2 would overflow; t = 1 / (2 theta) to working precision
+    else {
+        t = __ddiv_rn(1.0, __dadd_rn(fabs(theta), __dsqrt_rn(__dadd_rn(__dmul_rn(theta, theta), 1.0))));
+        if (theta < 0.0) t = -t;
+    }
+    const double c = __ddiv_rn(1.0, __dsqrt_rn(__dadd_rn(__dmul_rn(t, t), 1.0))), s = __dmul_rn(t, c);
+    const double app = __dsub_rn(A[p][p], __dmul_rn(t, apq)), aqq = __dadd_rn(A[q][q], __dmul_rn(t, apq));
+    const double arp = A[r][p], arq = A[r][q];
+    A[r][p] = A[p][r] = __dsub_rn(__dmul_rn(c, arp), __dmul_rn(s, arq));
+    A[r][q] = A[q][r] = __dadd_rn(__dmul_rn(s, arp), __dmul_rn(c, arq));
+    A[p][p] = app; A[q][q] = aqq; A[p][q] = A[q][p] = 0.0;
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+        const double vp = V[i][p], vq = V[i][q];
+        V[i][p] = __dsub_rn(__dmul_rn(c, vp), __dmul_rn(s, vq));
+        V[i][q] = __dadd_rn(__dmul_rn(s, vp), __dmul_rn(c, vq));
+    }
+}
+
+// unit eigenvector of the smallest eigenvalue of the symmetric C = {c00, c01, c02, c11, c12, c22} with + - * / sqrt only:
+// C scaled by its largest |entry| (a zero matrix gives the zero vector), cyclic Jacobi over (0,1), (0,2), (1,2) until the
+// off-diagonal is exactly zero or kJacobiSweeps sweeps; among equal eigenvalues the highest index (C = I gives (0, 0, 1))
+__device__ void smallest_eigenvector(const double (&C)[6], double (&n)[3]) {
+    double s = 0.0;
+#pragma unroll
+    for (int i = 0; i < 6; ++i) s = fmax(s, fabs(C[i]));
+    if (!(s > 0.0)) { n[0] = n[1] = n[2] = 0.0; return; }
+    const double a00 = __ddiv_rn(C[0], s), a01 = __ddiv_rn(C[1], s), a02 = __ddiv_rn(C[2], s), a11 = __ddiv_rn(C[3], s),
+                 a12 = __ddiv_rn(C[4], s), a22 = __ddiv_rn(C[5], s);
+    double A[3][3] = {{a00, a01, a02}, {a01, a11, a12}, {a02, a12, a22}};
+    double V[3][3] = {{1.0, 0.0, 0.0}, {0.0, 1.0, 0.0}, {0.0, 0.0, 1.0}};
+    for (int sweep = 0; sweep < kJacobiSweeps; ++sweep) {
+        if (A[0][1] == 0.0 && A[0][2] == 0.0 && A[1][2] == 0.0) break;
+        jacobi_rotate(A, V, 0, 1);
+        jacobi_rotate(A, V, 0, 2);
+        jacobi_rotate(A, V, 1, 2);
+    }
+    int m = 0;
+    if (A[1][1] <= A[m][m]) m = 1;
+    if (A[2][2] <= A[m][m]) m = 2;
+    const double x = V[0][m], y = V[1][m], z = V[2][m];
+    const double len = __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(x, x), __dmul_rn(y, y)), __dmul_rn(z, z)));
+    n[0] = __ddiv_rn(x, len); n[1] = __ddiv_rn(y, len); n[2] = __ddiv_rn(z, len);
+}
+
+// one warp per query: the neighbour list in (d2, index) order, Open3D's ComputeCovariance (nine cumulants summed in
+// neighbour order by lanes 0..8, over the count; C = I below 3 neighbours), the smallest eigenvector, then the fallbacks
+// and the sign of Open3D's EstimateNormals
+__global__ void __launch_bounds__(kKnnWarps * 32) normals_kernel(KnnArgs a, const double* __restrict__ prior, double r2,
+                                                                 double* __restrict__ out) {
+    __shared__ double s_best[kKnnWarps][kKnnMaxK];
+    __shared__ int s_bidx[kKnnWarps][kKnnMaxK];
+    __shared__ int s_nbr[kKnnWarps][kKnnMaxK];
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    const int64_t qpos = (int64_t)blockIdx.x * kKnnWarps + wid;
+    if (qpos >= a.nq) return;
+    double* best = s_best[wid];
+    int* bidx = s_bidx[wid];
+    int* nbr = s_nbr[wid];
+    const int64_t qi = a.qidx ? (int64_t)a.qidx[qpos] : qpos;
+    const double q[3] = {a.qpts[3 * (size_t)qi], a.qpts[3 * (size_t)qi + 1], a.qpts[3 * (size_t)qi + 2]};
+    const int k = a.k;
+    int found = 0, pos = 0, reg_idx = 0x7fffffff, thr_idx = 0;
+    double thr = 0.0, reg_best = INFINITY;
+    bool done = false;
+#pragma unroll 1
+    for (int level = a.fine_rings > 0 ? 0 : 1; level < 3 && !done; ++level) {
+        const int last = level == 0 ? a.fine_rings : (level == 1 ? a.coarse_rings : 0x3fffffff);
+        found = 0; thr = 0.0; thr_idx = 0; pos = 0; reg_best = INFINITY; reg_idx = 0x7fffffff;
+        __syncwarp();
+        done = knn_search_level<true>(a.lv[level], a.pts, q, k, last, lane, best, bidx, reg_best, reg_idx, found, thr, thr_idx, pos, r2);
+    }
+    if (k <= 32) {
+        if (lane < found) nbr[lane] = reg_idx;
+    } else {
+        __syncwarp();
+        for (int e = lane; e < found; e += 32) {
+            const double v = best[e];
+            const int vi = bidx[e];
+            int rank = 0;
+            for (int i = 0; i < found; ++i) rank += pair_less(best[i], bidx[i], v, vi);
+            nbr[rank] = vi;
+        }
+    }
+    __syncwarp();
+    // lane c < 9 sums cumulant c: x, y, z, xx, xy, xz, yy, yz, zz (nibble c of U / V; V = 0xF: first order)
+    double cum = 0.0;
+    if (lane < 9) {
+        const int u = (int)((0x211000210ull >> (4 * lane)) & 0xF), v = (int)((0x221210FFFull >> (4 * lane)) & 0xF);
+        for (int j = 0; j < found; ++j) {
+            const size_t p = 3 * (size_t)nbr[j];
+            const double x = a.pts[p + u];
+            cum = __dadd_rn(cum, v == 0xF ? x : __dmul_rn(x, a.pts[p + v]));
+        }
+        cum = __ddiv_rn(cum, (double)found);
+    }
+    double m[9];
+#pragma unroll
+    for (int c = 0; c < 9; ++c) m[c] = __shfl_sync(0xffffffffu, cum, c);
+    if (lane != 0) return;
+    double C[6] = {1.0, 0.0, 0.0, 1.0, 0.0, 1.0};
+    if (found >= 3) {
+        C[0] = __dsub_rn(m[3], __dmul_rn(m[0], m[0]));
+        C[1] = __dsub_rn(m[4], __dmul_rn(m[0], m[1]));
+        C[2] = __dsub_rn(m[5], __dmul_rn(m[0], m[2]));
+        C[3] = __dsub_rn(m[6], __dmul_rn(m[1], m[1]));
+        C[4] = __dsub_rn(m[7], __dmul_rn(m[1], m[2]));
+        C[5] = __dsub_rn(m[8], __dmul_rn(m[2], m[2]));
+    }
+    double n[3];
+    smallest_eigenvector(C, n);
+    const double* pr = prior ? prior + 3 * (size_t)qi : nullptr;
+    if (n[0] == 0.0 && n[1] == 0.0 && n[2] == 0.0) {
+        if (pr) { n[0] = pr[0]; n[1] = pr[1]; n[2] = pr[2]; }
+        else { n[2] = 1.0; }
+    } else if (pr) {
+        if (__dadd_rn(__dadd_rn(__dmul_rn(n[0], pr[0]), __dmul_rn(n[1], pr[1])), __dmul_rn(n[2], pr[2])) < 0.0) {
+            n[0] = -n[0]; n[1] = -n[1]; n[2] = -n[2];
+        }
+    } else {
+        int b = 0;
+        if (fabs(n[1]) > fabs(n[b])) b = 1;
+        if (fabs(n[2]) > fabs(n[b])) b = 2;
+        if (n[b] < 0.0) { n[0] = -n[0]; n[1] = -n[1]; n[2] = -n[2]; }
+    }
+    out[3 * (size_t)qi] = n[0]; out[3 * (size_t)qi + 1] = n[1]; out[3 * (size_t)qi + 2] = n[2];
 }
 
 // sum over buckets of size^2: sum / n = the number of points sharing a cell with a typical point
@@ -793,17 +987,14 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
 // strictly closer than `radius` (KDTree SearchHybrid(point, radius, 1)), or -1.  The radius bounds the search, so a uniform
 // grid with cell = radius needs the 27 cells around the query only: one thread per query, exact FP64 squared distances in
 // the (dx^2 + dy^2) + dz^2 order, ties broken towards the lower target index (deterministic).
-__global__ void __launch_bounds__(128) nn_within_kernel(KnnGrid g, const double* __restrict__ pts, const double* __restrict__ qpts,
-                                                        int64_t nq, double r2, int32_t* __restrict__ out_idx, double* __restrict__ out_d2) {
-    const int64_t qi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (qi >= nq) return;
-    const double q[3] = {qpts[3 * qi], qpts[3 * qi + 1], qpts[3 * qi + 2]};
+__device__ __forceinline__ void nn_within_search(const KnnGrid& g, const double* __restrict__ pts, const double (&q)[3], double r2,
+                                                 int& bi, double& best) {
     int c[3];
 #pragma unroll
     for (int ax = 0; ax < 3; ++ax)      // may lie outside the grid: clamp to one cell beyond it (still "no cell in range")
         c[ax] = (int)fmin(fmax(floor(__ddiv_rn(__dsub_rn(q[ax], g.mn[ax]), g.cell)), -2.0), (double)g.dim[ax] + 1.0);
-    double best = r2;
-    int bi = -1;
+    best = r2;
+    bi = -1;
     for (int dz = -1; dz <= 1; ++dz)
         for (int dy = -1; dy <= 1; ++dy)
             for (int dx = -1; dx <= 1; ++dx) {
@@ -819,9 +1010,91 @@ __global__ void __launch_bounds__(128) nn_within_kernel(KnnGrid g, const double*
                     if (d2 < best || (d2 == best && bi >= 0 && pi < bi)) { best = d2; bi = pi; }
                 }
             }
+}
+
+__global__ void __launch_bounds__(128) nn_within_kernel(KnnGrid g, const double* __restrict__ pts, const double* __restrict__ qpts,
+                                                        int64_t nq, double r2, int32_t* __restrict__ out_idx, double* __restrict__ out_d2) {
+    const int64_t qi = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (qi >= nq) return;
+    const double q[3] = {qpts[3 * qi], qpts[3 * qi + 1], qpts[3 * qi + 2]};
+    int bi;
+    double best;
+    nn_within_search(g, pts, q, r2, bi, best);
     out_idx[qi] = bi;
     if (out_d2) out_d2[qi] = bi >= 0 ? best : -1.0;
 }
+
+// ---- point-to-plane ICP (o3d.pipelines.registration.registration_icp with TransformationEstimationPointToPlane)
+constexpr int kIcpThreads = 128;        // source points per CTA
+constexpr int kIcpTerms = 30;           // 21 JtJ (upper triangle, row-major), 6 Jtr, r^2, inliers, Euclidean d^2 of the match
+constexpr int kIcpSumThreads = 256;
+
+// one thread per source point at the current pose: its correspondence (nn_within_kernel's rule), r = n.(s - t) and
+// J = [s x n, n] with the target's normal n, and the CTA's sum of the 30 terms by a fixed halving tree in source order
+__global__ void __launch_bounds__(kIcpThreads) icp_assoc_kernel(KnnGrid g, const double* __restrict__ tgt, const double* __restrict__ tn,
+                                                                int has_target, const double* __restrict__ src, int64_t n, double r2,
+                                                                int32_t* __restrict__ corr, double* __restrict__ partials, int P) {
+    __shared__ double sm[kIcpTerms][kIcpThreads];
+    const int lane = threadIdx.x;
+    const int64_t i = (int64_t)blockIdx.x * kIcpThreads + lane;
+    bool matched = false;
+    if (i < n) {
+        const double p[3] = {src[3 * i], src[3 * i + 1], src[3 * i + 2]};
+        int bi = -1;
+        double d2 = 0.0;
+        if (has_target) nn_within_search(g, tgt, p, r2, bi, d2);
+        corr[i] = bi;
+        if (bi >= 0) {
+            const size_t m = 3 * (size_t)bi;
+            const double N[3] = {tn[m], tn[m + 1], tn[m + 2]};
+            const double r = __dadd_rn(__dadd_rn(__dmul_rn(__dsub_rn(p[0], tgt[m]), N[0]), __dmul_rn(__dsub_rn(p[1], tgt[m + 1]), N[1])),
+                                       __dmul_rn(__dsub_rn(p[2], tgt[m + 2]), N[2]));
+            const double J[6] = {__dsub_rn(__dmul_rn(p[1], N[2]), __dmul_rn(p[2], N[1])), __dsub_rn(__dmul_rn(p[2], N[0]), __dmul_rn(p[0], N[2])),
+                                 __dsub_rn(__dmul_rn(p[0], N[1]), __dmul_rn(p[1], N[0])), N[0], N[1], N[2]};
+            int k = 0;
+#pragma unroll
+            for (int a = 0; a < 6; ++a)
+#pragma unroll
+                for (int b = a; b < 6; ++b) sm[k++][lane] = __dmul_rn(J[a], J[b]);
+#pragma unroll
+            for (int a = 0; a < 6; ++a) sm[21 + a][lane] = __dmul_rn(J[a], r);
+            sm[27][lane] = __dmul_rn(r, r);
+            sm[28][lane] = 1.0;
+            sm[29][lane] = d2;
+            matched = true;
+        }
+    }
+    if (!matched)                        // no point or no correspondence: its terms are 0
+#pragma unroll
+        for (int k = 0; k < kIcpTerms; ++k) sm[k][lane] = 0.0;
+    // fixed halving tree: lane i += lane i + 64, then i + 32, ... (absent points hold 0)
+    for (int s = kIcpThreads / 2; s > 0; s >>= 1) {
+        __syncthreads();
+        for (int j = lane; j < kIcpTerms * s; j += kIcpThreads) {
+            const int k = j / s, e = j - k * s;
+            sm[k][e] = __dadd_rn(sm[k][e], sm[k][e + s]);
+        }
+    }
+    __syncthreads();
+    if (lane < kIcpTerms) partials[(size_t)lane * P + blockIdx.x] = sm[lane][0];
+}
+
+// the CTA partials padded with zeros to P = 2^k, summed by a fixed pairwise tree (i += i + P/2, then i + P/4, ...), as
+// track.cu's solve kernel sums its tiles; out[30] = the totals
+__global__ void __launch_bounds__(kIcpSumThreads) icp_sum_kernel(double* __restrict__ buf, int n_cta, int P, double* __restrict__ out) {
+    for (int h = P / 2; h > 0; h >>= 1) {
+        for (int j = threadIdx.x; j < kIcpTerms * h; j += kIcpSumThreads) {
+            const int k = j / h, i = j - k * h;
+            const double x = i < n_cta ? buf[(size_t)k * P + i] : 0.0;
+            const double y = i + h < n_cta ? buf[(size_t)k * P + i + h] : 0.0;
+            buf[(size_t)k * P + i] = __dadd_rn(x, y);
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x < kIcpTerms) out[threadIdx.x] = buf[(size_t)threadIdx.x * P];
+}
+
+int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s);
 
 int otslam_cloud_nn_within(const double* source, int64_t n_source, const double* target, int64_t n_target, double radius,
                            int32_t* out_index, double* out_dist2, int device) {
@@ -878,6 +1151,125 @@ int otslam_cloud_nn_distance(const double* source, int64_t n_source, const doubl
     OT_LAUNCHED();
     timer.stop();
     OT_CUDA(cudaMemcpy(out_dist, dout.p, n_source * 8, cudaMemcpyDefault));
+    return OTSLAM_OK;
+}
+
+int otslam_cloud_estimate_normals(const double* points, int64_t n, const double* prior_normals, double radius, int max_nn,
+                                  double* out_normals, int device) {
+    // ---- every argument is checked before any CUDA call
+    if (n < 0) return set_error(OTSLAM_ERR_INVALID, "estimate_normals: n < 0");
+    if (n > 0x7fffffffLL) return set_error(OTSLAM_ERR_INVALID, "estimate_normals: more than 2^31 - 1 points");
+    if (n && (!points || !out_normals)) return set_error(OTSLAM_ERR_INVALID, "estimate_normals: null points or out_normals");
+    if (max_nn < 1 || max_nn > kKnnMaxK) return set_error(OTSLAM_ERR_INVALID, "estimate_normals: max_nn must be in 1..128");
+    if (!(radius > 0.0)) return set_error(OTSLAM_ERR_INVALID, "estimate_normals: radius must be > 0 (finite, or +inf for a k-NN search)");
+    if (n == 0) return OTSLAM_OK;
+    OT_TRY(use_device(device));
+    DevBuf<double> dp, dprior, dout;
+    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(dout.alloc(n * 3));
+    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
+    if (prior_normals) { OT_CUDA(dprior.alloc(n * 3)); OT_CUDA(cudaMemcpy(dprior.p, prior_normals, n * 24, cudaMemcpyDefault)); }
+    OpTimer timer;
+    KnnArgs a;
+    GridBuffers bc, bf, bt;
+    OT_TRY(build_search(dp.p, n, bc, bf, bt, a));
+    a.pts = dp.p; a.qpts = dp.p; a.qidx = a.fine_rings ? a.lv[0].idx : a.lv[1].idx;   // visit queries cell by cell
+    a.nq = n; a.mode = 0; a.n = n; a.k = (int)std::min<int64_t>(max_nn, n); a.dbar = nullptr;
+    normals_kernel<<<(unsigned)((n + kKnnWarps - 1) / kKnnWarps), kKnnWarps * 32>>>(a, prior_normals ? dprior.p : nullptr,
+                                                                                    radius * radius, dout.p);
+    OT_LAUNCHED();
+    timer.stop();
+    OT_CUDA(cudaMemcpy(out_normals, dout.p, n * 24, cudaMemcpyDefault));
+    return OTSLAM_OK;
+}
+
+int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, const double* target, const double* target_normals,
+                                    int64_t n_target, double max_distance, const double init[16], double relative_fitness,
+                                    double relative_rmse, int max_iteration, double transform_out[16], double* fitness,
+                                    double* inlier_rmse, int32_t* iterations, int32_t* corr_index, int device) {
+    // ---- every argument is checked before any CUDA call
+    if (n_source < 0 || n_target < 0) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: negative point count");
+    if (n_source > 0x7fffffffLL || n_target > 0x7fffffffLL)
+        return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: more than 2^31 - 1 points");
+    if (n_source && !source) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: null source");
+    if (n_target && (!target || !target_normals)) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: null target or target_normals");
+    if (!init || !transform_out) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: null init or transform_out");
+    if (!(max_distance > 0.0) || !std::isfinite(max_distance))
+        return set_error(OTSLAM_ERR_INVALID, "[RegistrationICP] Invalid max_correspondence_distance.");
+    for (int k = 0; k < 16; ++k)
+        if (!std::isfinite(init[k])) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: init is not finite");
+    if (!(relative_fitness >= 0.0) || !(relative_rmse >= 0.0))
+        return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: relative_fitness and relative_rmse must be >= 0");
+    if (max_iteration < 0) return set_error(OTSLAM_ERR_INVALID, "icp_point_to_plane: max_iteration < 0");
+    double T[16];
+    for (int k = 0; k < 16; ++k) T[k] = init[k];
+    if (n_source == 0) {
+        for (int k = 0; k < 16; ++k) transform_out[k] = T[k];
+        if (fitness) *fitness = 0.0;
+        if (inlier_rmse) *inlier_rmse = 0.0;
+        if (iterations) *iterations = 0;
+        return OTSLAM_OK;
+    }
+    OT_TRY(use_device(device));
+    const int64_t n = n_source;
+    const int n_cta = (int)((n + kIcpThreads - 1) / kIcpThreads);
+    int P = 1;
+    while (P < n_cta) P *= 2;
+    DevBuf<double> ds0, ds1, dt, dtn, dpart, dsum;
+    DevBuf<int32_t> dcorr;
+    OT_CUDA(ds0.alloc(n * 3)); OT_CUDA(ds1.alloc(n * 3)); OT_CUDA(dcorr.alloc(n));
+    OT_CUDA(dpart.alloc((size_t)kIcpTerms * P)); OT_CUDA(dsum.alloc(kIcpTerms));
+    OT_CUDA(cudaMemcpy(ds0.p, source, n * 24, cudaMemcpyDefault));
+    if (n_target) {
+        OT_CUDA(dt.alloc(n_target * 3)); OT_CUDA(dtn.alloc(n_target * 3));
+        OT_CUDA(cudaMemcpy(dt.p, target, n_target * 24, cudaMemcpyDefault));
+        OT_CUDA(cudaMemcpy(dtn.p, target_normals, n_target * 24, cudaMemcpyDefault));
+    }
+    OpTimer timer;
+    // the target's grid once per call, cell = max_distance (otslam_cloud_nn_within's)
+    KnnGrid g = {};
+    GridBuffers b;
+    if (n_target) {
+        double mn[3], mx[3];
+        OT_TRY(cloud_minmax(dt.p, n_target, mn, mx));
+        OT_TRY(build_grid(dt.p, n_target, mn, mx, max_distance, 1 << 20, b, g));
+    }
+    const double r2 = max_distance * max_distance;
+    double* cur = ds1.p;
+    double* other = ds0.p;
+    OT_TRY(device_rigid_transform(ds0.p, n, T, ds1.p, 0));
+    double S[kIcpTerms];
+    auto evaluate = [&](double& fit, double& rmse) -> int {
+        icp_assoc_kernel<<<n_cta, kIcpThreads>>>(g, dt.p, dtn.p, n_target > 0, cur, n, r2, dcorr.p, dpart.p, P);
+        OT_LAUNCHED();
+        icp_sum_kernel<<<1, kIcpSumThreads>>>(dpart.p, n_cta, P, dsum.p);
+        OT_LAUNCHED();
+        OT_CUDA(cudaMemcpy(S, dsum.p, sizeof(S), cudaMemcpyDeviceToHost));
+        fit = S[28] / (double)n;
+        rmse = S[28] > 0.0 ? std::sqrt(S[29] / S[28]) : 0.0;
+        return OTSLAM_OK;
+    };
+    double fit = 0.0, rmse = 0.0;
+    OT_TRY(evaluate(fit, rmse));
+    int it = 0;
+    while (it < max_iteration) {
+        // RegistrationICP: update = the solve's transform, or the identity when it fails or there is no correspondence
+        double U[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1}, xi[6], Tn[16];
+        if (S[28] > 0.0 && solve6(S, xi)) euler_update(xi, U);
+        matmul4(U, T, Tn);
+        for (int k = 0; k < 16; ++k) T[k] = Tn[k];
+        OT_TRY(device_rigid_transform(cur, n, U, other, 0));
+        std::swap(cur, other);
+        const double fit0 = fit, rmse0 = rmse;
+        OT_TRY(evaluate(fit, rmse));
+        ++it;
+        if (std::fabs(fit0 - fit) < relative_fitness && std::fabs(rmse0 - rmse) < relative_rmse) break;
+    }
+    timer.stop();
+    if (corr_index) OT_CUDA(cudaMemcpy(corr_index, dcorr.p, n * 4, cudaMemcpyDefault));
+    for (int k = 0; k < 16; ++k) transform_out[k] = T[k];
+    if (fitness) *fitness = fit;
+    if (inlier_rmse) *inlier_rmse = rmse;
+    if (iterations) *iterations = it;
     return OTSLAM_OK;
 }
 

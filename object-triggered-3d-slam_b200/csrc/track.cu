@@ -20,6 +20,7 @@
 #include <cmath>
 #include <vector>
 
+#include "icp_solve.h"
 #include "raycast.cuh"
 
 namespace otslam {
@@ -30,7 +31,6 @@ constexpr int kTileW = 16, kTileH = 8, kTilePx = kTileW * kTileH;
 constexpr int kTerms = 30;                          // 21 JtJ (upper triangle, row-major), 6 Jtr, r^2, inliers, valid pixels
 constexpr int kSolveThreads = 256;
 constexpr double kMinInliers = 64.0;
-constexpr double kPivotRel = 1e-10;
 constexpr double kConverged = 1e-6;                 // max |xi_i| (radians, metres) of a converged step
 constexpr double kStalled = 1e-5;                   // ... or a step this small that is not smaller than the one before
 constexpr int kMaxLevels = 4;                       // pyramid levels, 0 = full resolution
@@ -162,41 +162,6 @@ __global__ void __launch_bounds__(kTilePx) track_assoc_kernel(const TrackArgs a,
     }
     __syncthreads();
     if (lane < kTerms) a.partials[((size_t)blockIdx.z * kTerms + lane) * a.P + blockIdx.y * a.tiles_x + blockIdx.x] = sm[lane][0];
-}
-
-// Cholesky solve of A xi = -b (A from the 21 upper-triangle sums); false when a pivot is <= kPivotRel * max diag(A)
-__device__ bool solve6(const double* S, double xi[6]) {
-    double A[6][6], L[6][6], y[6];
-    int k = 0;
-    for (int i = 0; i < 6; ++i)
-        for (int j = i; j < 6; ++j) { A[i][j] = S[k]; A[j][i] = S[k]; ++k; }
-    double maxd = A[0][0];
-    for (int i = 1; i < 6; ++i)
-        if (A[i][i] > maxd) maxd = A[i][i];
-    const double thr = dm(kPivotRel, maxd);
-    for (int j = 0; j < 6; ++j) {
-        double s = A[j][j];
-        for (int c = 0; c < j; ++c) s = ds(s, dm(L[j][c], L[j][c]));
-        if (!(s > thr)) return false;
-        L[j][j] = __dsqrt_rn(s);
-        for (int i = j + 1; i < 6; ++i) {
-            double w = A[i][j];
-            for (int c = 0; c < j; ++c) w = ds(w, dm(L[i][c], L[j][c]));
-            L[i][j] = __ddiv_rn(w, L[j][j]);
-        }
-    }
-    for (int i = 0; i < 6; ++i) {
-        double w = S[21 + i];
-        for (int c = 0; c < i; ++c) w = ds(w, dm(L[i][c], y[c]));
-        y[i] = __ddiv_rn(w, L[i][i]);
-    }
-    for (int i = 5; i >= 0; --i) {
-        double w = y[i];
-        for (int c = i + 1; c < 6; ++c) w = ds(w, dm(L[c][i], xi[c]));
-        xi[i] = __ddiv_rn(w, L[i][i]);
-    }
-    for (int i = 0; i < 6; ++i) xi[i] = -xi[i];
-    return true;
 }
 
 __global__ void __launch_bounds__(kSolveThreads) track_solve_kernel(const TrackArgs a, int it, int max_it, int report) {

@@ -309,6 +309,78 @@ class PointCloud:
         idx = idx[:m.value].copy()
         return self.select_by_index(idx), idx.tolist()
 
+    # ---- normals: PointCloud.estimate_normals and the orientation helpers (DESIGN.md §4 "Normals and point-to-plane
+    # registration"); the normals registration_icp(..., TransformationEstimationPointToPlane()) needs on its target
+    def estimate_normals(self, search_param=None, fast_normal_computation=True):
+        """Normals from the covariance of each point's neighbours (search_param: KDTreeSearchParamKNN (default, 30
+        neighbours) or KDTreeSearchParamHybrid).  A cloud that already has normals orients the new ones along them; one
+        without gets the sign that makes the largest-magnitude component positive.  fast_normal_computation is accepted
+        for compatibility: there is one eigen solver."""
+        radius, max_nn = (search_param or KDTreeSearchParamKNN())._radius_max_nn()
+        n = len(self._points)
+        prior = self._normals if self.has_normals() else None
+        out = np.empty((n, 3), np.float64)
+        _lib.check(_lib.lib.otslam_cloud_estimate_normals(_lib.ptr(self._points), n, _lib.ptr(prior), radius, max_nn, _lib.ptr(out), 0))
+        self._normals = out
+
+    def _require_normals(self):
+        if not self.has_normals():
+            raise RuntimeError("No normals in the PointCloud. Call EstimateNormals() first.")
+
+    def orient_normals_to_align_with_direction(self, orientation_reference=(0.0, 0.0, 1.0)):
+        """Open3D's rule: a zero normal becomes the reference, one with n . reference < 0 is flipped."""
+        self._require_normals()
+        ref = np.asarray(orientation_reference, np.float64).reshape(3)
+        nrm = self._normals.copy()
+        zero = np.linalg.norm(nrm, axis=1) == 0.0
+        flip = ~zero & ((nrm @ ref) < 0.0)
+        nrm[flip] *= -1.0
+        nrm[zero] = ref
+        self._normals = nrm
+
+    def orient_normals_towards_camera_location(self, camera_location=(0.0, 0.0, 0.0)):
+        """Open3D's rule with reference = camera_location - point: a zero normal becomes the normalised reference ((0, 0,
+        1) when that is zero too), one with n . reference < 0 is flipped."""
+        self._require_normals()
+        ref = np.asarray(camera_location, np.float64).reshape(1, 3) - self._points
+        nrm = self._normals.copy()
+        zero = np.linalg.norm(nrm, axis=1) == 0.0
+        flip = ~zero & (np.einsum("ij,ij->i", nrm, ref) < 0.0)
+        nrm[flip] *= -1.0
+        rlen = np.linalg.norm(ref, axis=1)
+        nrm[zero & (rlen > 0.0)] = ref[zero & (rlen > 0.0)] / rlen[zero & (rlen > 0.0), None]
+        nrm[zero & (rlen == 0.0)] = (0.0, 0.0, 1.0)
+        self._normals = nrm
+
+
+_MAX_NN = 128          # neighbours a normal estimation may keep (otslam_cloud_estimate_normals)
+
+
+class KDTreeSearchParamKNN:
+    """The knn nearest neighbours (1..128)."""
+
+    def __init__(self, knn=30):
+        self.knn = int(knn)
+
+    def _radius_max_nn(self):
+        return float("inf"), self.knn
+
+
+class KDTreeSearchParamHybrid:
+    """At most max_nn (1..128) nearest neighbours strictly within radius."""
+
+    def __init__(self, radius, max_nn):
+        self.radius, self.max_nn = float(radius), int(max_nn)
+
+    def _radius_max_nn(self):
+        return self.radius, self.max_nn
+
+
+class KDTreeSearchParamRadius:
+    def __init__(self, radius):
+        raise RuntimeError(f"KDTreeSearchParamRadius (an unbounded neighbour count) is not supported: normal estimation keeps at "
+                           f"most {_MAX_NN} neighbours; use KDTreeSearchParamHybrid(radius, max_nn) with max_nn <= {_MAX_NN}")
+
 
 class _ResidentArray:
     """Stand-in for a mesh array that still lives in HBM (what Open3D exposes as a Vector3dVector):
@@ -452,4 +524,5 @@ class TriangleMesh:
         return TriangleMesh()
 
 
-__all__ = ["Image", "RGBDImage", "PointCloud", "TriangleMesh", "Vector3dVector", "Vector3iVector"]
+__all__ = ["Image", "RGBDImage", "PointCloud", "TriangleMesh", "Vector3dVector", "Vector3iVector", "KDTreeSearchParamKNN",
+           "KDTreeSearchParamHybrid", "KDTreeSearchParamRadius"]

@@ -1,4 +1,5 @@
 """o3d.pipelines.integration: ScalableTSDFVolume on the GPU (reconstruct_rgbd.py:79-83,107,112)."""
+import ctypes as C
 import enum
 import os
 import types
@@ -165,6 +166,16 @@ class TransformationEstimationPointToPoint:
         return T
 
 
+class TransformationEstimationPointToPlane:
+    """Point-to-plane estimation: registration_icp runs the whole loop on the GPU in one call
+    (otslam_cloud_icp_point_to_plane); the target needs normals (PointCloud.estimate_normals)."""
+
+    def __init__(self, kernel=None):
+        if kernel is not None:
+            raise RuntimeError("TransformationEstimationPointToPlane(kernel=...): robust kernels are not supported")
+        self.kernel = None
+
+
 class ICPConvergenceCriteria:
     def __init__(self, relative_fitness=1e-6, relative_rmse=1e-6, max_iteration=30):
         self.relative_fitness, self.relative_rmse, self.max_iteration = float(relative_fitness), float(relative_rmse), int(max_iteration)
@@ -208,13 +219,16 @@ def evaluate_registration(source, target, max_correspondence_distance, transform
 
 
 def registration_icp(source, target, max_correspondence_distance, init=None, estimation_method=None, criteria=None):
-    """registration_icp(source, target, threshold, init, TransformationEstimationPointToPoint(), ICPConvergenceCriteria(...))."""
+    """registration_icp(source, target, threshold, init, TransformationEstimationPointToPoint() or
+    TransformationEstimationPointToPlane(), ICPConvergenceCriteria(...))."""
     estimation_method = estimation_method or TransformationEstimationPointToPoint()
     criteria = criteria or ICPConvergenceCriteria()
-    if not isinstance(estimation_method, TransformationEstimationPointToPoint):
-        raise RuntimeError("only TransformationEstimationPointToPoint is supported")
+    if not isinstance(estimation_method, (TransformationEstimationPointToPoint, TransformationEstimationPointToPlane)):
+        raise RuntimeError("only TransformationEstimationPointToPoint and TransformationEstimationPointToPlane are supported")
     if max_correspondence_distance <= 0:
         raise RuntimeError("[RegistrationICP] Invalid max_correspondence_distance.")
+    if isinstance(estimation_method, TransformationEstimationPointToPlane):
+        return _registration_icp_point_to_plane(source, target, max_correspondence_distance, init, criteria)
     T = np.eye(4) if init is None else np.array(init, np.float64)
     tgt = np.ascontiguousarray(np.asarray(target.points), np.float64)
     pcd = geometry.PointCloud(np.asarray(source.points))
@@ -245,6 +259,30 @@ def registration_icp(source, target, max_correspondence_distance, init=None, est
     return result
 
 
+def _registration_icp_point_to_plane(source, target, max_correspondence_distance, init, criteria):
+    if not target.has_normals():
+        raise RuntimeError("TransformationEstimationPointToPlane and TransformationEstimationColoredICP "
+                           "require pre-computed normal vectors for target PointCloud.")
+    src = np.ascontiguousarray(np.asarray(source.points), np.float64)
+    tgt = np.ascontiguousarray(np.asarray(target.points), np.float64)
+    tn = np.ascontiguousarray(np.asarray(target.normals), np.float64)
+    T0 = np.ascontiguousarray(np.eye(4) if init is None else init, np.float64).reshape(16)
+    T = np.empty(16)
+    fit, rmse, it = C.c_double(), C.c_double(), C.c_int32()
+    corr = np.empty(len(src), np.int32)
+    _lib.check(_lib.lib.otslam_cloud_icp_point_to_plane(
+        _lib.ptr(src), len(src), _lib.ptr(tgt), _lib.ptr(tn), len(tgt), float(max_correspondence_distance), _lib.ptr(T0),
+        criteria.relative_fitness, criteria.relative_rmse, criteria.max_iteration, _lib.ptr(T), C.byref(fit), C.byref(rmse),
+        C.byref(it), _lib.ptr(corr), 0))
+    r = RegistrationResult()
+    r.transformation = T.reshape(4, 4)
+    r.fitness, r.inlier_rmse = fit.value, rmse.value
+    sel = np.nonzero(corr >= 0)[0]
+    r.correspondence_set = np.stack([sel.astype(np.int32), corr[sel]], 1) if len(sel) else np.zeros((0, 2), np.int32)
+    return r
+
+
 registration = types.SimpleNamespace(registration_icp=registration_icp, evaluate_registration=evaluate_registration,
                                      TransformationEstimationPointToPoint=TransformationEstimationPointToPoint,
+                                     TransformationEstimationPointToPlane=TransformationEstimationPointToPlane,
                                      ICPConvergenceCriteria=ICPConvergenceCriteria, RegistrationResult=RegistrationResult)
