@@ -319,6 +319,42 @@ int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, cons
                                     int64_t n_target, double max_distance, const double init[16], double relative_fitness,
                                     double relative_rmse, int max_iteration, double transform_out[16], double* fitness,
                                     double* inlier_rmse, int32_t* iterations, int32_t* corr_index, int device);
+/* PointCloud.cluster_dbscan(eps, min_points) (no reference call site): separates the objects of a cloud.  Rule in DESIGN.md
+ * §4 "Plane segmentation and DBSCAN clustering":
+ *   neighbours of point i = the points j with d2 < eps^2, d2 = (dx^2 + dy^2) + dz^2 in FP64 without FMA (otslam_cloud_nn_within's
+ *     arithmetic), point i itself included;
+ *   core point = at least min_points neighbours; clusters = the connected components of the core points (two core points
+ *     joined when d2 < eps^2), labelled 0, 1, ... in increasing order of their smallest point index;
+ *   a non-core point with a core neighbour takes the smallest label among its core neighbours, any other point -1.
+ * This is what Open3D's ClusterDBSCAN loop computes.  out_labels [n]; *n_clusters (nullable) = the number of clusters.
+ * points and out_labels may be device pointers.  eps finite and > 0, min_points >= 0, 0 <= n < 2^31, non-null points and
+ * out_labels when n > 0: otherwise OTSLAM_ERR_INVALID before any CUDA call.  otslam_last_op_device_ms() = device ms of the
+ * grid build and the kernels.  No neighbour list is stored; when every point lies within eps of every other the cost grows
+ * with n^2 (as Open3D's does). */
+int otslam_cloud_cluster_dbscan(const double* points, int64_t n, double eps, int64_t min_points, int32_t* out_labels, int32_t* n_clusters,
+                                int device);
+/* PointCloud.segment_plane(distance_threshold, ransac_n, num_iterations, probability) (no reference call site): the
+ * dominant plane by RANSAC, Open3D's SegmentPlane run over hypotheses h = 0 .. num_iterations - 1 in order.  Rule in
+ * DESIGN.md §4 "Plane segmentation and DBSCAN clustering":
+ *   sample: r = ransac_n distinct indices by Floyd's algorithm, for k = 0 .. r-1: j = n - r + k,
+ *     t = min(floor(u01(seed, h r + k) (j + 1)), j), j instead when t was drawn already (u01: the mesh sampler's RNG);
+ *   plane: r = 3 Open3D's ComputeTrianglePlane ((p1 - p0) x (p2 - p0) normalised, d = -abc.p0; invalid when the cross
+ *     product is 0), r > 3 GetPlaneFromPoints over the sample in draw order;
+ *   evaluation: dist = |((a x + b y) + c z) + d|, inlier when dist < distance_threshold, fitness = count / n,
+ *     rmse = sum dist / sqrt(count) (0 without inliers), the sum by the fixed tree of DESIGN.md;
+ *   selection: h > B is skipped (B starts unbounded), invalid planes are skipped, a hypothesis replaces the best one when
+ *     its fitness is greater or equal with a strictly smaller rmse; then B = 0 when fitness = 1, else
+ *     q = log(1 - probability) / log(1 - fitness^r) and B = floor(q) when 0 <= q < num_iterations, num_iterations otherwise;
+ *   result: out_inliers [n] = the best hypothesis's inliers ascending (*n_inliers of them), plane_out = GetPlaneFromPoints
+ *     over them (sums by fixed trees); (0, 0, 0, 0) and no inliers without a valid best plane.
+ * *n_evaluated (nullable) = the hypotheses not skipped by B, invalid ones included.  points and out_inliers may be device
+ * pointers; plane_out and the scalars are host pointers.  distance_threshold finite and >= 0, 3 <= ransac_n <= 16,
+ * num_iterations >= 0, 0 < probability <= 1, ransac_n <= n < 2^31: otherwise OTSLAM_ERR_INVALID before any CUDA call
+ * (n < ransac_n: "There must be at least 'ransac_n' points.").  otslam_last_op_device_ms() = device ms of the search and
+ * the refit. */
+int otslam_cloud_segment_plane(const double* points, int64_t n, double distance_threshold, int ransac_n, int num_iterations,
+                               double probability, uint64_t seed, double plane_out[4], int64_t* out_inliers, int64_t* n_inliers,
+                               int32_t* n_evaluated, int device);
 /* create_map_cloud's pixel loop (fusion/hybrid_map.py:45-55); out sized w*h*3 (or NULL to count) */
 int otslam_grid_to_points(const uint8_t* gray, int width, int height, double resolution, double origin_x,
                           double origin_y, int threshold, double* out_points, int64_t* n_out, int device);

@@ -84,6 +84,8 @@ _SIGS = {
     "otslam_cloud_nn_within": (_i, [_vp, _i64, _vp, _i64, _d, _vp, _vp, _i]),
     "otslam_cloud_estimate_normals": (_i, [_vp, _i64, _vp, _d, _i, _vp, _i]),
     "otslam_cloud_icp_point_to_plane": (_i, [_vp, _i64, _vp, _vp, _i64, _d, _vp, _d, _d, _i, _vp, _vp, _vp, _vp, _vp, _i]),
+    "otslam_cloud_cluster_dbscan": (_i, [_vp, _i64, _d, _i64, _vp, _vp, _i]),
+    "otslam_cloud_segment_plane": (_i, [_vp, _i64, _d, _i, _i, _d, _u64, _vp, _vp, _vp, _vp, _i]),
     "otslam_grid_to_points": (_i, [_vp, _i, _i, _d, _d, _d, _i, _vp, C.POINTER(_i64), _i]),
     "otslam_cloud_transform": (_i, [_vp, _vp, _i64, _vp, _vp, _vp, _i]),
     "otslam_cloud_center": (_i, [_vp, _i64, _vp, _i]),

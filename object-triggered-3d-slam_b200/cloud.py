@@ -102,6 +102,41 @@ class DeviceCloud:
         take = lambda t: None if t is None else t.index_select(0, idx)  # noqa: E731
         return DeviceCloud(take(self.points), take(self.colors), take(self.normals)), idx
 
+    def select_by_index(self, idx, invert=False):
+        """The points (colours, normals) at idx, a CUDA or host integer index; invert=True keeps all the others, in order."""
+        import torch
+        idx = torch.as_tensor(idx, dtype=torch.int64, device=self.points.device)
+        if invert:
+            keep = torch.ones(len(self), dtype=torch.bool, device=self.points.device)
+            keep[idx] = False
+            idx = torch.nonzero(keep).flatten()
+        take = lambda t: None if t is None else t.index_select(0, idx)  # noqa: E731
+        return DeviceCloud(take(self.points), take(self.colors), take(self.normals))
+
+    def segment_plane(self, distance_threshold, ransac_n, num_iterations, probability=0.99999999, seed=0):
+        """PointCloud.segment_plane -> (plane as a float64 ndarray [4], inlier indices as a CUDA int64 tensor)."""
+        import torch
+        n = len(self)
+        plane = np.zeros(4, np.float64)
+        idx = torch.empty(n, dtype=torch.int64, device=self.points.device)
+        m = C.c_int64(0)
+        _sync()
+        _lib.check(_lib.lib.otslam_cloud_segment_plane(_lib.ptr(self.points), n, float(distance_threshold), int(ransac_n),
+                                                       int(num_iterations), float(probability), C.c_uint64(int(seed) & 0xFFFFFFFFFFFFFFFF),
+                                                       _lib.ptr(plane), _lib.ptr(idx), C.byref(m), None, self.device_index))
+        _sync()
+        return plane, idx[:m.value]
+
+    def cluster_dbscan(self, eps, min_points):
+        """PointCloud.cluster_dbscan -> labels as a CUDA int32 tensor (-1 = noise)."""
+        import torch
+        labels = torch.empty(len(self), dtype=torch.int32, device=self.points.device)
+        _sync()
+        _lib.check(_lib.lib.otslam_cloud_cluster_dbscan(_lib.ptr(self.points), len(self), float(eps), int(min_points), _lib.ptr(labels),
+                                                        None, self.device_index))
+        _sync()
+        return labels
+
     def to_numpy(self):
         from .slab import to_host
         ts = [t for t in (self.points, self.colors, self.normals) if t is not None]

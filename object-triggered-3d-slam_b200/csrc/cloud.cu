@@ -179,10 +179,6 @@ __global__ void __launch_bounds__(256) tri_area_kernel(const double* __restrict_
 // ---- sequential-order accumulation (surface area, area CDF, outlier-filter statistics): ordered_sum.cu
 int device_ordered_sum(double* d_x, int64_t n, int mode, const double* d_div, double mean, double* d_out, cudaStream_t s);
 
-__device__ __forceinline__ double u01(uint64_t seed, uint64_t ctr) {
-    return __dmul_rn((double)(splitmix64(seed * 0xD1342543DE82EF95ull + ctr) >> 11), 1.0 / 9007199254740992.0);
-}
-
 // triangle t owns samples [end[t-1], end[t]) with end[t] = llround(cdf[t]*n) (last forced to n)
 __global__ void __launch_bounds__(256) sample_kernel(const double* __restrict__ v, const double* __restrict__ col,
                                                      const double* __restrict__ nrm, const int32_t* __restrict__ f, int64_t nf,

@@ -84,6 +84,10 @@ __host__ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
     x = (x ^ (x >> 27)) * 0x94D049BB133111EBull;
     return x ^ (x >> 31);
 }
+// uniform double in [0, 1) from (seed, counter): the mesh sampler's RNG (cloud.cu) and RANSAC's sampling (segment.cu)
+__device__ __forceinline__ double u01(uint64_t seed, uint64_t ctr) {
+    return __dmul_rn((double)(splitmix64(seed * 0xD1342543DE82EF95ull + ctr) >> 11), 1.0 / 9007199254740992.0);
+}
 
 // ---- multi-object arenas (config 3: multi_reconstruct_rgbd_filter.py, several objects, each "its own volume"): the
 // objects share ONE block hash / pool / per-batch work list, so that one integration launch covers the union of their

@@ -18,7 +18,7 @@
 #include <vector>
 
 #include "icp_solve.h"
-#include "volume.cuh"
+#include "knn_grid.cuh"
 
 namespace otslam {
 
@@ -59,7 +59,7 @@ __global__ void __launch_bounds__(256) minmax_kernel(const double* __restrict__ 
     }
 }
 
-static int cloud_minmax(const double* d_pts, int64_t n, double* mn, double* mx) {
+int cloud_minmax(const double* d_pts, int64_t n, double* mn, double* mx) {
     DevBuf<unsigned long long> mm;
     OT_CUDA(mm.alloc(6));
     unsigned long long init[6] = {~0ull, ~0ull, ~0ull, 0, 0, 0};
@@ -72,13 +72,6 @@ static int cloud_minmax(const double* d_pts, int64_t n, double* mn, double* mx) 
     return OTSLAM_OK;
 }
 
-// key = floor((p - origin) / cell) per axis packed as kx << sh_x | ky << sh_y | kz with just enough
-// bits per axis (the host sizes them from the bounding box), so the sort needs few passes and
-// key order == lexicographic (x, y, z)
-struct KeyLayout {
-    int sh_x, sh_y, bits;
-    uint64_t mask_y, mask_z;
-};
 static int nbits_for(double n_cells) {
     int b = 1;
     while (b < 62 && (double)(1ull << b) < n_cells) ++b;
@@ -90,9 +83,6 @@ static KeyLayout make_layout(double nx, double ny, double nz) {
     L.sh_y = bz; L.sh_x = by + bz; L.bits = bx + by + bz;
     L.mask_y = (1ull << by) - 1; L.mask_z = (1ull << bz) - 1;
     return L;
-}
-__host__ __device__ inline uint64_t layout_key(const KeyLayout& L, int x, int y, int z) {
-    return ((uint64_t)(uint32_t)x << L.sh_x) | ((uint64_t)(uint32_t)y << L.sh_y) | (uint64_t)(uint32_t)z;
 }
 
 __global__ void __launch_bounds__(256) cell_key_kernel(const double* __restrict__ pts, int64_t n, double ox, double oy, double oz,
@@ -295,15 +285,6 @@ __global__ void __launch_bounds__(256) cell_hash_build_kernel(const uint64_t* __
     if (m < n_seg) hash_insert_absent(t, sorted_keys[seg_start[m]], (int32_t)m);
 }
 
-// one level of the search structure: points bucketed by uniform-grid cell (sorted by cell key), cell -> bucket hash
-struct KnnGrid {
-    const int32_t* idx;         // sorted position -> original index
-    const int32_t* seg_start;   // [n_seg+1]
-    HashTable cells;            // cell key -> segment id
-    double mn[3], cell;
-    int dim[3];
-    KeyLayout L;
-};
 
 // Two levels.  Scanned clouds are surfaces: a grid sized for ~2 points per cell of the bounding-box VOLUME
 // puts hundreds of points into every occupied cell (1 M points on a table: ~200), and each query then
@@ -755,19 +736,13 @@ static int upload_shell_table() {
     return OTSLAM_OK;
 }
 
-// ---- host side of the search structure
-struct GridBuffers {
-    DevBuf<uint64_t> k0, k1, hk;
-    DevBuf<int32_t> i0, i1, seg, hv;
-    int64_t n_seg = 0;
-};
 
 static int sort_pairs(DevBuf<uint64_t>& k_in, DevBuf<int32_t>& v_in, DevBuf<uint64_t>& k_out, DevBuf<int32_t>& v_out, int64_t n, int bits);
 static int find_segments(const uint64_t* d_keys, int64_t n, DevBuf<int32_t>& seg_start, int64_t* n_seg);
 
 // bucket the n points of d_pts on a grid of `cell`-sized cells over [mn, mx] (at most max_dim cells per axis)
-static int build_grid(const double* d_pts, int64_t n, const double mn[3], const double mx[3], double cell, int max_dim, GridBuffers& b,
-                      KnnGrid& g) {
+int build_grid(const double* d_pts, int64_t n, const double mn[3], const double mx[3], double cell, int max_dim, GridBuffers& b,
+               KnnGrid& g) {
     const double ext[3] = {mx[0] - mn[0], mx[1] - mn[1], mx[2] - mn[2]};
     const double maxext = std::max(ext[0], std::max(ext[1], ext[2]));
     cell = std::max(cell, maxext / (double)max_dim);
@@ -982,35 +957,6 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
     return OTSLAM_OK;
 }
 
-// ---- correspondence search of point-to-point ICP (o3d.pipelines.registration.registration_icp,
-// /root/reference/eval/eval_table_chair/eval_table_chair.py:90-104): for every source point the nearest target point
-// strictly closer than `radius` (KDTree SearchHybrid(point, radius, 1)), or -1.  The radius bounds the search, so a uniform
-// grid with cell = radius needs the 27 cells around the query only: one thread per query, exact FP64 squared distances in
-// the (dx^2 + dy^2) + dz^2 order, ties broken towards the lower target index (deterministic).
-__device__ __forceinline__ void nn_within_search(const KnnGrid& g, const double* __restrict__ pts, const double (&q)[3], double r2,
-                                                 int& bi, double& best) {
-    int c[3];
-#pragma unroll
-    for (int ax = 0; ax < 3; ++ax)      // may lie outside the grid: clamp to one cell beyond it (still "no cell in range")
-        c[ax] = (int)fmin(fmax(floor(__ddiv_rn(__dsub_rn(q[ax], g.mn[ax]), g.cell)), -2.0), (double)g.dim[ax] + 1.0);
-    best = r2;
-    bi = -1;
-    for (int dz = -1; dz <= 1; ++dz)
-        for (int dy = -1; dy <= 1; ++dy)
-            for (int dx = -1; dx <= 1; ++dx) {
-                const int x = c[0] + dx, y = c[1] + dy, z = c[2] + dz;
-                if (x < 0 || x >= g.dim[0] || y < 0 || y >= g.dim[1] || z < 0 || z >= g.dim[2]) continue;
-                const int seg = hash_find(g.cells, layout_key(g.L, x, y, z));
-                if (seg < 0) continue;
-                for (int j = g.seg_start[seg]; j < g.seg_start[seg + 1]; ++j) {
-                    const int pi = g.idx[j];
-                    const double ex = __dsub_rn(q[0], pts[3 * (size_t)pi]), ey = __dsub_rn(q[1], pts[3 * (size_t)pi + 1]),
-                                 ez = __dsub_rn(q[2], pts[3 * (size_t)pi + 2]);
-                    const double d2 = __dadd_rn(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(ey, ey)), __dmul_rn(ez, ez));
-                    if (d2 < best || (d2 == best && bi >= 0 && pi < bi)) { best = d2; bi = pi; }
-                }
-            }
-}
 
 __global__ void __launch_bounds__(128) nn_within_kernel(KnnGrid g, const double* __restrict__ pts, const double* __restrict__ qpts,
                                                         int64_t nq, double r2, int32_t* __restrict__ out_idx, double* __restrict__ out_d2) {

@@ -352,6 +352,27 @@ class PointCloud:
         nrm[zero & (rlen == 0.0)] = (0.0, 0.0, 1.0)
         self._normals = nrm
 
+    # ---- segmentation (DESIGN.md §4 "Plane segmentation and DBSCAN clustering"): drop the floor, keep the object's cluster
+    def segment_plane(self, distance_threshold, ransac_n, num_iterations, probability=0.99999999, seed=None):
+        """Open3D's RANSAC plane fit -> (plane [a, b, c, d] with a x + b y + c z + d = 0, inlier indices as a list).
+        The hypotheses are drawn from seed (None: the next seed of o3d.utility.random.seed, or an unseeded one)."""
+        n = len(self._points)
+        plane = np.zeros(4, np.float64)
+        idx = np.empty(n, np.int64)
+        m = C.c_int64(0)
+        _lib.check(_lib.lib.otslam_cloud_segment_plane(_lib.ptr(self._points), n, float(distance_threshold), int(ransac_n),
+                                                       int(num_iterations), float(probability),
+                                                       C.c_uint64(_next_seed(seed) & 0xFFFFFFFFFFFFFFFF), _lib.ptr(plane),
+                                                       _lib.ptr(idx), C.byref(m), None, 0))
+        return plane, idx[:m.value].tolist()
+
+    def cluster_dbscan(self, eps, min_points, print_progress=False):
+        """DBSCAN labels (int32, -1 = noise), clusters numbered in the order of their smallest point index."""
+        n = len(self._points)
+        labels = np.empty(n, np.int32)
+        _lib.check(_lib.lib.otslam_cloud_cluster_dbscan(_lib.ptr(self._points), n, float(eps), int(min_points), _lib.ptr(labels), None, 0))
+        return labels
+
 
 _MAX_NN = 128          # neighbours a normal estimation may keep (otslam_cloud_estimate_normals)
 
