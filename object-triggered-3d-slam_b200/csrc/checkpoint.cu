@@ -35,8 +35,6 @@
 
 namespace otslam {
 
-int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
-
 constexpr char kCkptMagic[8] = {'O', 'T', 'S', 'L', 'A', 'M', 'C', 'K'};
 constexpr uint32_t kCkptVersion = 1;
 constexpr int64_t kCkptPage = 4096;

@@ -13,38 +13,10 @@
 #include <algorithm>
 #include <vector>
 
+#include "cta_ops.cuh"
 #include "volume.cuh"
 
 namespace otslam {
-
-int device_vertex_normals(const double* d_verts, int64_t nv, const int32_t* d_faces, int64_t nf, double* d_normals,
-                          cudaStream_t s);
-int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
-
-// ---------------------------------------------------------------------------------------------
-// ordered compaction helpers: each CTA of 256 threads handles 1024 consecutive items (4 per
-// thread, consecutive), count pass -> scan over CTAs -> emit pass with intra-CTA ranks.
-// ---------------------------------------------------------------------------------------------
-constexpr int kItemsPerThread = 4;
-constexpr int kItemsPerCta = 256 * kItemsPerThread;
-
-__device__ __forceinline__ int cta_exclusive_rank(int mine, int* warp_sum /*[8]*/, int* total) {
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int base = 0, tot = 0;
-    for (int w = 0; w < 8; ++w) {
-        if (w < wid) base += warp_sum[w];
-        tot += warp_sum[w];
-    }
-    if (total) *total = tot;
-    return base + inc - mine;
-}
 
 // ---- back-projection
 struct BackprojArgs {
@@ -68,7 +40,7 @@ __global__ void __launch_bounds__(256) backproject_kernel(BackprojArgs a, const 
         mine += (d[k] > 0.f);
     }
     int total;
-    const int rank = cta_exclusive_rank(mine, warp_sum, &total);
+    const int rank = cta_exclusive_scan<int, 8>(mine, warp_sum, &total);
     if (!base) {
         if (threadIdx.x == 0) counts[blockIdx.x] = total;
         return;
@@ -109,7 +81,7 @@ __global__ void __launch_bounds__(256) zfilter_kernel(const double* __restrict__
         mine += keep[k];
     }
     int total;
-    const int rank = cta_exclusive_rank(mine, warp_sum, &total);
+    const int rank = cta_exclusive_scan<int, 8>(mine, warp_sum, &total);
     if (!base) {
         if (threadIdx.x == 0) counts[blockIdx.x] = total;
         return;
@@ -143,7 +115,7 @@ __global__ void __launch_bounds__(256) grid_points_kernel(const uint8_t* __restr
         mine += occ[k];
     }
     int total;
-    const int rank = cta_exclusive_rank(mine, warp_sum, &total);
+    const int rank = cta_exclusive_scan<int, 8>(mine, warp_sum, &total);
     if (!base) {
         if (threadIdx.x == 0) counts[blockIdx.x] = total;
         return;
@@ -175,9 +147,6 @@ __global__ void __launch_bounds__(256) tri_area_kernel(const double* __restrict_
     const double x2 = __dsub_rn(__dmul_rn(e1[0], e2[1]), __dmul_rn(e1[1], e2[0]));
     area[t] = __dmul_rn(0.5, __dsqrt_rn(__dadd_rn(__dadd_rn(__dmul_rn(x0, x0), __dmul_rn(x1, x1)), __dmul_rn(x2, x2))));
 }
-
-// ---- sequential-order accumulation (surface area, area CDF, outlier-filter statistics): ordered_sum.cu
-int device_ordered_sum(double* d_x, int64_t n, int mode, const double* d_div, double mean, double* d_out, cudaStream_t s);
 
 // triangle t owns samples [end[t-1], end[t]) with end[t] = llround(cdf[t]*n) (last forced to n)
 __global__ void __launch_bounds__(256) sample_kernel(const double* __restrict__ v, const double* __restrict__ col,
@@ -238,6 +207,18 @@ __global__ void __launch_bounds__(256) rigid_kernel(const double* __restrict__ p
         for (int r = 0; r < 3; ++r)
             out_nrm[3 * i + r] = __dadd_rn(__dadd_rn(__dmul_rn(a.m[st * r], p), __dmul_rn(a.m[st * r + 1], q)), __dmul_rn(a.m[st * r + 2], w));
     }
+}
+
+// p' = (T * [p, 1]).xyz / w on device buffers (otslam_cloud_transform's arithmetic), queued on stream s; the cloud ICP
+// moves its source by each update with it
+int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s) {
+    if (n <= 0) return OTSLAM_OK;
+    RigidArgs a;
+    for (int i = 0; i < 16; ++i) a.m[i] = T[i];
+    a.mode = 0;
+    rigid_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_in, nullptr, n, a, d_out, nullptr);
+    OT_LAUNCHED();
+    return OTSLAM_OK;
 }
 
 __global__ void __launch_bounds__(256) axis_extract_kernel(const double* __restrict__ pts, int64_t n, int axis, double* __restrict__ out) {
@@ -308,20 +289,6 @@ __global__ void __launch_bounds__(256) merge_pack_kernel(MergeArgs a, uint8_t* _
     for (int64_t i = threadIdx.x; i < nvec; i += 256)
         reinterpret_cast<uint4*>(o)[i] = reinterpret_cast<const uint4*>(stage)[i];
     for (int64_t i = nvec * 16 + threadIdx.x; i < nbytes; i += 256) o[i] = stage[i];
-}
-
-template <typename F>
-static int compact_two_pass(int64_t n_items, cudaStream_t s, int64_t* n_out, DevBuf<int>& counts, DevBuf<int64_t>& base, F launch) {
-    const int n_cta = (int)((n_items + kItemsPerCta - 1) / kItemsPerCta);
-    *n_out = 0;
-    if (n_cta == 0) return OTSLAM_OK;
-    OT_CUDA(counts.alloc(n_cta));
-    OT_CUDA(base.alloc(n_cta + 1));
-    OT_TRY(launch(n_cta, (const int64_t*)nullptr, counts.p));
-    OT_TRY(device_exclusive_scan(counts.p, base.p, n_cta, s));
-    OT_CUDA(cudaMemcpyAsync(n_out, base.p + n_cta, 8, cudaMemcpyDefault, s));
-    OT_CUDA(cudaStreamSynchronize(s));
-    return OTSLAM_OK;
 }
 
 }  // namespace otslam
@@ -504,18 +471,6 @@ int otslam_grid_to_points(const uint8_t* gray, int width, int height, double res
     OT_TRY(launch((int)((n + kItemsPerCta - 1) / kItemsPerCta), base.p, nullptr));
     timer.stop();
     OT_CUDA(cudaMemcpy(out_points, op.p, m * 24, cudaMemcpyDefault));
-    return OTSLAM_OK;
-}
-
-// p' = (T * [p, 1]).xyz / w on device buffers (otslam_cloud_transform's arithmetic), queued on stream s; the cloud ICP
-// moves its source by each update with it
-int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s) {
-    if (n <= 0) return OTSLAM_OK;
-    RigidArgs a;
-    for (int i = 0; i < 16; ++i) a.m[i] = T[i];
-    a.mode = 0;
-    rigid_kernel<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_in, nullptr, n, a, d_out, nullptr);
-    OT_LAUNCHED();
     return OTSLAM_OK;
 }
 

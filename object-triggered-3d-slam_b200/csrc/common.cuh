@@ -230,4 +230,18 @@ struct OpTimer {
     }
 };
 
+// ---- device routines shared between translation units; each queues its work on stream s
+// scan.cu: exclusive prefix sum of n int32 into int64, the total at d_out[n]
+int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
+// knn.cu: stable LSD radix sort of (u64 key, i32 value) pairs by the low `bits` bits; result in (kb, vb), (ka, va) clobbered
+int device_sort_pairs(uint64_t* ka, int32_t* va, uint64_t* kb, int32_t* vb, int64_t n, int bits, cudaStream_t s);
+// ordered_sum.cu: the left-to-right FP64 chain over the terms of d_x[0..n), bit-identical to the scalar loop; term mode 0:
+// x, 2: x > 0 ? x : 0, 3: x > 0 ? (x - mean)^2 : 0, the sum into *d_out; mode 1: x / *d_div, d_x becomes the inclusive prefix
+int device_ordered_sum(double* d_x, int64_t n, int mode, const double* d_div, double mean, double* d_out, cudaStream_t s);
+// cloud.cu: p' = (T * [p, 1]).xyz / w of n points, otslam_cloud_transform's arithmetic
+int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s);
+// extract.cu: compute_vertex_normals of a device mesh, each vertex's face normals added in triangle order
+int device_vertex_normals(const double* d_verts, int64_t nv, const int32_t* d_faces, int64_t nf, double* d_normals,
+                          cudaStream_t s);
+
 }  // namespace otslam

@@ -17,6 +17,7 @@
 #include <algorithm>
 #include <vector>
 
+#include "cta_ops.cuh"
 #include "volume_lookup.cuh"
 
 #define MC_TABLE_QUAL static const
@@ -158,30 +159,19 @@ __global__ void __launch_bounds__(256) mc_classify_kernel(ExtractCtx c, uint32_t
 __global__ void __launch_bounds__(128) mc_count_kernel(const int32_t* __restrict__ bslots, const uint32_t* __restrict__ flags,
                                                        uint16_t* __restrict__ word_prefix, int* __restrict__ vcount) {
     __shared__ int warp_sum[4];
-    const int i = blockIdx.x, t = threadIdx.x, lane = t & 31, wid = t >> 5;
+    const int i = blockIdx.x, t = threadIdx.x;
     const int slot = bslots[i];
     const uint32_t* f = flags + (size_t)slot * kFlagWords;
     uint16_t* wp = word_prefix + (size_t)slot * kFlagWords;
     // thread t owns words 3t..3t+2
     const int c0 = __popc(f[3 * t]), c1 = __popc(f[3 * t + 1]), c2 = __popc(f[3 * t + 2]);
-    int v = c0 + c1 + c2, inc = v;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int base = 0;
-    for (int w = 0; w < wid; ++w) base += warp_sum[w];
-    const int ex = base + inc - v;
+    const int v = c0 + c1 + c2;
+    const int ex = cta_exclusive_scan<int, 4>(v, warp_sum, nullptr);
     wp[3 * t] = (uint16_t)ex;
     wp[3 * t + 1] = (uint16_t)(ex + c0);
     wp[3 * t + 2] = (uint16_t)(ex + c0 + c1);
-    if (t == 127) vcount[i] = base + inc;
+    if (t == 127) vcount[i] = ex + v;
 }
-
-// exclusive scan int32 -> int64 with the total at out[n]: scan.cu
-int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
 
 __global__ void scatter_base_kernel(const int32_t* __restrict__ bslots, const int64_t* __restrict__ vbase, int n,
                                     int64_t* __restrict__ vbase_by_slot) {
@@ -272,7 +262,7 @@ __global__ void __launch_bounds__(256) mc_faces_kernel(ExtractCtx c, const uint3
                                                        const int64_t* __restrict__ fbase, int32_t* __restrict__ faces) {
     __shared__ int nslot[8];
     __shared__ int warp_sum[8];
-    const int i = blockIdx.x, t = threadIdx.x, lane = t & 31, wid = t >> 5;
+    const int i = blockIdx.x, t = threadIdx.x;
     if (fbase[i + 1] == fbase[i]) return;
     const uint64_t key = c.bkeys[i];
     const int slot = c.bslots[i];
@@ -284,16 +274,7 @@ __global__ void __launch_bounds__(256) mc_faces_kernel(ExtractCtx c, const uint3
     int mine = 0;
 #pragma unroll
     for (int k = 0; k < 16; ++k) mine += d_ntri[(pw[k >> 2] >> (8 * (k & 3))) & 0xFF];
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int base = 0;
-    for (int w = 0; w < wid; ++w) base += warp_sum[w];
-    int64_t fo = fbase[i] + base + inc - mine;
+    int64_t fo = fbase[i] + cta_exclusive_scan<int, 8>(mine, warp_sum, nullptr);
     for (int k = 0; k < 16; ++k) {
         const int cube = (pw[k >> 2] >> (8 * (k & 3))) & 0xFF;
         if (!cube) continue;
@@ -415,7 +396,7 @@ __global__ void __launch_bounds__(256) pc_extract_kernel(ExtractCtx c, const int
                                                          int32_t* __restrict__ ekeys) {
     __shared__ int nslot[8];
     __shared__ int warp_sum[8];
-    const int i = blockIdx.x, t = threadIdx.x, lane = t & 31, wid = t >> 5;
+    const int i = blockIdx.x, t = threadIdx.x;
     const uint64_t key = c.bkeys[i];
     const int slot = c.bslots[i];
     int kx, ky, kz;
@@ -450,20 +431,12 @@ __global__ void __launch_bounds__(256) pc_extract_kernel(ExtractCtx c, const int
             ++mine;
         }
     }
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int n = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += n;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int base = 0;
-    for (int w = 0; w < wid; ++w) base += warp_sum[w];
+    const int rank = cta_exclusive_scan<int, 8>(mine, warp_sum, nullptr);
     if (count_only) {
-        if (t == 255) pcount[i] = base + inc;
+        if (t == 255) pcount[i] = rank + mine;
         return;
     }
-    int64_t o = pbase[i] + base + inc - mine;
+    int64_t o = pbase[i] + rank;
     for (int k = 0; k < 16; ++k) {
         const uint32_t h = (hits[k >> 3] >> (3 * (k & 7))) & 7u;
         if (!h) continue;

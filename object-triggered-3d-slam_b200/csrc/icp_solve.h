@@ -1,5 +1,6 @@
-// icp_solve.h -- the 6x6 Gauss-Newton solve shared by the point-to-plane solvers: frame-to-model tracking (track.cu, on the
-// device) and cloud-to-cloud ICP (knn.cu, on the host), plus the Euler-angle update of the cloud ICP.  Every FP64 operation
+// icp_solve.h -- the point-to-plane terms and the 6x6 Gauss-Newton solve shared by the point-to-plane solvers: frame-to-model
+// tracking (track.cu, all on the device) and cloud-to-cloud ICP (knn.cu, terms on the device, solve on the host), plus the
+// Euler-angle update of the cloud ICP.  Every FP64 operation
 // is explicit round-to-nearest with no FMA, so the device and the host (compiled with -ffp-contract=off) give the same bits.
 // Plain C++ too: the CPU model of the cloud ICP (tests/models/normals_icp_model.cpp) includes this file rather than
 // restating it.
@@ -51,6 +52,24 @@ OT_HD inline double rn_sqrt(double a) {
 #else
     return std::sqrt(a);
 #endif
+}
+
+// The point-to-plane terms of one correspondence, in the layout solve6 reads: p the source point at the current pose, n the
+// model's normal, e = p - the model's point; r = (n0 e0 + n1 e1) + n2 e2 and J = [p x n, n].  t[stride * k] = term k:
+// 0..20 J_a J_b for a <= b (row-major), 21..26 J_a r, 27 r^2, 28 1.0 (one inlier).  Terms after 28 are the caller's.
+OT_HD inline void point_to_plane_terms(const double p[3], const double n[3], const double e[3], double* t, int stride) {
+    const double r = rn_add(rn_add(rn_mul(n[0], e[0]), rn_mul(n[1], e[1])), rn_mul(n[2], e[2]));
+    const double J[6] = {rn_sub(rn_mul(p[1], n[2]), rn_mul(p[2], n[1])), rn_sub(rn_mul(p[2], n[0]), rn_mul(p[0], n[2])),
+                         rn_sub(rn_mul(p[0], n[1]), rn_mul(p[1], n[0])), n[0], n[1], n[2]};
+    int k = 0;
+#pragma unroll
+    for (int a = 0; a < 6; ++a)
+#pragma unroll
+        for (int b = a; b < 6; ++b) t[stride * k++] = rn_mul(J[a], J[b]);
+#pragma unroll
+    for (int a = 0; a < 6; ++a) t[stride * (21 + a)] = rn_mul(J[a], r);
+    t[stride * 27] = rn_mul(r, r);
+    t[stride * 28] = 1.0;
 }
 
 // Cholesky solve of A xi = -b, A from S[0..20] (upper triangle, row-major) and b = S[21..26]; false when a pivot is

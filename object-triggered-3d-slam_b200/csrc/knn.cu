@@ -17,12 +17,11 @@
 #include <cstdlib>
 #include <vector>
 
+#include "cta_ops.cuh"
 #include "icp_solve.h"
 #include "knn_grid.cuh"
 
 namespace otslam {
-
-int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
 
 // ---- exact min / max of FP64 coordinates via order-preserving integer keys
 __device__ __forceinline__ unsigned long long d2key(double d) {
@@ -189,57 +188,15 @@ int device_sort_pairs(uint64_t* ka_in, int32_t* va_in, uint64_t* kb_out, int32_t
     // (stream order protects them) and every operator synchronises before it returns
     return OTSLAM_OK;
 }
-static int sort_pairs(DevBuf<uint64_t>& k_in, DevBuf<int32_t>& v_in, DevBuf<uint64_t>& k_out, DevBuf<int32_t>& v_out, int64_t n,
-                      int bits) {
-    return device_sort_pairs(k_in.p, v_in.p, k_out.p, v_out.p, n, bits, 0);
-}
+// segment heads of the sorted keys: the first key of each run of equal keys
+struct SegmentHead {
+    const uint64_t* keys;
+    __device__ bool operator()(int64_t p) const { return p == 0 || keys[p] != keys[p - 1]; }
+};
 
-// segment heads of the sorted keys: count pass / emit pass (ordered)
-__global__ void __launch_bounds__(256) seg_heads_kernel(const uint64_t* __restrict__ keys, int64_t n, const int64_t* __restrict__ base,
-                                                        int* __restrict__ counts, int32_t* __restrict__ seg_start) {
-    __shared__ int warp_sum[8];
-    const int64_t p0 = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 4;
-    bool head[4];
-    int mine = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int64_t p = p0 + k;
-        head[k] = (p < n) && (p == 0 || keys[p] != keys[p - 1]);
-        mine += head[k];
-    }
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += v;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int b = 0, tot = 0;
-    for (int w = 0; w < 8; ++w) { if (w < wid) b += warp_sum[w]; tot += warp_sum[w]; }
-    if (!base) {
-        if (threadIdx.x == 0) counts[blockIdx.x] = tot;
-        return;
-    }
-    int64_t o = base[blockIdx.x] + b + inc - mine;
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-        if (head[k]) seg_start[o++] = (int32_t)(p0 + k);
-}
-
+// seg_start[0..n_seg) = the segment heads in order, seg_start[n_seg] = n
 static int find_segments(const uint64_t* d_keys, int64_t n, DevBuf<int32_t>& seg_start, int64_t* n_seg) {
-    const int n_cta = (int)((n + 1023) / 1024);
-    DevBuf<int> counts;
-    DevBuf<int64_t> base;
-    OT_CUDA(counts.alloc(n_cta));
-    OT_CUDA(base.alloc(n_cta + 1));
-    seg_heads_kernel<<<n_cta, 256>>>(d_keys, n, nullptr, counts.p, nullptr);
-    OT_LAUNCHED();
-    OT_TRY(device_exclusive_scan(counts.p, base.p, n_cta, 0));
-    OT_CUDA(cudaMemcpy(n_seg, base.p + n_cta, 8, cudaMemcpyDefault));
-    OT_CUDA(seg_start.alloc(*n_seg + 1));
-    seg_heads_kernel<<<n_cta, 256>>>(d_keys, n, base.p, nullptr, seg_start.p);
-    OT_LAUNCHED();
+    OT_TRY(select_indices(SegmentHead{d_keys}, n, 0, seg_start, n_seg, 1));
     const int32_t nn = (int32_t)n;
     OT_CUDA(cudaMemcpy(seg_start.p + *n_seg, &nn, 4, cudaMemcpyDefault));
     return OTSLAM_OK;
@@ -736,10 +693,6 @@ static int upload_shell_table() {
     return OTSLAM_OK;
 }
 
-
-static int sort_pairs(DevBuf<uint64_t>& k_in, DevBuf<int32_t>& v_in, DevBuf<uint64_t>& k_out, DevBuf<int32_t>& v_out, int64_t n, int bits);
-static int find_segments(const uint64_t* d_keys, int64_t n, DevBuf<int32_t>& seg_start, int64_t* n_seg);
-
 // bucket the n points of d_pts on a grid of `cell`-sized cells over [mn, mx] (at most max_dim cells per axis)
 int build_grid(const double* d_pts, int64_t n, const double mn[3], const double mx[3], double cell, int max_dim, GridBuffers& b,
                KnnGrid& g) {
@@ -754,7 +707,7 @@ int build_grid(const double* d_pts, int64_t n, const double mn[3], const double 
     cell_key_kernel<<<(unsigned)((n + 255) / 256), 256>>>(d_pts, n, mn[0], mn[1], mn[2], cell, g.dim[0] - 1, g.dim[1] - 1, g.dim[2] - 1,
                                                          g.L, b.k0.p, b.i0.p);
     OT_LAUNCHED();
-    OT_TRY(sort_pairs(b.k0, b.i0, b.k1, b.i1, n, g.L.bits));
+    OT_TRY(device_sort_pairs(b.k0.p, b.i0.p, b.k1.p, b.i1.p, n, g.L.bits, 0));
     OT_TRY(find_segments(b.k1.p, n, b.seg, &b.n_seg));
     uint32_t cap = 1024;
     while (!hash_fits(b.n_seg, cap)) cap <<= 1;
@@ -812,41 +765,12 @@ static int build_search(const double* d_pts, int64_t n, GridBuffers& bc, GridBuf
     return OTSLAM_OK;
 }
 
-// sequential-order sums for the global mean / sigma: cloud.cu's ordered accumulation, modes 2 and 3
-int device_ordered_sum(double* d_x, int64_t n, int mode, const double* d_div, double mean, double* d_out, cudaStream_t s);
-
-__global__ void __launch_bounds__(256) sor_select_kernel(const double* __restrict__ dbar, int64_t n, double thr,
-                                                         const int64_t* __restrict__ base, int* __restrict__ counts,
-                                                         int64_t* __restrict__ out_idx) {
-    __shared__ int warp_sum[8];
-    const int64_t p0 = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 4;
-    bool keep[4];
-    int mine = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int64_t p = p0 + k;
-        keep[k] = (p < n) && (dbar[p] > 0.0) && (dbar[p] < thr);
-        mine += keep[k];
-    }
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += v;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int b = 0, tot = 0;
-    for (int w = 0; w < 8; ++w) { if (w < wid) b += warp_sum[w]; tot += warp_sum[w]; }
-    if (!base) {
-        if (threadIdx.x == 0) counts[blockIdx.x] = tot;
-        return;
-    }
-    int64_t o = base[blockIdx.x] + b + inc - mine;
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-        if (keep[k]) out_idx[o++] = p0 + k;
-}
+// the points remove_statistical_outlier keeps: 0 < dbar < thr
+struct SorKeep {
+    const double* dbar;
+    double thr;
+    __device__ bool operator()(int64_t p) const { return dbar[p] > 0.0 && dbar[p] < thr; }
+};
 
 }  // namespace otslam
 
@@ -883,7 +807,7 @@ int otslam_cloud_voxel_down_sample(const double* points, const double* colors, i
     OT_CUDA(k0.alloc(n)); OT_CUDA(k1.alloc(n)); OT_CUDA(i0.alloc(n)); OT_CUDA(i1.alloc(n));
     cell_key_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dp.p, n, vmin[0], vmin[1], vmin[2], voxel_size, -1, -1, -1, L, k0.p, i0.p);
     OT_LAUNCHED();
-    OT_TRY(sort_pairs(k0, i0, k1, i1, n, L.bits));
+    OT_TRY(device_sort_pairs(k0.p, i0.p, k1.p, i1.p, n, L.bits, 0));
     DevBuf<int32_t> seg;
     int64_t m = 0;
     OT_TRY(find_segments(k1.p, n, seg, &m));
@@ -938,20 +862,11 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
     OT_CUDA(cudaMemcpy(&sq, scal.p, 8, cudaMemcpyDefault));
     const double sd = valid > 1 ? std::sqrt(sq / (double)(valid - 1)) : 0.0;
     const double thr = mean + std_ratio * sd;
-    const int n_cta = (int)((n + 1023) / 1024);
-    DevBuf<int> counts;
-    DevBuf<int64_t> base, oidx;
-    OT_CUDA(counts.alloc(n_cta)); OT_CUDA(base.alloc(n_cta + 1));
-    sor_select_kernel<<<n_cta, 256>>>(dbar.p, n, thr, nullptr, counts.p, nullptr);
-    OT_LAUNCHED();
-    OT_TRY(device_exclusive_scan(counts.p, base.p, n_cta, 0));
+    DevBuf<int64_t> oidx;
     int64_t m = 0;
-    OT_CUDA(cudaMemcpy(&m, base.p + n_cta, 8, cudaMemcpyDefault));
+    OT_TRY(select_indices(SorKeep{dbar.p, thr}, n, 0, oidx, &m));
     *n_out = m;
     if (m == 0) return OTSLAM_OK;
-    OT_CUDA(oidx.alloc(m));
-    sor_select_kernel<<<n_cta, 256>>>(dbar.p, n, thr, base.p, nullptr, oidx.p);
-    OT_LAUNCHED();
     timer.stop();
     OT_CUDA(cudaMemcpy(out_indices, oidx.p, m * 8, cudaMemcpyDefault));
     return OTSLAM_OK;
@@ -993,19 +908,8 @@ __global__ void __launch_bounds__(kIcpThreads) icp_assoc_kernel(KnnGrid g, const
         if (bi >= 0) {
             const size_t m = 3 * (size_t)bi;
             const double N[3] = {tn[m], tn[m + 1], tn[m + 2]};
-            const double r = __dadd_rn(__dadd_rn(__dmul_rn(__dsub_rn(p[0], tgt[m]), N[0]), __dmul_rn(__dsub_rn(p[1], tgt[m + 1]), N[1])),
-                                       __dmul_rn(__dsub_rn(p[2], tgt[m + 2]), N[2]));
-            const double J[6] = {__dsub_rn(__dmul_rn(p[1], N[2]), __dmul_rn(p[2], N[1])), __dsub_rn(__dmul_rn(p[2], N[0]), __dmul_rn(p[0], N[2])),
-                                 __dsub_rn(__dmul_rn(p[0], N[1]), __dmul_rn(p[1], N[0])), N[0], N[1], N[2]};
-            int k = 0;
-#pragma unroll
-            for (int a = 0; a < 6; ++a)
-#pragma unroll
-                for (int b = a; b < 6; ++b) sm[k++][lane] = __dmul_rn(J[a], J[b]);
-#pragma unroll
-            for (int a = 0; a < 6; ++a) sm[21 + a][lane] = __dmul_rn(J[a], r);
-            sm[27][lane] = __dmul_rn(r, r);
-            sm[28][lane] = 1.0;
+            const double e[3] = {__dsub_rn(p[0], tgt[m]), __dsub_rn(p[1], tgt[m + 1]), __dsub_rn(p[2], tgt[m + 2])};
+            point_to_plane_terms(p, N, e, &sm[0][lane], kIcpThreads);
             sm[29][lane] = d2;
             matched = true;
         }
@@ -1013,34 +917,9 @@ __global__ void __launch_bounds__(kIcpThreads) icp_assoc_kernel(KnnGrid g, const
     if (!matched)                        // no point or no correspondence: its terms are 0
 #pragma unroll
         for (int k = 0; k < kIcpTerms; ++k) sm[k][lane] = 0.0;
-    // fixed halving tree: lane i += lane i + 64, then i + 32, ... (absent points hold 0)
-    for (int s = kIcpThreads / 2; s > 0; s >>= 1) {
-        __syncthreads();
-        for (int j = lane; j < kIcpTerms * s; j += kIcpThreads) {
-            const int k = j / s, e = j - k * s;
-            sm[k][e] = __dadd_rn(sm[k][e], sm[k][e + s]);
-        }
-    }
-    __syncthreads();
+    cta_halving_tree(sm);                // absent points add 0
     if (lane < kIcpTerms) partials[(size_t)lane * P + blockIdx.x] = sm[lane][0];
 }
-
-// the CTA partials padded with zeros to P = 2^k, summed by a fixed pairwise tree (i += i + P/2, then i + P/4, ...), as
-// track.cu's solve kernel sums its tiles; out[30] = the totals
-__global__ void __launch_bounds__(kIcpSumThreads) icp_sum_kernel(double* __restrict__ buf, int n_cta, int P, double* __restrict__ out) {
-    for (int h = P / 2; h > 0; h >>= 1) {
-        for (int j = threadIdx.x; j < kIcpTerms * h; j += kIcpSumThreads) {
-            const int k = j / h, i = j - k * h;
-            const double x = i < n_cta ? buf[(size_t)k * P + i] : 0.0;
-            const double y = i + h < n_cta ? buf[(size_t)k * P + i + h] : 0.0;
-            buf[(size_t)k * P + i] = __dadd_rn(x, y);
-        }
-        __syncthreads();
-    }
-    if (threadIdx.x < kIcpTerms) out[threadIdx.x] = buf[(size_t)threadIdx.x * P];
-}
-
-int device_rigid_transform(const double* d_in, int64_t n, const double T[16], double* d_out, cudaStream_t s);
 
 int otslam_cloud_nn_within(const double* source, int64_t n_source, const double* target, int64_t n_target, double radius,
                            int32_t* out_index, double* out_dist2, int device) {
@@ -1158,8 +1037,7 @@ int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, cons
     OT_TRY(use_device(device));
     const int64_t n = n_source;
     const int n_cta = (int)((n + kIcpThreads - 1) / kIcpThreads);
-    int P = 1;
-    while (P < n_cta) P *= 2;
+    const int P = pow2_at_least(n_cta);
     DevBuf<double> ds0, ds1, dt, dtn, dpart, dsum;
     DevBuf<int32_t> dcorr;
     OT_CUDA(ds0.alloc(n * 3)); OT_CUDA(ds1.alloc(n * 3)); OT_CUDA(dcorr.alloc(n));
@@ -1187,7 +1065,7 @@ int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, cons
     auto evaluate = [&](double& fit, double& rmse) -> int {
         icp_assoc_kernel<<<n_cta, kIcpThreads>>>(g, dt.p, dtn.p, n_target > 0, cur, n, r2, dcorr.p, dpart.p, P);
         OT_LAUNCHED();
-        icp_sum_kernel<<<1, kIcpSumThreads>>>(dpart.p, n_cta, P, dsum.p);
+        tree_rows_kernel<kIcpSumThreads><<<kIcpTerms, kIcpSumThreads>>>(dpart.p, n_cta, P, dsum.p);
         OT_LAUNCHED();
         OT_CUDA(cudaMemcpy(S, dsum.p, sizeof(S), cudaMemcpyDeviceToHost));
         fit = S[28] / (double)n;

@@ -2,7 +2,7 @@
 // compaction of the path and by the radix sort.  Three phases over tiles of 2048 items (256 threads x
 // 8 consecutive items, coalesced 16-byte loads): per-tile sums, scan of the tile sums (one CTA), per-tile
 // scan with the tile's base.  Inputs that fit one tile take a single launch.
-#include "common.cuh"
+#include "cta_ops.cuh"
 
 namespace otslam {
 
@@ -19,28 +19,6 @@ __device__ __forceinline__ void scan_load(const int* __restrict__ in, int64_t ba
     }
 }
 
-// CTA-wide exclusive scan of one int64 per thread (256 threads); returns the exclusive prefix, *total = CTA sum
-__device__ __forceinline__ int64_t cta_scan256(int64_t mine, int64_t* warp_sums /*[8]*/, int64_t* total) {
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    int64_t inc = mine;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int64_t u = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += u;
-    }
-    if (lane == 31) warp_sums[w] = inc;
-    __syncthreads();
-    int64_t before = 0, tot = 0;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        const int64_t s = warp_sums[k];
-        if (k < w) before += s;
-        tot += s;
-    }
-    if (total) *total = tot;
-    return before + inc - mine;
-}
-
 __global__ void __launch_bounds__(256) scan_tile_sum_kernel(const int* __restrict__ in, int64_t n, int64_t* __restrict__ tile_sum) {
     __shared__ int64_t ws[8];
     int v[kScanItems];
@@ -49,7 +27,7 @@ __global__ void __launch_bounds__(256) scan_tile_sum_kernel(const int* __restric
 #pragma unroll
     for (int k = 0; k < kScanItems; ++k) s += v[k];
     int64_t tot;
-    cta_scan256(s, ws, &tot);
+    cta_exclusive_scan<int64_t, 8>(s, ws, &tot);
     if (threadIdx.x == 0) tile_sum[blockIdx.x] = tot;
 }
 
@@ -63,7 +41,7 @@ __global__ void __launch_bounds__(256) scan_tile_base_kernel(int64_t* __restrict
         const int64_t i = base + threadIdx.x;
         const int64_t v = i < n_tiles ? tile_sum[i] : 0;
         int64_t tot;
-        const int64_t ex = cta_scan256(v, ws, &tot);
+        const int64_t ex = cta_exclusive_scan<int64_t, 8>(v, ws, &tot);
         if (i < n_tiles) tile_sum[i] = carry + ex;
         __syncthreads();
         if (threadIdx.x == 0) carry += tot;
@@ -82,7 +60,7 @@ __global__ void __launch_bounds__(256) scan_tile_kernel(const int* __restrict__ 
 #pragma unroll
     for (int k = 0; k < kScanItems; ++k) s += v[k];
     int64_t tot;
-    int64_t acc = cta_scan256(s, ws, &tot) + (tile_base ? tile_base[blockIdx.x] : 0);
+    int64_t acc = cta_exclusive_scan<int64_t, 8>(s, ws, &tot) + (tile_base ? tile_base[blockIdx.x] : 0);
 #pragma unroll
     for (int k = 0; k < kScanItems; ++k) {
         if (base + k < n) out[base + k] = acc;

@@ -13,11 +13,10 @@
 #include <cmath>
 #include <cstdint>
 
+#include "cta_ops.cuh"
 #include "knn_grid.cuh"
 
 namespace otslam {
-
-int device_exclusive_scan(const int* d_in, int64_t* d_out, int n, cudaStream_t s);
 
 // ---------------------------------------------------------------------------------------------
 // DBSCAN
@@ -266,55 +265,15 @@ __global__ void __launch_bounds__(kSegThreads) ransac_eval_kernel(const double* 
     }
 }
 
-// one CTA per row of n_cta partials padded with zeros to P = 2^k: the fixed pairwise tree i += i + P/2, then i + P/4, ...
-// out[row] = the row's total
-__global__ void __launch_bounds__(256) tree_rows_kernel(double* __restrict__ buf, int n_cta, int P, double* __restrict__ out) {
-    double* row = buf + (size_t)blockIdx.x * P;
-    for (int h = P / 2; h > 0; h >>= 1) {
-        for (int i = threadIdx.x; i < h; i += 256) {
-            const double a = i < n_cta ? row[i] : 0.0, b = i + h < n_cta ? row[i + h] : 0.0;
-            row[i] = a + b;
-        }
-        __syncthreads();
+// an inlier of the selected plane, by the test of its evaluation
+struct PlaneInlier {
+    const double* pts;
+    const double4* plane;
+    double thr;
+    __device__ bool operator()(int64_t p) const {
+        return plane_dist(*plane, pts[3 * p], pts[3 * p + 1], pts[3 * p + 2]) < thr;
     }
-    if (threadIdx.x == 0) out[blockIdx.x] = row[0];
-}
-
-// the selected plane's inliers in ascending order, sor_select_kernel's two passes (counts per CTA, then emit at the
-// scanned bases)
-__global__ void __launch_bounds__(256) plane_select_kernel(const double* __restrict__ pts, int64_t n, const double4* __restrict__ plane,
-                                                           double thr, const int64_t* __restrict__ base, int* __restrict__ counts,
-                                                           int64_t* __restrict__ out_idx) {
-    __shared__ int warp_sum[8];
-    const double4 pl = *plane;
-    const int64_t p0 = ((int64_t)blockIdx.x * 256 + threadIdx.x) * 4;
-    bool keep[4];
-    int mine = 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        const int64_t p = p0 + k;
-        keep[k] = p < n && plane_dist(pl, pts[3 * p], pts[3 * p + 1], pts[3 * p + 2]) < thr;
-        mine += keep[k];
-    }
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-    int inc = mine;
-    for (int o = 1; o < 32; o <<= 1) {
-        const int v = __shfl_up_sync(0xffffffffu, inc, o);
-        if (lane >= o) inc += v;
-    }
-    if (lane == 31) warp_sum[wid] = inc;
-    __syncthreads();
-    int b = 0, tot = 0;
-    for (int w = 0; w < 8; ++w) { if (w < wid) b += warp_sum[w]; tot += warp_sum[w]; }
-    if (!base) {
-        if (threadIdx.x == 0) counts[blockIdx.x] = tot;
-        return;
-    }
-    int64_t o = base[blockIdx.x] + b + inc - mine;
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-        if (keep[k]) out_idx[o++] = p0 + k;
-}
+};
 
 // the refit's sums over the m inliers, positions as in ransac_eval_kernel: mode 0 the 3 coordinate sums, mode 1 the 6
 // centred moments xx, xy, xz, yy, yz, zz about cen; partials[term][cta]
@@ -350,12 +309,6 @@ __global__ void __launch_bounds__(kSegThreads) refit_sum_kernel(const double* __
     if (threadIdx.x < n_terms) partials[(size_t)threadIdx.x * P + blockIdx.x] = cta_tree8(ws[threadIdx.x]);
 }
 
-static int pow2_at_least(int64_t x) {
-    int P = 1;
-    while (P < x) P *= 2;
-    return P;
-}
-
 // the rows' fixed-tree totals of n_terms partial rows -> host
 static int refit_sums(const double* d_pts, const int64_t* d_idx, int64_t m, int mode, const double cen[3], double* h_out) {
     const int n_cta = (int)((m + kSegTile - 1) / kSegTile), P = pow2_at_least(n_cta), n_terms = mode == 0 ? 3 : 6;
@@ -363,7 +316,7 @@ static int refit_sums(const double* d_pts, const int64_t* d_idx, int64_t m, int 
     OT_CUDA(part.alloc((size_t)n_terms * P)); OT_CUDA(tot.alloc(n_terms));
     refit_sum_kernel<<<n_cta, kSegThreads>>>(d_pts, d_idx, m, mode, cen[0], cen[1], cen[2], part.p, P);
     OT_LAUNCHED();
-    tree_rows_kernel<<<n_terms, 256>>>(part.p, n_cta, P, tot.p);
+    tree_rows_kernel<256><<<n_terms, 256>>>(part.p, n_cta, P, tot.p);
     OT_LAUNCHED();
     OT_CUDA(cudaMemcpy(h_out, tot.p, n_terms * sizeof(double), cudaMemcpyDeviceToHost));
     return OTSLAM_OK;
@@ -457,7 +410,7 @@ int otslam_cloud_segment_plane(const double* points, int64_t n, double distance_
         OT_LAUNCHED();
         ransac_eval_kernel<<<n_cta, kSegThreads>>>(dp.p, n, planes.p, wn, distance_threshold, part.p, P);
         OT_LAUNCHED();
-        tree_rows_kernel<<<2 * wn, 256>>>(part.p, n_cta, P, res.p);
+        tree_rows_kernel<256><<<2 * wn, 256>>>(part.p, n_cta, P, res.p);
         OT_LAUNCHED();
         OT_CUDA(cudaMemcpy(h_res, res.p, 2 * wn * sizeof(double), cudaMemcpyDeviceToHost));
         for (int w = 0; w < wn; ++w) {
@@ -484,18 +437,9 @@ int otslam_cloud_segment_plane(const double* points, int64_t n, double distance_
     if (n_evaluated) *n_evaluated = evaluated;
     if (!have_best) return OTSLAM_OK;
     // the best plane's inliers (the same test as its evaluation), then GetPlaneFromPoints over them by the fixed trees
-    const int n_sel = (int)((n + 1023) / 1024);
-    DevBuf<int> counts;
-    DevBuf<int64_t> base, oidx;
-    OT_CUDA(counts.alloc(n_sel)); OT_CUDA(base.alloc(n_sel + 1));
-    plane_select_kernel<<<n_sel, 256>>>(dp.p, n, best_plane.p, distance_threshold, nullptr, counts.p, nullptr);
-    OT_LAUNCHED();
-    OT_TRY(device_exclusive_scan(counts.p, base.p, n_sel, 0));
+    DevBuf<int64_t> oidx;
     int64_t m = 0;
-    OT_CUDA(cudaMemcpy(&m, base.p + n_sel, 8, cudaMemcpyDeviceToHost));
-    OT_CUDA(oidx.alloc(m));
-    plane_select_kernel<<<n_sel, 256>>>(dp.p, n, best_plane.p, distance_threshold, base.p, nullptr, oidx.p);
-    OT_LAUNCHED();
+    OT_TRY(select_indices(PlaneInlier{dp.p, best_plane.p, distance_threshold}, n, 0, oidx, &m));
     double sum[3], mom[6], cen[3] = {0.0, 0.0, 0.0};
     OT_TRY(refit_sums(dp.p, oidx.p, m, 0, cen, sum));
     for (int a = 0; a < 3; ++a) cen[a] = sum[a] / (double)m;

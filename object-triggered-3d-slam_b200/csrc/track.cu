@@ -20,6 +20,7 @@
 #include <cmath>
 #include <vector>
 
+#include "cta_ops.cuh"
 #include "icp_solve.h"
 #include "raycast.cuh"
 
@@ -131,20 +132,8 @@ __global__ void __launch_bounds__(kTilePx) track_assoc_kernel(const TrackArgs a,
                     if (N[0] != 0.0 || N[1] != 0.0 || N[2] != 0.0) {
                         const double e[3] = {ds(p[0], (double)a.vertex[m]), ds(p[1], (double)a.vertex[m + 1]),
                                              ds(p[2], (double)a.vertex[m + 2])};
-                        if (da(da(dm(e[0], e[0]), dm(e[1], e[1])), dm(e[2], e[2])) <= a.ddiff2) {
-                            const double r = da(da(dm(N[0], e[0]), dm(N[1], e[1])), dm(N[2], e[2]));
-                            const double J[6] = {ds(dm(p[1], N[2]), dm(p[2], N[1])), ds(dm(p[2], N[0]), dm(p[0], N[2])),
-                                                 ds(dm(p[0], N[1]), dm(p[1], N[0])), N[0], N[1], N[2]};
-                            int k = 0;
-#pragma unroll
-                            for (int i = 0; i < 6; ++i)
-#pragma unroll
-                                for (int j = i; j < 6; ++j) t[k++] = dm(J[i], J[j]);
-#pragma unroll
-                            for (int i = 0; i < 6; ++i) t[21 + i] = dm(J[i], r);
-                            t[27] = dm(r, r);
-                            t[28] = 1.0;
-                        }
+                        if (da(da(dm(e[0], e[0]), dm(e[1], e[1])), dm(e[2], e[2])) <= a.ddiff2)
+                            point_to_plane_terms(p, N, e, t, 1);
                     }
                 }
             }
@@ -152,15 +141,7 @@ __global__ void __launch_bounds__(kTilePx) track_assoc_kernel(const TrackArgs a,
     }
 #pragma unroll
     for (int k = 0; k < kTerms; ++k) sm[k][lane] = t[k];
-    // fixed pairwise tree: lane i += lane i + 64, then i + 32, ... (absent pixels hold 0)
-    for (int s = kTilePx / 2; s > 0; s >>= 1) {
-        __syncthreads();
-        for (int j = lane; j < kTerms * s; j += kTilePx) {
-            const int k = j / s, i = j - k * s;
-            sm[k][i] = da(sm[k][i], sm[k][i + s]);
-        }
-    }
-    __syncthreads();
+    cta_halving_tree(sm);                // absent pixels add 0
     if (lane < kTerms) a.partials[((size_t)blockIdx.z * kTerms + lane) * a.P + blockIdx.y * a.tiles_x + blockIdx.x] = sm[lane][0];
 }
 
@@ -168,16 +149,7 @@ __global__ void __launch_bounds__(kSolveThreads) track_solve_kernel(const TrackA
     TrackFrame& f = a.frames[blockIdx.x];
     if (!report && !f.active) return;
     double* buf = a.partials + (size_t)blockIdx.x * kTerms * a.P;
-    // fixed pairwise tree over the tile partials padded to P = 2^k: i += i + P/2, then i + P/4, ...
-    for (int h = a.P / 2; h > 0; h >>= 1) {
-        for (int j = threadIdx.x; j < kTerms * h; j += kSolveThreads) {
-            const int k = j / h, i = j - k * h;
-            const double x = i < a.n_tiles ? buf[(size_t)k * a.P + i] : 0.0;
-            const double y = i + h < a.n_tiles ? buf[(size_t)k * a.P + i + h] : 0.0;
-            buf[(size_t)k * a.P + i] = da(x, y);
-        }
-        __syncthreads();
-    }
+    cta_tree_rows<kSolveThreads>(buf, kTerms, a.n_tiles, a.P);
     if (threadIdx.x != 0) return;
     double S[kTerms];
     for (int k = 0; k < kTerms; ++k) S[k] = buf[(size_t)k * a.P];
@@ -332,8 +304,7 @@ int otslam_volume_track_pyramid(otslam_volume* v, int n_frames, const uint16_t* 
         t.W = W; t.H = H;
         t.tiles_x = (W + kTileW - 1) / kTileW;
         t.n_tiles = t.tiles_x * ((H + kTileH - 1) / kTileH);
-        t.P = 1;
-        while (t.P < t.n_tiles) t.P *= 2;
+        t.P = pow2_at_least(t.n_tiles);
         t.scale = (float)depth_scale;
         t.dmax = depth_max; t.ddiff2 = depth_diff[l] * depth_diff[l];
         t.fx = li[0]; t.fy = li[1]; t.cx = li[2]; t.cy = li[3];

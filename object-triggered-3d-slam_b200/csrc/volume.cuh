@@ -136,6 +136,4 @@ inline HashTable volume_hash(const otslam_volume* v) { return {v->d_keys, v->d_v
 // grow); pool chunks for blocks_needed slots
 int reserve_hash(otslam_volume* v, int64_t n_entries);
 int ensure_pool(otslam_volume* v, int64_t blocks_needed);
-// knn.cu: stable LSD radix sort of (u64 key, i32 value) pairs by the low `bits` bits; result in (kb, vb), (ka, va) clobbered
-int device_sort_pairs(uint64_t* ka, int32_t* va, uint64_t* kb, int32_t* vb, int64_t n, int bits, cudaStream_t s);
 }
