@@ -72,7 +72,8 @@ int otslam_selftest_ordered_sum(int64_t n, uint64_t seed, int pattern, uint64_t*
 
 /* ---- volume life cycle: o3d.pipelines.integration.ScalableTSDFVolume(voxel_length, sdf_trunc,
  *      color_type) (3d_model/reconstruct_rgbd.py:79-83); volume_unit_resolution = 16,
- *      depth_sampling_stride = 4 as in Open3D. `slab` may be NULL. */
+ *      depth_sampling_stride = 4 as in Open3D. `slab` may be NULL.  A failed allocation returns OTSLAM_ERR_NOMEM,
+ *      as in every other entry point. */
 int otslam_volume_create(double voxel_length, double sdf_trunc, int color_type, int device,
                          const otslam_slab_spec* slab, otslam_volume** out);
 int otslam_volume_destroy(otslam_volume* v);
@@ -392,6 +393,7 @@ int otslam_grid_smart_paste(uint8_t* base, const uint8_t* overlay, int width, in
  * CMYK JPEG, interlaced or palette PNG, another image size ...): decode it with the stock decoder and otslam_decoder_put it;
  * 2 = missing or damaged (CRC / structure), the reference's "Read image failed". */
 typedef struct otslam_decoder otslam_decoder;
+/* a stream or event that cannot be created for lack of memory returns OTSLAM_ERR_NOMEM, as in every other entry point */
 int otslam_decoder_create(int device, int height, int width, int max_frames, otslam_decoder** out);
 int otslam_decoder_destroy(otslam_decoder* d);
 /* n <= max_frames files per kind, read by host threads; either path array may be NULL (kind not wanted) */

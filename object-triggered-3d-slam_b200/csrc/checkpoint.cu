@@ -258,20 +258,19 @@ __global__ void __launch_bounds__(256) ckpt_insert_kernel(const uint64_t* __rest
 // =============================================================================================
 // host side
 // =============================================================================================
-// page-locked staging pair, CUDA events per chunk (kernel / copy times), all released on every return path
+// page-locked staging pair, CUDA events per chunk (kernel / copy times); the I/O threads are joined on every return path
+// before the buffers and events go
 struct Staging {
-    void* host[2] = {nullptr, nullptr};
-    std::vector<cudaEvent_t> ev;     // per chunk: kernel start / end, copy start / end
+    PinnedArray<char, cudaHostAllocPortable> host[2];
+    std::vector<Event> ev;           // per chunk: kernel start / end, copy start / end
     std::thread io[2];
     ~Staging() {
         for (auto& t : io) if (t.joinable()) t.join();
-        for (void* p : host) if (p) cudaFreeHost(p);
-        for (cudaEvent_t e : ev) cudaEventDestroy(e);
     }
     int init(int n_chunks) {
-        for (auto& p : host) OT_CUDA(cudaHostAlloc(&p, (size_t)kCkptChunk * kBlockFileBytes, cudaHostAllocPortable));
-        ev.assign((size_t)n_chunks * 4, nullptr);
-        for (auto& e : ev) OT_CUDA(cudaEventCreate(&e));
+        for (auto& p : host) OT_CUDA(p.reserve((size_t)kCkptChunk * kBlockFileBytes));
+        ev.resize((size_t)n_chunks * 4);
+        for (auto& e : ev) OT_CUDA(e.create());
         return OTSLAM_OK;
     }
     void join(int b) { if (io[b].joinable()) io[b].join(); }
@@ -378,16 +377,16 @@ int otslam_volume_save(otslam_volume* v, const char* path) {
             const int b = c & 1, j0 = c * kCkptChunk, nb = std::min(kCkptChunk, m - j0);
             st.join(b);                                           // chunk c-2's write from host[b] is done
             if (!io_ok) break;
-            cudaEvent_t* e = &st.ev[(size_t)c * 4];
+            const Event* e = &st.ev[(size_t)c * 4];
             OT_CUDA(cudaEventRecord(e[0], s));
-            ckpt_gather_kernel<<<nb, 256, 0, s>>>(v->d_chunks, slots.p + j0, keys3.p + (size_t)j0 * 3, stage[b].p, cks.p + j0);
+            ckpt_gather_kernel<<<nb, 256, 0, s>>>(v->d_chunks.p, slots.p + j0, keys3.p + (size_t)j0 * 3, stage[b].p, cks.p + j0);
             OT_LAUNCHED();
             OT_CUDA(cudaEventRecord(e[1], s));
             OT_CUDA(cudaEventRecord(e[2], s));
-            OT_CUDA(cudaMemcpyAsync(st.host[b], stage[b].p, (size_t)nb * kBlockFileBytes, cudaMemcpyDeviceToHost, s));
+            OT_CUDA(cudaMemcpyAsync(st.host[b].p, stage[b].p, (size_t)nb * kBlockFileBytes, cudaMemcpyDeviceToHost, s));
             OT_CUDA(cudaEventRecord(e[3], s));
             const int dev = v->device, fd = f.fd;
-            void* src = st.host[b];
+            void* src = st.host[b].p;
             const int64_t off = L.rec_off + (int64_t)j0 * kBlockFileBytes;
             st.io[b] = std::thread([=, &file_ns, &io_ok]() {      // overlaps the gather + copy of chunk c+1
                 cudaSetDevice(dev);
@@ -460,7 +459,7 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
         int64_t total = 0;
         OT_CUDA(cudaMemcpyAsync(&hb, bad.p, 4, cudaMemcpyDeviceToHost, s));
         OT_CUDA(cudaMemcpyAsync(&total, pos.p + n, 8, cudaMemcpyDeviceToHost, s));
-        OT_CUDA(cudaMemcpyAsync(&base, v->d_counters + kPoolCount, 4, cudaMemcpyDeviceToHost, s));   // first free pool slot
+        OT_CUDA(cudaMemcpyAsync(&base, v->d_counters.p + kPoolCount, 4, cudaMemcpyDeviceToHost, s));   // first free pool slot
         OT_CUDA(cudaStreamSynchronize(s));
         if (hb & kBadRange) return set_error(OTSLAM_ERR_OVERFLOW, "checkpoint block key outside the volume's key range (arena objects: |kx| < 2^17)");
         if (hb & kBadOrder) return set_error(OTSLAM_ERR_FORMAT, "checkpoint keys are not strictly ascending (duplicate or unordered key)");
@@ -487,7 +486,7 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
                 const int b = c & 1, j0 = c * kCkptChunk, j1 = std::min(m, j0 + kCkptChunk);
                 cudaSetDevice(v->device);
                 if (c >= 2 && cudaEventSynchronize(st.ev[(size_t)(c - 2) * 4 + 3]) != cudaSuccess) { io_ok = false; return; }
-                char* dst = static_cast<char*>(st.host[b]);
+                char* dst = st.host[b].p;
                 for (int j = j0; j < j1;) {
                     int k = j + 1;
                     while (k < j1 && hidx[(size_t)k] == hidx[(size_t)k - 1] + 1) ++k;
@@ -505,18 +504,18 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
                     st.join(b);
                     if (!io_ok) return set_error(OTSLAM_ERR_FORMAT, std::string("cannot read the records of ") + path);
                     if (c + 1 < n_chunks) st.io[b ^ 1] = std::thread(read_chunk, c + 1);   // overlaps the copy + verify of chunk c
-                    cudaEvent_t* e = &st.ev[(size_t)c * 4];
+                    const Event* e = &st.ev[(size_t)c * 4];
                     OT_CUDA(cudaEventRecord(e[2], s));
                     for (int j = 0; j < nb;) {              // whole blocks into their slots, split at pool-chunk boundaries
                         const int slot = base + j0 + j, run = std::min(nb - j, kChunkBlocks - (slot & (kChunkBlocks - 1)));
-                        OT_CUDA(cudaMemcpyAsync(v->chunks[(size_t)(slot >> kChunkBlocksLog2)] + (size_t)(slot & (kChunkBlocks - 1)) * kVox,
-                                                static_cast<char*>(st.host[b]) + (size_t)j * kBlockFileBytes, (size_t)run * kBlockFileBytes,
+                        OT_CUDA(cudaMemcpyAsync(v->chunks[(size_t)(slot >> kChunkBlocksLog2)].p + (size_t)(slot & (kChunkBlocks - 1)) * kVox,
+                                                st.host[b].p + (size_t)j * kBlockFileBytes, (size_t)run * kBlockFileBytes,
                                                 cudaMemcpyHostToDevice, s));
                         j += run;
                     }
                     OT_CUDA(cudaEventRecord(e[3], s));
                     OT_CUDA(cudaEventRecord(e[0], s));
-                    ckpt_verify_kernel<<<nb, 256, 0, s>>>(v->d_chunks, base + j0, kept_idx.p + j0, keys3.p, cks.p, frames, no_color, bad.p);
+                    ckpt_verify_kernel<<<nb, 256, 0, s>>>(v->d_chunks.p, base + j0, kept_idx.p + j0, keys3.p, cks.p, frames, no_color, bad.p);
                     OT_LAUNCHED();
                     OT_CUDA(cudaEventRecord(e[1], s));
                 }
@@ -532,7 +531,7 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
                 cudaStreamSynchronize(s);
                 for (int j = 0; j < m;) {
                     const int slot = base + j, run = std::min(m - j, kChunkBlocks - (slot & (kChunkBlocks - 1)));
-                    cudaMemsetAsync(v->chunks[(size_t)(slot >> kChunkBlocksLog2)] + (size_t)(slot & (kChunkBlocks - 1)) * kVox, 0,
+                    cudaMemsetAsync(v->chunks[(size_t)(slot >> kChunkBlocksLog2)].p + (size_t)(slot & (kChunkBlocks - 1)) * kVox, 0,
                                     (size_t)run * kBlockFileBytes, s);
                     j += run;
                 }
@@ -541,18 +540,17 @@ int otslam_volume_load(otslam_volume* v, const char* path, int64_t* n_loaded) {
             }
             // every check passed: insert
             OT_TRY(reserve_hash(v, (int64_t)base + m));
-            cudaEvent_t ei[2];
-            OT_CUDA(cudaEventCreate(&ei[0])); OT_CUDA(cudaEventCreate(&ei[1]));
+            Event ei[2];
+            OT_CUDA(ei[0].create()); OT_CUDA(ei[1].create());
             OT_CUDA(cudaEventRecord(ei[0], s));
             ckpt_insert_kernel<<<(m + 255) / 256, 256, 0, s>>>(kept_keys.p, m, base, volume_hash(v));
             OT_LAUNCHED();
             OT_CUDA(cudaEventRecord(ei[1], s));
             const int pool = base + m;
-            OT_CUDA(cudaMemcpyAsync(v->d_counters + kPoolCount, &pool, 4, cudaMemcpyHostToDevice, s));
+            OT_CUDA(cudaMemcpyAsync(v->d_counters.p + kPoolCount, &pool, 4, cudaMemcpyHostToDevice, s));
             OT_CUDA(cudaStreamSynchronize(s));
             float ins_ms = 0.f;
             cudaEventElapsedTime(&ins_ms, ei[0], ei[1]);
-            cudaEventDestroy(ei[0]); cudaEventDestroy(ei[1]);
             st.times(g_ckpt_prof[0], g_ckpt_prof[1]);
             g_ckpt_prof[0] += ins_ms;
             v->n_blocks = pool;

@@ -3,9 +3,11 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <algorithm>
 #include <atomic>
 #include <cstdio>
 #include <string>
+#include <utility>
 
 #include "../../include/otslam_b200.h"
 
@@ -206,16 +208,82 @@ struct DevBuf {
     }
 };
 
+// ---- owning handles for the long-lived resources (the volume, the decoder, checkpoint staging): move-only, released by
+// the destructor.  Unlike DevBuf they bypass the scratch cache: cudaMalloc / cudaHostAlloc, freed when the owner goes.
+// DeviceArray<T> / PinnedArray<T>: an array's capacity is 0 whenever its pointer is null.
+template <typename T, bool kPinned, unsigned kHostFlags = cudaHostAllocDefault>
+struct CudaArray {
+    T* p = nullptr;
+    size_t cap = 0;
+    CudaArray() = default;
+    CudaArray(CudaArray&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    CudaArray& operator=(CudaArray&& o) noexcept {
+        if (this != &o) { release(); std::swap(p, o.p); std::swap(cap, o.cap); }
+        return *this;
+    }
+    ~CudaArray() { release(); }
+    void release() {
+        if (p) { if constexpr (kPinned) cudaFreeHost(p); else cudaFree(p); }
+        p = nullptr;
+        cap = 0;
+    }
+    // room for n elements: with less, frees the old allocation and allocates max(n, want) ({nullptr, 0} if that fails)
+    cudaError_t reserve(size_t n, size_t want = 0) {
+        if (n <= cap) return cudaSuccess;
+        release();
+        want = std::max(n, want);
+        cudaError_t e;
+        if constexpr (kPinned) e = cudaHostAlloc((void**)&p, want * sizeof(T), kHostFlags);
+        else e = cudaMalloc((void**)&p, want * sizeof(T));
+        if (e == cudaSuccess) cap = want;
+        else p = nullptr;
+        return e;
+    }
+};
+template <typename T>
+using DeviceArray = CudaArray<T, false>;
+template <typename T, unsigned kHostFlags = cudaHostAllocDefault>
+using PinnedArray = CudaArray<T, true, kHostFlags>;
+
+// Event / Stream: null until create() succeeds; convert to the raw handle
+template <typename H, cudaError_t (*kDestroy)(H)>
+struct CudaHandle {
+    H h = nullptr;
+    CudaHandle() = default;
+    CudaHandle(CudaHandle&& o) noexcept : h(o.h) { o.h = nullptr; }
+    ~CudaHandle() { reset(); }
+    void reset(H n = nullptr) {
+        if (h) kDestroy(h);
+        h = n;
+    }
+    operator H() const { return h; }
+};
+struct Event : CudaHandle<cudaEvent_t, cudaEventDestroy> {
+    cudaError_t create(unsigned flags = cudaEventDefault) {
+        cudaEvent_t e = nullptr;
+        const cudaError_t r = cudaEventCreateWithFlags(&e, flags);
+        if (r == cudaSuccess) reset(e);
+        return r;
+    }
+};
+struct Stream : CudaHandle<cudaStream_t, cudaStreamDestroy> {
+    cudaError_t create(unsigned flags, int priority = 0) {   // 0: the default priority
+        cudaStream_t s = nullptr;
+        const cudaError_t r = cudaStreamCreateWithPriority(&s, flags, priority);
+        if (r == cudaSuccess) reset(s);
+        return r;
+    }
+};
+
 // Device-side duration of a stateless operator's kernel section (uploads before it and downloads
 // after it excluded): events on the operators' stream, read back by otslam_last_op_device_ms().
 struct OpTimer {
-    cudaEvent_t a = nullptr, b = nullptr;
+    Event a, b;
     bool stopped = false;
     cudaStream_t st;
     explicit OpTimer(cudaStream_t s = 0) : st(s) {
         g_last_op_ms = -1.0;
-        if (cudaEventCreate(&a) != cudaSuccess || cudaEventCreate(&b) != cudaSuccess) { a = b = nullptr; return; }
-        cudaEventRecord(a, st);
+        if (a.create() == cudaSuccess && b.create() == cudaSuccess) cudaEventRecord(a, st);
     }
     void stop() {
         if (!stopped && b) cudaEventRecord(b, st);
@@ -225,8 +293,6 @@ struct OpTimer {
         stop();
         float ms = 0.f;
         if (b && cudaEventSynchronize(b) == cudaSuccess && cudaEventElapsedTime(&ms, a, b) == cudaSuccess) g_last_op_ms = ms;
-        if (a) cudaEventDestroy(a);
-        if (b) cudaEventDestroy(b);
     }
 };
 

@@ -500,7 +500,7 @@ static int make_ctx(otslam_volume* v, ExtractCtx& c) {
     OT_TRY(volume_selected_blocks_device(v, &dk, &ds, &n, &x_off));
     c.x_off = x_off;
     c.arena = v->n_objects > 0;
-    c.table = volume_hash(v); c.chunks = v->d_chunks;
+    c.table = volume_hash(v); c.chunks = v->d_chunks.p;
     c.bkeys = dk; c.bslots = ds; c.n = n; c.slab = v->slab;
     c.vl = v->voxel_length; c.half = 0.5 * v->voxel_length; c.unit = v->unit_length;
     return OTSLAM_OK;

@@ -28,6 +28,7 @@
 #include <cstdlib>
 #include <cstring>
 #include <map>
+#include <memory>
 #include <string>
 #include <thread>
 #include <vector>
@@ -189,38 +190,11 @@ __global__ void __launch_bounds__(256) jpeg_color_kernel(const JpegFrame* __rest
 // ---------------------------------------------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------------------------------------------
+// decoder buffers grow with head room (pinned n / 2, device n / 4) unless the call site asks for more
 template <typename T>
-struct Pinned {                   // page-locked, grows geometrically
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n, size_t want = 0) {              // need n elements; when growing, allocate `want` (>= n)
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFreeHost(p);
-        p = nullptr;
-        cap = 0;
-        want = std::max(want, n + n / 2);
-        cudaError_t e = cudaHostAlloc((void**)&p, want * sizeof(T), cudaHostAllocDefault);
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    ~Pinned() { if (p) cudaFreeHost(p); }
-};
+cudaError_t grow(PinnedArray<T>& a, size_t n, size_t want = 0) { return a.reserve(n, std::max(want, n + n / 2)); }
 template <typename T>
-struct Device {
-    T* p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t n, size_t want = 0) {
-        if (n <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-        want = std::max(want, n + n / 4);
-        cudaError_t e = cudaMalloc((void**)&p, want * sizeof(T));
-        if (e == cudaSuccess) cap = want;
-        return e;
-    }
-    ~Device() { if (p) cudaFree(p); }
-};
+cudaError_t grow(DeviceArray<T>& a, size_t n, size_t want = 0) { return a.reserve(n, std::max(want, n + n / 4)); }
 
 int host_threads() {
     const char* e = getenv("OTSLAM_DECODE_THREADS");
@@ -273,27 +247,22 @@ bool read_file(const char* path, std::vector<uint8_t>& out) {
 
 struct otslam_decoder {
     int device = 0, H = 0, W = 0, max_frames = 0;
-    cudaStream_t s_png = nullptr, s_jpg = nullptr;
-    cudaEvent_t ev[8] = {};
-    Pinned<uint8_t> h_zblob, h_jblob;
-    Device<uint8_t> d_zblob, d_jblob, d_raw, d_samples, d_rgb;
-    Device<uint16_t> d_depth;
-    Device<int16_t> d_coef;
-    Pinned<PngJob> h_jobs;
-    Device<PngJob> d_jobs;
-    Pinned<JpegFrame> h_frames;
-    Device<JpegFrame> d_frames;
-    Pinned<JpegTables> h_tables;
-    Device<JpegTables> d_tables;
-    Pinned<int32_t> h_status, h_slots;
-    Device<int32_t> d_status, d_slots;
+    Stream s_png, s_jpg;
+    Event ev[8];
+    PinnedArray<uint8_t> h_zblob, h_jblob;
+    DeviceArray<uint8_t> d_zblob, d_jblob, d_raw, d_samples, d_rgb;
+    DeviceArray<uint16_t> d_depth;
+    DeviceArray<int16_t> d_coef;
+    PinnedArray<PngJob> h_jobs;
+    DeviceArray<PngJob> d_jobs;
+    PinnedArray<JpegFrame> h_frames;
+    DeviceArray<JpegFrame> d_frames;
+    PinnedArray<JpegTables> h_tables;
+    DeviceArray<JpegTables> d_tables;
+    PinnedArray<int32_t> h_status, h_slots;
+    DeviceArray<int32_t> d_status, d_slots;
     int n_decoded = 0;
     double ms[6] = {};
-    ~otslam_decoder() {
-        for (auto& e : ev) if (e) cudaEventDestroy(e);
-        if (s_png) cudaStreamDestroy(s_png);
-        if (s_jpg) cudaStreamDestroy(s_jpg);
-    }
 };
 
 namespace {
@@ -335,13 +304,13 @@ int decode_sources(otslam_decoder* d, int n, const Source* color, const Source* 
     }
     const int n_png = (int)png_src.size(), n_jpg = (int)jpg_src.size();
     const size_t cap_jobs = (size_t)d->max_frames * 2;           // data-independent sizes: see the device buffers below
-    OT_CUDA(d->h_zblob.reserve((size_t)ztotal + 16, (size_t)ztotal * 2 + 16));
-    OT_CUDA(d->h_jblob.reserve((size_t)jtotal + 16, (size_t)jtotal * 2 + 16));
-    OT_CUDA(d->h_jobs.reserve(std::max(1, n_png), cap_jobs));
-    OT_CUDA(d->h_frames.reserve(std::max(1, n_jpg), (size_t)d->max_frames));
-    OT_CUDA(d->h_tables.reserve(kMaxTableSets));
-    OT_CUDA(d->h_status.reserve((size_t)std::max(1, n_png + n_jpg), cap_jobs));
-    OT_CUDA(d->h_slots.reserve((size_t)std::max(1, n_jpg), (size_t)d->max_frames));
+    OT_CUDA(grow(d->h_zblob, (size_t)ztotal + 16, (size_t)ztotal * 2 + 16));
+    OT_CUDA(grow(d->h_jblob, (size_t)jtotal + 16, (size_t)jtotal * 2 + 16));
+    OT_CUDA(grow(d->h_jobs, std::max(1, n_png), cap_jobs));
+    OT_CUDA(grow(d->h_frames, std::max(1, n_jpg), (size_t)d->max_frames));
+    OT_CUDA(grow(d->h_tables, kMaxTableSets));
+    OT_CUDA(grow(d->h_status, (size_t)std::max(1, n_png + n_jpg), cap_jobs));
+    OT_CUDA(grow(d->h_slots, (size_t)std::max(1, n_jpg), (size_t)d->max_frames));
 
     // ---- parse in parallel: PNG chunk walk + CRC + IDAT compaction; JPEG marker walk + scan copy
     std::vector<JpegHeader> jhdr((size_t)n_jpg);
@@ -425,18 +394,18 @@ int decode_sources(otslam_decoder* d, int n, const Source* color, const Source* 
     for (int q = 0; q < n_jpg; ++q)
         if (d->h_frames.p[q].status == IC_OK) blk_frame = std::max<int64_t>(blk_frame, d->h_frames.p[q].n_blocks);
     const size_t cap_frames = (size_t)d->max_frames * ((depth ? 1 : 0) + (color ? 1 : 0));      // >= n_png, >= n_jpg
-    OT_CUDA(d->d_zblob.reserve((size_t)ztotal + 16, (size_t)ztotal * 2 + 16));
-    OT_CUDA(d->d_jblob.reserve((size_t)jtotal + 16, (size_t)jtotal * 2 + 16));
-    OT_CUDA(d->d_raw.reserve((size_t)raw_total + 16, cap_frames * (size_t)raw_frame + 16));
-    OT_CUDA(d->d_coef.reserve((size_t)blk_total * 64 + 64, (size_t)d->max_frames * (size_t)blk_frame * 64 + 64));
-    OT_CUDA(d->d_samples.reserve((size_t)blk_total * 64 + 64, (size_t)d->max_frames * (size_t)blk_frame * 64 + 64));
-    OT_CUDA(d->d_jobs.reserve(std::max(1, n_png), cap_frames));
-    OT_CUDA(d->d_frames.reserve(std::max(1, n_jpg), (size_t)d->max_frames));
-    OT_CUDA(d->d_tables.reserve(kMaxTableSets));
-    OT_CUDA(d->d_status.reserve((size_t)std::max(1, n_png + n_jpg), cap_frames));
-    OT_CUDA(d->d_slots.reserve((size_t)std::max(1, n_jpg), (size_t)d->max_frames));
-    if (depth) OT_CUDA(d->d_depth.reserve((size_t)d->max_frames * px));
-    if (color) OT_CUDA(d->d_rgb.reserve((size_t)d->max_frames * px * 3));
+    OT_CUDA(grow(d->d_zblob, (size_t)ztotal + 16, (size_t)ztotal * 2 + 16));
+    OT_CUDA(grow(d->d_jblob, (size_t)jtotal + 16, (size_t)jtotal * 2 + 16));
+    OT_CUDA(grow(d->d_raw, (size_t)raw_total + 16, cap_frames * (size_t)raw_frame + 16));
+    OT_CUDA(grow(d->d_coef, (size_t)blk_total * 64 + 64, (size_t)d->max_frames * (size_t)blk_frame * 64 + 64));
+    OT_CUDA(grow(d->d_samples, (size_t)blk_total * 64 + 64, (size_t)d->max_frames * (size_t)blk_frame * 64 + 64));
+    OT_CUDA(grow(d->d_jobs, std::max(1, n_png), cap_frames));
+    OT_CUDA(grow(d->d_frames, std::max(1, n_jpg), (size_t)d->max_frames));
+    OT_CUDA(grow(d->d_tables, kMaxTableSets));
+    OT_CUDA(grow(d->d_status, (size_t)std::max(1, n_png + n_jpg), cap_frames));
+    OT_CUDA(grow(d->d_slots, (size_t)std::max(1, n_jpg), (size_t)d->max_frames));
+    if (depth) OT_CUDA(grow(d->d_depth, (size_t)d->max_frames * px));
+    if (color) OT_CUDA(grow(d->d_rgb, (size_t)d->max_frames * px * 3));
 
     // ---- PNG stream
     cudaStream_t sp = d->s_png, sj = d->s_jpg;
@@ -524,20 +493,15 @@ int otslam_decoder_create(int device, int height, int width, int max_frames, ots
         return set_error(OTSLAM_ERR_INVALID, "decoder_create: bad arguments (max_frames <= 16384, height x width <= 2^28)");
     *out = nullptr;
     OT_TRY(use_device(device));
-    auto* d = new otslam_decoder();
+    std::unique_ptr<otslam_decoder> d(new otslam_decoder());
     d->device = device;
     d->H = height;
     d->W = width;
     d->max_frames = max_frames;
-    cudaError_t e = cudaStreamCreateWithFlags(&d->s_png, cudaStreamNonBlocking);
-    if (e == cudaSuccess) e = cudaStreamCreateWithFlags(&d->s_jpg, cudaStreamNonBlocking);
-    for (auto& ev : d->ev)
-        if (e == cudaSuccess) e = cudaEventCreate(&ev);
-    if (e != cudaSuccess) {
-        delete d;
-        return set_error(OTSLAM_ERR_CUDA, std::string("decoder_create: ") + cudaGetErrorString(e));
-    }
-    *out = d;
+    OT_CUDA(d->s_png.create(cudaStreamNonBlocking));
+    OT_CUDA(d->s_jpg.create(cudaStreamNonBlocking));
+    for (auto& ev : d->ev) OT_CUDA(ev.create());
+    *out = d.release();
     return OTSLAM_OK;
 }
 
@@ -595,11 +559,11 @@ int otslam_decoder_put(otslam_decoder* d, int slot, const uint16_t* depth, const
     OT_TRY(use_device(d->device));
     const size_t px = (size_t)d->H * d->W;
     if (depth) {
-        OT_CUDA(d->d_depth.reserve((size_t)d->max_frames * px));
+        OT_CUDA(grow(d->d_depth, (size_t)d->max_frames * px));
         OT_CUDA(cudaMemcpy(d->d_depth.p + (size_t)slot * px, depth, px * 2, cudaMemcpyDefault));
     }
     if (rgb) {
-        OT_CUDA(d->d_rgb.reserve((size_t)d->max_frames * px * 3));
+        OT_CUDA(grow(d->d_rgb, (size_t)d->max_frames * px * 3));
         OT_CUDA(cudaMemcpy(d->d_rgb.p + (size_t)slot * px * 3, rgb, px * 3, cudaMemcpyDefault));
     }
     return OTSLAM_OK;

@@ -219,11 +219,6 @@ static float ray_len(int u, int v, float cx, float cy, float ifx, float ify) {
     return std::sqrt((xc * xc + yc * yc) + 1.0f);
 }
 
-struct EventPair {
-    cudaEvent_t e[2] = {nullptr, nullptr};
-    ~EventPair() { for (cudaEvent_t x : e) if (x) cudaEventDestroy(x); }
-};
-
 bool ray_view(const double* e, RayView* out) {
     double pose[16];
     if (!finite_all(e, 16) || !inverse4(e, pose)) return false;
@@ -257,7 +252,7 @@ int ray_args(const otslam_volume* v, int width, int height, const double intr[4]
     a.cap = (int)raycast_cap(depth_min, depth_max, max_len, v->voxel_length);
     a.color = v->color_type == OTSLAM_COLOR_RGB8;
     a.gap = 0.99 * v->voxel_length;
-    a.c.table = volume_hash(v); a.c.chunks = v->d_chunks;
+    a.c.table = volume_hash(v); a.c.chunks = v->d_chunks.p;
     a.c.bkeys = nullptr; a.c.bslots = nullptr; a.c.n = 0; a.c.slab = v->slab;
     a.c.vl = v->voxel_length; a.c.half = 0.5 * v->voxel_length; a.c.unit = v->unit_length;
     a.c.x_off = v->n_objects > 0 ? obj_key_offset(v->sel_obj) : 0;
@@ -327,11 +322,11 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
     OT_CUDA(d_views.alloc((size_t)n_views)); OT_CUDA(d_hits.alloc(1));
     if (host_bytes_per_view)
         for (auto& b : staging) OT_CUDA(b.alloc(host_bytes_per_view * (size_t)std::min(chunk, n_views)));
-    EventPair rendered, copied;
+    Event rendered[2], copied[2];
     if (host_bytes_per_view)
         for (int b = 0; b < 2; ++b) {
-            OT_CUDA(cudaEventCreateWithFlags(&rendered.e[b], cudaEventDisableTiming));
-            OT_CUDA(cudaEventCreateWithFlags(&copied.e[b], cudaEventDisableTiming));
+            OT_CUDA(rendered[b].create(cudaEventDisableTiming));
+            OT_CUDA(copied[b].create(cudaEventDisableTiming));
         }
     OT_CUDA(cudaMemcpyAsync(d_views.p, views.data(), sizeof(RayView) * views.size(), cudaMemcpyHostToDevice, s));
     OT_CUDA(cudaMemsetAsync(d_hits.p, 0, 8, s));
@@ -341,7 +336,7 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
         for (int first = 0, k = 0; first < n_views; first += chunk, ++k) {
             const int nv = std::min(chunk, n_views - first);
             const int buf = k & 1;
-            if (host_bytes_per_view && k >= 2) OT_CUDA(cudaStreamWaitEvent(s, copied.e[buf], 0));   // staging buffer free again
+            if (host_bytes_per_view && k >= 2) OT_CUDA(cudaStreamWaitEvent(s, copied[buf], 0));   // staging buffer free again
             uint8_t* stage = host_bytes_per_view ? staging[buf].p : nullptr;
             uint8_t* dst[4];
             size_t off = 0;
@@ -353,13 +348,13 @@ int otslam_volume_raycast(otslam_volume* v, int n_views, int width, int height, 
             }
             OT_TRY(raycast_launch(a, d_views.p + first, nv, (float*)dst[0], (float*)dst[1], (float*)dst[2], dst[3], s));
             if (host_bytes_per_view) {
-                OT_CUDA(cudaEventRecord(rendered.e[buf], s));
-                OT_CUDA(cudaStreamWaitEvent(cs, rendered.e[buf], 0));
+                OT_CUDA(cudaEventRecord(rendered[buf], s));
+                OT_CUDA(cudaStreamWaitEvent(cs, rendered[buf], 0));
                 for (int j = 0; j < 4; ++j)
                     if (outs[j] && host[j])
                         OT_CUDA(cudaMemcpyAsync((uint8_t*)outs[j] + elem[j] * (size_t)px * first, dst[j], elem[j] * (size_t)px * nv,
                                                 cudaMemcpyDeviceToHost, cs));
-                OT_CUDA(cudaEventRecord(copied.e[buf], cs));
+                OT_CUDA(cudaEventRecord(copied[buf], cs));
             }
         }
         timer.stop();

@@ -43,6 +43,19 @@ struct PointsResult {
     void release();
 };
 
+// block hash (hash_table.cuh): the entry index is the handle used by the per-batch work list.  Built whole or not at all
+// (volume.cu: new_hash).
+struct BlockHash {
+    uint32_t cap = 0;
+    DeviceArray<uint64_t> keys;
+    DeviceArray<int32_t> vals;     // entry -> pool slot
+    // kNB-buffered per batch: allocation of batches b+1, b+2 runs on pre_stream while batch b integrates
+    DeviceArray<uint32_t> masks[kNB];   // entry -> bit f set when frame f of the batch touches it
+    DeviceArray<int32_t> list[kNB];     // entries touched by the batch (each once)
+    DeviceArray<int32_t> order[kNB];    // the same entries, most-frames-first (launch order of the integration CTAs)
+    DeviceArray<uint32_t> lmask[kNB];   // their frame masks in that order (the hash-side masks are cleared when this is built)
+};
+
 }  // namespace otslam
 
 struct otslam_volume {
@@ -50,8 +63,8 @@ struct otslam_volume {
     double voxel_length = 0, sdf_trunc = 0, unit_length = 0;
     int color_type = OTSLAM_COLOR_RGB8;
     otslam::SlabSpec slab{0, 8, 1, 0, 1};
-    cudaStream_t stream = nullptr, copy_stream = nullptr, pre_stream = nullptr;
-    bool own_stream = true;
+    otslam::Stream main_stream, copy_stream, pre_stream;
+    cudaStream_t stream = nullptr;         // main_stream, or the caller's (otslam_volume_set_stream)
     int batch = otslam::kMaxBatch;
     int zsplit = 0;                // CTAs per block along z in the integration kernel: 0 = default (2), 1, 2, 4, 8
     int n_objects = 0;             // > 0: multi-object arena (object id in the block key), see common.cuh
@@ -59,40 +72,31 @@ struct otslam_volume {
     int64_t obj_frames[otslam::kMaxObjects] = {};   // frames integrated per object (the 65535 limit is per voxel)
     int64_t frames_integrated = 0;
 
-    // block hash (hash_table.cuh; volume_hash() below): the entry index is the handle used by the per-batch work list
-    uint32_t cap = 0;
-    uint64_t* d_keys = nullptr;
-    int32_t* d_vals = nullptr;     // entry -> pool slot
-    // kNB-buffered per batch: allocation of batches b+1, b+2 runs on pre_stream while batch b integrates
-    uint32_t* d_masks[otslam::kNB] = {};   // entry -> bit f set when frame f of the batch touches it
-    int32_t* d_list[otslam::kNB] = {};     // entries touched by the batch (each once)
-    int32_t* d_order[otslam::kNB] = {};    // the same entries, most-frames-first (launch order of the integration CTAs)
-    uint32_t* d_lmask[otslam::kNB] = {};   // their frame masks in that order (the hash-side masks are cleared when this is built)
+    otslam::BlockHash hash;        // volume_hash() below
 
     // block pool: chunks of kChunkBlocks blocks, 64 KiB per block
-    std::vector<uint4*> chunks;
-    uint4** d_chunks = nullptr;
+    std::vector<otslam::DeviceArray<uint4>> chunks;
+    otslam::DeviceArray<uint4*> d_chunks;   // [kMaxChunks]
     int64_t n_blocks = 0;          // host mirror of the pool counter
 
-    int* d_counters = nullptr;
-    int* h_counters = nullptr;     // pinned [kNB][kNumCounters]
+    otslam::DeviceArray<int> d_counters;
+    otslam::PinnedArray<int> h_counters;     // [kNB][kNumCounters]
     std::vector<uint4*> h_chunk_table;   // never reallocates (reserved to kMaxChunks): async copies read from it
-    cudaEvent_t ev_pre_done[otslam::kNB] = {}, ev_k4_done[otslam::kNB] = {}, ev_main = nullptr;
+    otslam::Event ev_pre_done[otslam::kNB], ev_k4_done[otslam::kNB], ev_main;
 
     // frame staging (kNB buffers)
-    uint16_t* d_raw_depth[otslam::kNB] = {};
-    uint8_t* d_raw_rgb[otslam::kNB] = {};
-    uint2* d_packed[otslam::kNB] = {};
-    float* d_tiles[otslam::kNB] = {};      // max-depth tiles of the packed frames (integration kernel's brick cull)
+    otslam::DeviceArray<uint8_t> d_raw_depth[otslam::kNB];   // u16 or f32 frames as uploaded
+    otslam::DeviceArray<uint8_t> d_raw_rgb[otslam::kNB];
+    otslam::DeviceArray<uint2> d_packed[otslam::kNB];
+    otslam::DeviceArray<float> d_tiles[otslam::kNB];        // max-depth tiles of the packed frames (integration kernel's brick cull)
     bool cull = true;                      // OTSLAM_K4_CULL=0 turns the brick cull off (results are the same)
-    size_t raw_frames_cap = 0, raw_px_cap = 0, packed_cap = 0, packed_px = 0, tiles_cap = 0;
-    size_t raw_depth_bytes_per_px = 2;
-    cudaEvent_t ev_copied[otslam::kNB] = {}, ev_raw_free[otslam::kNB] = {};
-    otslam::FrameDev* d_frames[otslam::kNB] = {};
-    otslam::FrameDev* h_frames = nullptr;  // pinned [kNB][kMaxBatch]
+    size_t packed_px = 0;                  // image size of d_packed's zero sentinels
+    otslam::Event ev_copied[otslam::kNB], ev_raw_free[otslam::kNB];
+    otslam::DeviceArray<otslam::FrameDev> d_frames[otslam::kNB];   // [kMaxBatch]
+    otslam::PinnedArray<otslam::FrameDev> h_frames;               // [kNB][kMaxBatch]
 
     // depth->camera-distance multiplier image, cached per intrinsics (SURVEY A.2)
-    float* d_mult = nullptr;
+    otslam::DeviceArray<float> d_mult;
     int mult_w = 0, mult_h = 0;
     double mult_intr[4] = {0, 0, 0, 0};
 
@@ -100,7 +104,7 @@ struct otslam_volume {
     bool profiling = false;
     double prof_ms[4] = {0, 0, 0, 0};
     int64_t prof_launches[4] = {0, 0, 0, 0};
-    std::vector<cudaEvent_t> prof_events;          // pairs, recycled
+    std::vector<otslam::Event> prof_events;        // pairs, recycled
     std::vector<int> prof_pending;                 // kernel id per recorded pair
     size_t prof_used = 0;
 
@@ -120,7 +124,9 @@ struct otslam_volume {
     int64_t n_halo = 0;
     std::vector<int64_t> halo_counts;    // pieces per destination rank
 
-    cudaEvent_t ev_ext = nullptr;        // otslam_volume_wait_stream
+    otslam::Event ev_ext;                // otslam_volume_wait_stream
+
+    ~otslam_volume();                    // drains the streams, releases the scratch-cache results
 };
 
 namespace otslam {
@@ -131,7 +137,7 @@ int volume_selected_blocks_device(otslam_volume* v, const uint64_t** d_keys, con
 // the same downloaded to the host (export_blocks)
 int volume_sorted_blocks(otslam_volume* v, std::vector<uint64_t>& keys, std::vector<int32_t>& slots);
 // the volume's block hash as the kernels take it
-inline HashTable volume_hash(const otslam_volume* v) { return {v->d_keys, v->d_vals, v->cap - 1}; }
+inline HashTable volume_hash(const otslam_volume* v) { return {v->hash.keys.p, v->hash.vals.p, v->hash.cap - 1}; }
 // volume.cu, used by checkpoint.cu: grow the block hash until it holds n_entries (drains both streams first when it must
 // grow); pool chunks for blocks_needed slots
 int reserve_hash(otslam_volume* v, int64_t n_entries);
