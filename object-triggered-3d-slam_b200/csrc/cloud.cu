@@ -309,9 +309,8 @@ int otslam_backproject_rgbd(const float* depth_m, const uint8_t* rgb, int width,
     a.W = width; a.H = height; a.fx = intr[0]; a.fy = intr[1]; a.cx = intr[2]; a.cy = intr[3];
     DevBuf<float> dd;
     DevBuf<uint8_t> dc;
-    OT_CUDA(dd.alloc(n));
-    OT_CUDA(cudaMemcpy(dd.p, depth_m, n * 4, cudaMemcpyDefault));
-    if (rgb) { OT_CUDA(dc.alloc(n * 3)); OT_CUDA(cudaMemcpy(dc.p, rgb, n * 3, cudaMemcpyDefault)); }
+    OT_CUDA(dd.upload(depth_m, n));
+    if (rgb) OT_CUDA(dc.upload(rgb, n * 3));
     a.depth = dd.p; a.rgb = rgb ? dc.p : nullptr;
     DevBuf<int> counts;
     DevBuf<int64_t> base;
@@ -329,8 +328,9 @@ int otslam_backproject_rgbd(const float* depth_m, const uint8_t* rgb, int width,
     OT_CUDA(dp.alloc(m * 3));
     if (rgb && colors) OT_CUDA(dcol.alloc(m * 3));
     OT_TRY(launch((int)((n + kItemsPerCta - 1) / kItemsPerCta), base.p, nullptr));
-    OT_CUDA(cudaMemcpy(points, dp.p, m * 24, cudaMemcpyDefault));
-    if (rgb && colors) OT_CUDA(cudaMemcpy(colors, dcol.p, m * 24, cudaMemcpyDefault));
+    OT_CUDA(dp.download(points, m * 3));
+    if (rgb && colors) OT_CUDA(dcol.download(colors, m * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -342,11 +342,11 @@ int otslam_mesh_vertex_normals(const double* vertices, int64_t n_vertices, const
     OT_TRY(use_device(device));
     DevBuf<double> dv, dn;
     DevBuf<int32_t> df;
-    OT_CUDA(dv.alloc(n_vertices * 3)); OT_CUDA(dn.alloc(n_vertices * 3)); OT_CUDA(df.alloc(n_faces * 3));
-    OT_CUDA(cudaMemcpy(dv.p, vertices, n_vertices * 24, cudaMemcpyDefault));
-    if (n_faces) OT_CUDA(cudaMemcpy(df.p, faces, n_faces * 12, cudaMemcpyDefault));
+    OT_CUDA(dv.upload(vertices, n_vertices * 3)); OT_CUDA(dn.alloc(n_vertices * 3));
+    OT_CUDA(n_faces ? df.upload(faces, n_faces * 3) : df.alloc(0));
     OT_TRY(device_vertex_normals(dv.p, n_vertices, df.p, n_faces, dn.p, 0));
-    OT_CUDA(cudaMemcpy(normals, dn.p, n_vertices * 24, cudaMemcpyDefault));
+    OT_CUDA(dn.download(normals, n_vertices * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -359,12 +359,10 @@ int otslam_mesh_sample_uniform(const double* vertices, const double* colors, con
     OT_TRY(use_device(device));
     DevBuf<double> dv, dc, dn, area, total, op, oc, on;
     DevBuf<int32_t> df;
-    OT_CUDA(dv.alloc(n_vertices * 3)); OT_CUDA(df.alloc(n_faces * 3)); OT_CUDA(area.alloc(n_faces)); OT_CUDA(total.alloc(1));
-    OT_CUDA(cudaMemcpy(dv.p, vertices, n_vertices * 24, cudaMemcpyDefault));
-    OT_CUDA(cudaMemcpy(df.p, faces, n_faces * 12, cudaMemcpyDefault));
+    OT_CUDA(dv.upload(vertices, n_vertices * 3)); OT_CUDA(df.upload(faces, n_faces * 3)); OT_CUDA(area.alloc(n_faces)); OT_CUDA(total.alloc(1));
     const bool has_c = colors && out_colors, has_n = normals && out_normals;
-    if (has_c) { OT_CUDA(dc.alloc(n_vertices * 3)); OT_CUDA(cudaMemcpy(dc.p, colors, n_vertices * 24, cudaMemcpyDefault)); OT_CUDA(oc.alloc(n_samples * 3)); }
-    if (has_n) { OT_CUDA(dn.alloc(n_vertices * 3)); OT_CUDA(cudaMemcpy(dn.p, normals, n_vertices * 24, cudaMemcpyDefault)); OT_CUDA(on.alloc(n_samples * 3)); }
+    if (has_c) { OT_CUDA(dc.upload(colors, n_vertices * 3)); OT_CUDA(oc.alloc(n_samples * 3)); }
+    if (has_n) { OT_CUDA(dn.upload(normals, n_vertices * 3)); OT_CUDA(on.alloc(n_samples * 3)); }
     OT_CUDA(op.alloc(n_samples * 3));
     OpTimer timer;
     tri_area_kernel<<<(unsigned)((n_faces + 255) / 256), 256>>>(dv.p, df.p, n_faces, area.p);
@@ -375,9 +373,10 @@ int otslam_mesh_sample_uniform(const double* vertices, const double* colors, con
                                                                area.p, n_samples, seed, op.p, oc.p, on.p);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_points, op.p, n_samples * 24, cudaMemcpyDefault));
-    if (has_c) OT_CUDA(cudaMemcpy(out_colors, oc.p, n_samples * 24, cudaMemcpyDefault));
-    if (has_n) OT_CUDA(cudaMemcpy(out_normals, on.p, n_samples * 24, cudaMemcpyDefault));
+    OT_CUDA(op.download(out_points, n_samples * 3));
+    if (has_c) OT_CUDA(oc.download(out_colors, n_samples * 3));
+    if (has_n) OT_CUDA(on.download(out_normals, n_samples * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -396,12 +395,12 @@ int otslam_volume_mesh_sample(otslam_volume* v, int64_t n_samples, uint64_t seed
     if (out_normals) OT_CUDA(on.alloc(n_samples * 3));
     {
         OpTimer timer(s);
-        tri_area_kernel<<<(unsigned)((m.nf + 255) / 256), 256, 0, s>>>(m.d_verts, m.d_faces, m.nf, area.p);
+        tri_area_kernel<<<(unsigned)((m.nf + 255) / 256), 256, 0, s>>>(m.verts.p, m.faces.p, m.nf, area.p);
         OT_LAUNCHED();
         OT_TRY(device_ordered_sum(area.p, m.nf, 0, nullptr, 0.0, total.p, s));
         OT_TRY(device_ordered_sum(area.p, m.nf, 1, total.p, 0.0, nullptr, s));
-        sample_kernel<<<(unsigned)((n_samples + 255) / 256), 256, 0, s>>>(m.d_verts, out_colors ? m.d_colors : nullptr,
-                                                                          out_normals ? m.d_normals : nullptr, m.d_faces, m.nf, area.p,
+        sample_kernel<<<(unsigned)((n_samples + 255) / 256), 256, 0, s>>>(m.verts.p, out_colors ? m.colors.p : nullptr,
+                                                                          out_normals ? m.normals.p : nullptr, m.faces.p, m.nf, area.p,
                                                                           n_samples, seed, op.p, oc.p, on.p);
         OT_LAUNCHED();
     }
@@ -419,10 +418,9 @@ int otslam_cloud_zfilter(const double* points, const double* colors, int64_t n, 
     if (n == 0) return OTSLAM_OK;
     OT_TRY(use_device(device));
     DevBuf<double> dp, dc, op, oc;
-    OT_CUDA(dp.alloc(n * 3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
+    OT_CUDA(dp.upload(points, n * 3));
     const bool has_c = colors && out_colors;
-    if (has_c) { OT_CUDA(dc.alloc(n * 3)); OT_CUDA(cudaMemcpy(dc.p, colors, n * 24, cudaMemcpyDefault)); }
+    if (has_c) OT_CUDA(dc.upload(colors, n * 3));
     DevBuf<int> counts;
     DevBuf<int64_t> base;
     cudaStream_t s = 0;
@@ -440,8 +438,9 @@ int otslam_cloud_zfilter(const double* points, const double* colors, int64_t n, 
     if (has_c) OT_CUDA(oc.alloc(m * 3));
     OT_TRY(launch((int)((n + kItemsPerCta - 1) / kItemsPerCta), base.p, nullptr));
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_points, op.p, m * 24, cudaMemcpyDefault));
-    if (has_c) OT_CUDA(cudaMemcpy(out_colors, oc.p, m * 24, cudaMemcpyDefault));
+    OT_CUDA(op.download(out_points, m * 3));
+    if (has_c) OT_CUDA(oc.download(out_colors, m * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -451,8 +450,7 @@ int otslam_grid_to_points(const uint8_t* gray, int width, int height, double res
     OT_TRY(use_device(device));
     const int64_t n = (int64_t)width * height;
     DevBuf<uint8_t> di;
-    OT_CUDA(di.alloc(n));
-    OT_CUDA(cudaMemcpy(di.p, gray, n, cudaMemcpyDefault));
+    OT_CUDA(di.upload(gray, n));
     DevBuf<int> counts;
     DevBuf<int64_t> base;
     DevBuf<double> op;
@@ -470,7 +468,8 @@ int otslam_grid_to_points(const uint8_t* gray, int width, int height, double res
     OT_CUDA(op.alloc(m * 3));
     OT_TRY(launch((int)((n + kItemsPerCta - 1) / kItemsPerCta), base.p, nullptr));
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_points, op.p, m * 24, cudaMemcpyDefault));
+    OT_CUDA(op.download(out_points, m * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -480,16 +479,16 @@ static int rigid_apply(const double* points, const double* normals, int64_t n, c
     if (n == 0) return OTSLAM_OK;
     OT_TRY(use_device(device));
     DevBuf<double> dp, dn, op, on;
-    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(op.alloc(n * 3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
+    OT_CUDA(dp.upload(points, n * 3)); OT_CUDA(op.alloc(n * 3));
     const bool has_n = normals && out_normals;
-    if (has_n) { OT_CUDA(dn.alloc(n * 3)); OT_CUDA(on.alloc(n * 3)); OT_CUDA(cudaMemcpy(dn.p, normals, n * 24, cudaMemcpyDefault)); }
+    if (has_n) { OT_CUDA(dn.upload(normals, n * 3)); OT_CUDA(on.alloc(n * 3)); }
     OpTimer timer;
     rigid_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dp.p, has_n ? dn.p : nullptr, n, a, op.p, has_n ? on.p : nullptr);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_points, op.p, n * 24, cudaMemcpyDefault));
-    if (has_n) OT_CUDA(cudaMemcpy(out_normals, on.p, n * 24, cudaMemcpyDefault));
+    OT_CUDA(op.download(out_points, n * 3));
+    if (has_n) OT_CUDA(on.download(out_normals, n * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -519,8 +518,7 @@ int otslam_cloud_center(const double* points, int64_t n, double center[3], int d
     if (n == 0) return OTSLAM_OK;
     OT_TRY(use_device(device));
     DevBuf<double> dp, ax, tot;
-    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(ax.alloc(n)); OT_CUDA(tot.alloc(3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
+    OT_CUDA(dp.upload(points, n * 3)); OT_CUDA(ax.alloc(n)); OT_CUDA(tot.alloc(3));
     OpTimer timer;
     for (int a = 0; a < 3; ++a) {     // coordinates may be negative: the exact chain replays such chunks scalar-wise, still in index order
         axis_extract_kernel<<<(unsigned)((n + 255) / 256), 256>>>(dp.p, n, a, ax.p);
@@ -541,14 +539,13 @@ int otslam_grid_smart_paste(uint8_t* base, const uint8_t* overlay, int width, in
     OT_TRY(use_device(device));
     const size_t n = (size_t)width * height;
     DevBuf<uint8_t> db, dov;
-    OT_CUDA(db.alloc(n)); OT_CUDA(dov.alloc(n));
-    OT_CUDA(cudaMemcpy(db.p, base, n, cudaMemcpyDefault));
-    OT_CUDA(cudaMemcpy(dov.p, overlay, n, cudaMemcpyDefault));
+    OT_CUDA(db.upload(base, n)); OT_CUDA(dov.upload(overlay, n));
     OpTimer timer;
     smart_paste_kernel<<<(unsigned)(((int64_t)w * h + 255) / 256), 256>>>(db.p, dov.p, width, x, y, w, h, unknown_pixel, threshold);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(base, db.p, n, cudaMemcpyDefault));
+    OT_CUDA(db.download(base, n));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 

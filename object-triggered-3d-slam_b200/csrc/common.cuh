@@ -175,15 +175,17 @@ __host__ __device__ inline bool slab_keeps(const SlabSpec& s, int kx, int ky, in
 // Scratch cache for the operators' temporaries and results: cudaMalloc / cudaFree cost 0.1-0.5 ms each
 // (and cudaFree synchronises the device), which dominated the post-stage operators (a dozen buffers
 // per call, kernels of a few hundred microseconds).  Freed blocks go to a per-device free list and
-// are handed out again to requests of similar size.  Every operator synchronises before it returns,
-// so a released block is idle -- except on an error return, which is why a release that follows an
-// error (the thread's error count moved since the allocation) drains the device first.
+// are handed out again to requests of similar size.  Every operator synchronises before it returns
+// (and the volume synchronises its stream before it replaces a result), so a released block is idle
+// -- except on an error return, which is why a release that follows an error (the thread's error
+// count moved since the allocation) drains the device first.
 // otslam_trim_scratch() releases the cache.
 extern thread_local uint64_t g_error_count;
 cudaError_t scratch_alloc(void** p, size_t bytes);
 void scratch_free(void* p);
 
-// RAII device buffer for the operators
+// RAII device buffer from the scratch cache: the operators' temporaries and results, and the volume's mesh, points,
+// sorted block list and halo pieces
 template <typename T>
 struct DevBuf {
     T* p = nullptr;
@@ -193,12 +195,17 @@ struct DevBuf {
     DevBuf(const DevBuf&) = delete;
     DevBuf& operator=(const DevBuf&) = delete;
     DevBuf(DevBuf&& o) noexcept : p(o.p), n(o.n), err_epoch(o.err_epoch) { o.p = nullptr; o.n = 0; }
+    DevBuf& operator=(DevBuf&& o) noexcept {
+        if (this != &o) { release(); std::swap(p, o.p); std::swap(n, o.n); std::swap(err_epoch, o.err_epoch); }
+        return *this;
+    }
     ~DevBuf() { release(); }
     void release() {
         if (!p) return;
         if (err_epoch != g_error_count) cudaDeviceSynchronize();
         scratch_free(p);
         p = nullptr;
+        n = 0;
     }
     cudaError_t alloc(size_t count) {
         release();
@@ -206,6 +213,13 @@ struct DevBuf {
         err_epoch = g_error_count;
         return scratch_alloc((void**)&p, (count ? count : 1) * sizeof(T));
     }
+    // alloc(count), then count elements from src; src and dst may be host or device pointers (unified addressing).  A
+    // device-to-device cudaMemcpy may return before it completes: an operator synchronises before it returns.
+    cudaError_t upload(const T* src, size_t count) {
+        const cudaError_t e = alloc(count);
+        return e != cudaSuccess ? e : cudaMemcpy(p, src, count * sizeof(T), cudaMemcpyDefault);
+    }
+    cudaError_t download(T* dst, size_t count) const { return cudaMemcpy(dst, p, count * sizeof(T), cudaMemcpyDefault); }
 };
 
 // ---- owning handles for the long-lived resources (the volume, the decoder, checkpoint staging): move-only, released by

@@ -516,7 +516,7 @@ int otslam_volume_extract_mesh(otslam_volume* v, int64_t* n_vertices, int64_t* n
     if (!v || !n_vertices || !n_faces) return set_error(OTSLAM_ERR_INVALID, "null argument");
     OT_TRY(use_device(v->device));
     OT_TRY(upload_tables());
-    v->mesh.release();
+    v->mesh = {};
     *n_vertices = 0; *n_faces = 0;
     OpTimer timer(v->stream);
     ExtractCtx c;
@@ -549,23 +549,21 @@ int otslam_volume_extract_mesh(otslam_volume* v, int64_t* n_vertices, int64_t* n
     OT_CUDA(cudaMemcpyAsync(&nf, fbase.p + n, 8, cudaMemcpyDeviceToHost, s));
     OT_CUDA(cudaStreamSynchronize(s));
     if (nv > 0x7fffffffLL || nf > 0x7fffffffLL) return set_error(OTSLAM_ERR_OVERFLOW, "mesh exceeds int32 indices");
-    MeshResult& m = v->mesh;
+    MeshResult m;
     m.nv = nv; m.nf = nf;
     if (nv > 0) {
-        OT_CUDA(scratch_alloc((void**)&m.d_verts, (size_t)nv * 24));
-        OT_CUDA(scratch_alloc((void**)&m.d_colors, (size_t)nv * 24));
-        OT_CUDA(scratch_alloc((void**)&m.d_normals, (size_t)nv * 24));
-        OT_CUDA(scratch_alloc((void**)&m.d_ekeys, (size_t)nv * 16));
-        OT_CUDA(scratch_alloc((void**)&m.d_faces, (size_t)std::max<int64_t>(nf, 1) * 12));
-        mc_vertices_kernel<<<n, 128, 0, s>>>(c, flags.p, wprefix.p, vbase.p, m.d_verts, m.d_colors, m.d_ekeys);
+        OT_CUDA(m.verts.alloc(nv * 3)); OT_CUDA(m.colors.alloc(nv * 3)); OT_CUDA(m.normals.alloc(nv * 3));
+        OT_CUDA(m.ekeys.alloc(nv * 4)); OT_CUDA(m.faces.alloc(nf * 3));
+        mc_vertices_kernel<<<n, 128, 0, s>>>(c, flags.p, wprefix.p, vbase.p, m.verts.p, m.colors.p, m.ekeys.p);
         OT_LAUNCHED();
         if (nf > 0) {
-            mc_faces_kernel<<<n, 256, 0, s>>>(c, flags.p, wprefix.p, vbase_slot.p, cube.p, fbase.p, m.d_faces);
+            mc_faces_kernel<<<n, 256, 0, s>>>(c, flags.p, wprefix.p, vbase_slot.p, cube.p, fbase.p, m.faces.p);
             OT_LAUNCHED();
         }
-        OT_TRY(device_vertex_normals(m.d_verts, nv, m.d_faces, nf, m.d_normals, s));
+        OT_TRY(device_vertex_normals(m.verts.p, nv, m.faces.p, nf, m.normals.p, s));
     }
     OT_CUDA(cudaStreamSynchronize(s));
+    v->mesh = std::move(m);
     *n_vertices = nv; *n_faces = nf;
     return OTSLAM_OK;
 }
@@ -576,12 +574,12 @@ int otslam_volume_mesh_copy(otslam_volume* v, double* vertices, double* colors, 
     OT_TRY(use_device(v->device));
     const MeshResult& m = v->mesh;
     if (m.nv > 0) {
-        if (vertices) OT_CUDA(cudaMemcpyAsync(vertices, m.d_verts, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
-        if (colors) OT_CUDA(cudaMemcpyAsync(colors, m.d_colors, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
-        if (normals) OT_CUDA(cudaMemcpyAsync(normals, m.d_normals, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
-        if (edge_keys) OT_CUDA(cudaMemcpyAsync(edge_keys, m.d_ekeys, (size_t)m.nv * 16, cudaMemcpyDefault, v->stream));
+        if (vertices) OT_CUDA(cudaMemcpyAsync(vertices, m.verts.p, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
+        if (colors) OT_CUDA(cudaMemcpyAsync(colors, m.colors.p, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
+        if (normals) OT_CUDA(cudaMemcpyAsync(normals, m.normals.p, (size_t)m.nv * 24, cudaMemcpyDefault, v->stream));
+        if (edge_keys) OT_CUDA(cudaMemcpyAsync(edge_keys, m.ekeys.p, (size_t)m.nv * 16, cudaMemcpyDefault, v->stream));
     }
-    if (m.nf > 0 && faces) OT_CUDA(cudaMemcpyAsync(faces, m.d_faces, (size_t)m.nf * 12, cudaMemcpyDefault, v->stream));
+    if (m.nf > 0 && faces) OT_CUDA(cudaMemcpyAsync(faces, m.faces.p, (size_t)m.nf * 12, cudaMemcpyDefault, v->stream));
     OT_CUDA(cudaStreamSynchronize(v->stream));     // destinations may be host or device pointers (unified addressing)
     return OTSLAM_OK;
 }
@@ -589,7 +587,7 @@ int otslam_volume_mesh_copy(otslam_volume* v, double* vertices, double* colors, 
 int otslam_volume_extract_points(otslam_volume* v, int64_t* n_points) {
     if (!v || !n_points) return set_error(OTSLAM_ERR_INVALID, "null argument");
     OT_TRY(use_device(v->device));
-    v->points.release();
+    v->points = {};
     *n_points = 0;
     OpTimer timer(v->stream);
     ExtractCtx c;
@@ -606,16 +604,15 @@ int otslam_volume_extract_points(otslam_volume* v, int64_t* n_points) {
     int64_t np = 0;
     OT_CUDA(cudaMemcpyAsync(&np, pbase.p + n, 8, cudaMemcpyDeviceToHost, s));
     OT_CUDA(cudaStreamSynchronize(s));
-    PointsResult& p = v->points;
+    PointsResult p;
     p.n = np;
     if (np > 0) {
-        OT_CUDA(scratch_alloc((void**)&p.d_pts, (size_t)np * 24));
-        OT_CUDA(scratch_alloc((void**)&p.d_cols, (size_t)np * 24));
-        OT_CUDA(scratch_alloc((void**)&p.d_ekeys, (size_t)np * 16));
-        pc_extract_kernel<<<n, 256, 0, s>>>(c, pbase.p, nullptr, p.d_pts, p.d_cols, p.d_ekeys);
+        OT_CUDA(p.pts.alloc(np * 3)); OT_CUDA(p.cols.alloc(np * 3)); OT_CUDA(p.ekeys.alloc(np * 4));
+        pc_extract_kernel<<<n, 256, 0, s>>>(c, pbase.p, nullptr, p.pts.p, p.cols.p, p.ekeys.p);
         OT_LAUNCHED();
         OT_CUDA(cudaStreamSynchronize(s));
     }
+    v->points = std::move(p);
     *n_points = np;
     return OTSLAM_OK;
 }
@@ -629,7 +626,7 @@ int otslam_volume_points_normals(otslam_volume* v, double* normals) {
     OT_TRY(make_ctx(v, c));
     DevBuf<double> dn;
     OT_CUDA(dn.alloc((size_t)p.n * 3));
-    pc_normals_kernel<<<(unsigned)((p.n + 127) / 128), 128, 0, v->stream>>>(c, p.d_pts, p.n, 0.99 * v->voxel_length, dn.p);
+    pc_normals_kernel<<<(unsigned)((p.n + 127) / 128), 128, 0, v->stream>>>(c, p.pts.p, p.n, 0.99 * v->voxel_length, dn.p);
     OT_LAUNCHED();
     OT_CUDA(cudaMemcpyAsync(normals, dn.p, (size_t)p.n * 24, cudaMemcpyDefault, v->stream));
     OT_CUDA(cudaStreamSynchronize(v->stream));
@@ -641,9 +638,9 @@ int otslam_volume_points_copy(otslam_volume* v, double* points, double* colors, 
     OT_TRY(use_device(v->device));
     const PointsResult& p = v->points;
     if (p.n > 0) {
-        if (points) OT_CUDA(cudaMemcpyAsync(points, p.d_pts, (size_t)p.n * 24, cudaMemcpyDefault, v->stream));
-        if (colors) OT_CUDA(cudaMemcpyAsync(colors, p.d_cols, (size_t)p.n * 24, cudaMemcpyDefault, v->stream));
-        if (edge_keys) OT_CUDA(cudaMemcpyAsync(edge_keys, p.d_ekeys, (size_t)p.n * 16, cudaMemcpyDefault, v->stream));
+        if (points) OT_CUDA(cudaMemcpyAsync(points, p.pts.p, (size_t)p.n * 24, cudaMemcpyDefault, v->stream));
+        if (colors) OT_CUDA(cudaMemcpyAsync(colors, p.cols.p, (size_t)p.n * 24, cudaMemcpyDefault, v->stream));
+        if (edge_keys) OT_CUDA(cudaMemcpyAsync(edge_keys, p.ekeys.p, (size_t)p.n * 16, cudaMemcpyDefault, v->stream));
         OT_CUDA(cudaStreamSynchronize(v->stream));
     }
     return OTSLAM_OK;

@@ -787,9 +787,8 @@ int otslam_cloud_voxel_down_sample(const double* points, const double* colors, i
     if (n > 0x7fffffffLL) return set_error(OTSLAM_ERR_OVERFLOW, "more than 2^31 points");
     OT_TRY(use_device(device));
     DevBuf<double> dp, dc;
-    OT_CUDA(dp.alloc(n * 3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
-    if (colors) { OT_CUDA(dc.alloc(n * 3)); OT_CUDA(cudaMemcpy(dc.p, colors, n * 24, cudaMemcpyDefault)); }
+    OT_CUDA(dp.upload(points, n * 3));
+    if (colors) OT_CUDA(dc.upload(colors, n * 3));
     OpTimer timer;
     double mn[3], mx[3];
     OT_TRY(cloud_minmax(dp.p, n, mn, mx));
@@ -819,10 +818,11 @@ int otslam_cloud_voxel_down_sample(const double* points, const double* colors, i
     voxel_mean_kernel<<<(unsigned)((m + 127) / 128), 128>>>(dp.p, colors ? dc.p : nullptr, k1.p, i1.p, seg.p, m, L, op.p, oc.p, ok.p, on.p);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_points, op.p, m * 24, cudaMemcpyDefault));
-    if (colors && out_colors) OT_CUDA(cudaMemcpy(out_colors, oc.p, m * 24, cudaMemcpyDefault));
-    if (out_keys) OT_CUDA(cudaMemcpy(out_keys, ok.p, m * 12, cudaMemcpyDefault));
-    if (out_counts) OT_CUDA(cudaMemcpy(out_counts, on.p, m * 4, cudaMemcpyDefault));
+    OT_CUDA(op.download(out_points, m * 3));
+    if (colors && out_colors) OT_CUDA(oc.download(out_colors, m * 3));
+    if (out_keys) OT_CUDA(ok.download(out_keys, m * 3));
+    if (out_counts) OT_CUDA(on.download(out_counts, m));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -839,8 +839,7 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
     if (k > kKnnMaxK) return set_error(OTSLAM_ERR_INVALID, "nb_neighbors > 128 is not supported on the GPU path");
     OT_TRY(use_device(device));
     DevBuf<double> dp;
-    OT_CUDA(dp.alloc(n * 3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
+    OT_CUDA(dp.upload(points, n * 3));
     OpTimer timer;
     KnnArgs a;
     GridBuffers bc, bf, bt;
@@ -851,7 +850,7 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
     a.nq = n; a.mode = 0; a.n = n; a.k = k; a.dbar = dbar.p;
     knn_mean_dist_kernel<<<(unsigned)((n + kKnnWarps - 1) / kKnnWarps), kKnnWarps * 32>>>(a);
     OT_LAUNCHED();
-    if (mean_dist) OT_CUDA(cudaMemcpy(mean_dist, dbar.p, n * 8, cudaMemcpyDefault));
+    if (mean_dist) OT_CUDA(dbar.download(mean_dist, n));
     // global statistics in sequential index order; scalars finished on the host in FP64
     double sum = 0.0, sq = 0.0;
     OT_TRY(device_ordered_sum(dbar.p, n, 2, nullptr, 0.0, scal.p, 0));
@@ -866,9 +865,9 @@ int otslam_cloud_remove_statistical_outlier(const double* points, int64_t n, int
     int64_t m = 0;
     OT_TRY(select_indices(SorKeep{dbar.p, thr}, n, 0, oidx, &m));
     *n_out = m;
-    if (m == 0) return OTSLAM_OK;
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_indices, oidx.p, m * 8, cudaMemcpyDefault));
+    if (m > 0) OT_CUDA(oidx.download(out_indices, m));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -930,13 +929,11 @@ int otslam_cloud_nn_within(const double* source, int64_t n_source, const double*
     OT_TRY(use_device(device));
     DevBuf<double> dt, dsrc, dd2;
     DevBuf<int32_t> di;
-    OT_CUDA(dsrc.alloc(n_source * 3)); OT_CUDA(di.alloc(n_source)); OT_CUDA(dd2.alloc(n_source));
-    OT_CUDA(cudaMemcpy(dsrc.p, source, n_source * 24, cudaMemcpyDefault));
+    OT_CUDA(dsrc.upload(source, n_source * 3)); OT_CUDA(di.alloc(n_source)); OT_CUDA(dd2.alloc(n_source));
     if (n_target == 0) {
         OT_CUDA(cudaMemset(di.p, 0xFF, (size_t)n_source * 4));
     } else {
-        OT_CUDA(dt.alloc(n_target * 3));
-        OT_CUDA(cudaMemcpy(dt.p, target, n_target * 24, cudaMemcpyDefault));
+        OT_CUDA(dt.upload(target, n_target * 3));
         OpTimer timer;
         double mn[3], mx[3];
         OT_TRY(cloud_minmax(dt.p, n_target, mn, mx));
@@ -947,10 +944,9 @@ int otslam_cloud_nn_within(const double* source, int64_t n_source, const double*
         nn_within_kernel<<<(unsigned)((n_source + 127) / 128), 128>>>(g, dt.p, dsrc.p, n_source, radius * radius, di.p, dd2.p);
         OT_LAUNCHED();
         timer.stop();
-        OT_CUDA(cudaDeviceSynchronize());
     }
-    OT_CUDA(cudaMemcpy(out_index, di.p, n_source * 4, cudaMemcpyDefault));
-    if (out_dist2 && n_target) OT_CUDA(cudaMemcpy(out_dist2, dd2.p, n_source * 8, cudaMemcpyDefault));
+    OT_CUDA(di.download(out_index, n_source));
+    if (out_dist2 && n_target) OT_CUDA(dd2.download(out_dist2, n_source));
     OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
@@ -964,9 +960,7 @@ int otslam_cloud_nn_distance(const double* source, int64_t n_source, const doubl
     if (n_target > 0x7fffffffLL || n_source > 0x7fffffffLL) return set_error(OTSLAM_ERR_OVERFLOW, "more than 2^31 points");
     OT_TRY(use_device(device));
     DevBuf<double> dt, dsrc, dout;
-    OT_CUDA(dt.alloc(n_target * 3)); OT_CUDA(dsrc.alloc(n_source * 3)); OT_CUDA(dout.alloc(n_source));
-    OT_CUDA(cudaMemcpy(dt.p, target, n_target * 24, cudaMemcpyDefault));
-    OT_CUDA(cudaMemcpy(dsrc.p, source, n_source * 24, cudaMemcpyDefault));
+    OT_CUDA(dt.upload(target, n_target * 3)); OT_CUDA(dsrc.upload(source, n_source * 3)); OT_CUDA(dout.alloc(n_source));
     OpTimer timer;
     KnnArgs a;
     GridBuffers bc, bf, bt;
@@ -975,7 +969,8 @@ int otslam_cloud_nn_distance(const double* source, int64_t n_source, const doubl
     knn_mean_dist_kernel<<<(unsigned)((n_source + kKnnWarps - 1) / kKnnWarps), kKnnWarps * 32>>>(a);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_dist, dout.p, n_source * 8, cudaMemcpyDefault));
+    OT_CUDA(dout.download(out_dist, n_source));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -990,9 +985,8 @@ int otslam_cloud_estimate_normals(const double* points, int64_t n, const double*
     if (n == 0) return OTSLAM_OK;
     OT_TRY(use_device(device));
     DevBuf<double> dp, dprior, dout;
-    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(dout.alloc(n * 3));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
-    if (prior_normals) { OT_CUDA(dprior.alloc(n * 3)); OT_CUDA(cudaMemcpy(dprior.p, prior_normals, n * 24, cudaMemcpyDefault)); }
+    OT_CUDA(dp.upload(points, n * 3)); OT_CUDA(dout.alloc(n * 3));
+    if (prior_normals) OT_CUDA(dprior.upload(prior_normals, n * 3));
     OpTimer timer;
     KnnArgs a;
     GridBuffers bc, bf, bt;
@@ -1003,7 +997,8 @@ int otslam_cloud_estimate_normals(const double* points, int64_t n, const double*
                                                                                     radius * radius, dout.p);
     OT_LAUNCHED();
     timer.stop();
-    OT_CUDA(cudaMemcpy(out_normals, dout.p, n * 24, cudaMemcpyDefault));
+    OT_CUDA(dout.download(out_normals, n * 3));
+    OT_CUDA(cudaDeviceSynchronize());
     return OTSLAM_OK;
 }
 
@@ -1040,14 +1035,9 @@ int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, cons
     const int P = pow2_at_least(n_cta);
     DevBuf<double> ds0, ds1, dt, dtn, dpart, dsum;
     DevBuf<int32_t> dcorr;
-    OT_CUDA(ds0.alloc(n * 3)); OT_CUDA(ds1.alloc(n * 3)); OT_CUDA(dcorr.alloc(n));
+    OT_CUDA(ds0.upload(source, n * 3)); OT_CUDA(ds1.alloc(n * 3)); OT_CUDA(dcorr.alloc(n));
     OT_CUDA(dpart.alloc((size_t)kIcpTerms * P)); OT_CUDA(dsum.alloc(kIcpTerms));
-    OT_CUDA(cudaMemcpy(ds0.p, source, n * 24, cudaMemcpyDefault));
-    if (n_target) {
-        OT_CUDA(dt.alloc(n_target * 3)); OT_CUDA(dtn.alloc(n_target * 3));
-        OT_CUDA(cudaMemcpy(dt.p, target, n_target * 24, cudaMemcpyDefault));
-        OT_CUDA(cudaMemcpy(dtn.p, target_normals, n_target * 24, cudaMemcpyDefault));
-    }
+    if (n_target) { OT_CUDA(dt.upload(target, n_target * 3)); OT_CUDA(dtn.upload(target_normals, n_target * 3)); }
     OpTimer timer;
     // the target's grid once per call, cell = max_distance (otslam_cloud_nn_within's)
     KnnGrid g = {};
@@ -1089,7 +1079,7 @@ int otslam_cloud_icp_point_to_plane(const double* source, int64_t n_source, cons
         if (std::fabs(fit0 - fit) < relative_fitness && std::fabs(rmse0 - rmse) < relative_rmse) break;
     }
     timer.stop();
-    if (corr_index) OT_CUDA(cudaMemcpy(corr_index, dcorr.p, n * 4, cudaMemcpyDefault));
+    if (corr_index) { OT_CUDA(dcorr.download(corr_index, n)); OT_CUDA(cudaDeviceSynchronize()); }
     for (int k = 0; k < 16; ++k) transform_out[k] = T[k];
     if (fitness) *fitness = fit;
     if (inlier_rmse) *inlier_rmse = rmse;

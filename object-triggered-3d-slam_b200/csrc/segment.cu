@@ -342,9 +342,8 @@ int otslam_cloud_cluster_dbscan(const double* points, int64_t n, double eps, int
     DevBuf<int> core, parent, root, flag;
     DevBuf<int64_t> rank;
     DevBuf<int32_t> dl;
-    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(core.alloc(n)); OT_CUDA(parent.alloc(n)); OT_CUDA(root.alloc(n)); OT_CUDA(flag.alloc(n));
+    OT_CUDA(dp.upload(points, n * 3)); OT_CUDA(core.alloc(n)); OT_CUDA(parent.alloc(n)); OT_CUDA(root.alloc(n)); OT_CUDA(flag.alloc(n));
     OT_CUDA(rank.alloc(n + 1)); OT_CUDA(dl.alloc(n));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
     OpTimer timer;
     double mn[3], mx[3];
     OT_TRY(cloud_minmax(dp.p, n, mn, mx));
@@ -367,7 +366,7 @@ int otslam_cloud_cluster_dbscan(const double* points, int64_t n, double eps, int
     timer.stop();
     int64_t total = 0;
     OT_CUDA(cudaMemcpy(&total, rank.p + n, 8, cudaMemcpyDeviceToHost));
-    OT_CUDA(cudaMemcpy(out_labels, dl.p, n * 4, cudaMemcpyDefault));
+    OT_CUDA(dl.download(out_labels, n));
     OT_CUDA(cudaDeviceSynchronize());
     if (n_clusters) *n_clusters = (int32_t)total;
     return OTSLAM_OK;
@@ -394,9 +393,8 @@ int otslam_cloud_segment_plane(const double* points, int64_t n, double distance_
     const int n_cta = (int)((n + kSegTile - 1) / kSegTile), P = pow2_at_least(n_cta);
     DevBuf<double> dp, part, res;
     DevBuf<double4> planes, best_plane;
-    OT_CUDA(dp.alloc(n * 3)); OT_CUDA(part.alloc((size_t)2 * kWave * P)); OT_CUDA(res.alloc(2 * kWave));
+    OT_CUDA(dp.upload(points, n * 3)); OT_CUDA(part.alloc((size_t)2 * kWave * P)); OT_CUDA(res.alloc(2 * kWave));
     OT_CUDA(planes.alloc(kWave)); OT_CUDA(best_plane.alloc(1));
-    OT_CUDA(cudaMemcpy(dp.p, points, n * 24, cudaMemcpyDefault));
     OpTimer timer;
     // Open3D's selection in hypothesis order: skip h > B; replace on a greater fitness, or an equal one with a smaller rmse
     int64_t B = INT64_MAX;
@@ -446,7 +444,7 @@ int otslam_cloud_segment_plane(const double* points, int64_t n, double distance_
     OT_TRY(refit_sums(dp.p, oidx.p, m, 1, cen, mom));
     timer.stop();
     plane_from_moments(cen, mom, plane_out);
-    OT_CUDA(cudaMemcpy(out_inliers, oidx.p, m * 8, cudaMemcpyDefault));
+    OT_CUDA(oidx.download(out_inliers, m));
     OT_CUDA(cudaDeviceSynchronize());
     *n_inliers = m;
     return OTSLAM_OK;

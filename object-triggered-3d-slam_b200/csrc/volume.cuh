@@ -26,21 +26,28 @@ constexpr int kNB = 3;          // batch buffers: allocation runs up to two batc
 enum CounterIdx { kPoolCount = 0, kListCount = 2, kFlags = 5, kNumCounters = 8 };
 enum Flags { kFlagHashFull = 1, kFlagKeyRange = 2, kFlagBoxTooLarge = 4 };
 
+// extraction results (extract.cu): built in a local and moved into the volume only after the stream has synchronised, so
+// a failed extraction leaves an empty result
 struct MeshResult {
     int64_t nv = 0, nf = 0;
-    double* d_verts = nullptr;    // [nv][3]
-    double* d_colors = nullptr;   // [nv][3]
-    double* d_normals = nullptr;  // [nv][3]
-    int32_t* d_faces = nullptr;   // [nf][3]
-    int32_t* d_ekeys = nullptr;   // [nv][4]
-    void release();
+    DevBuf<double> verts;     // [nv][3]
+    DevBuf<double> colors;    // [nv][3]
+    DevBuf<double> normals;   // [nv][3]
+    DevBuf<int32_t> faces;    // [nf][3]
+    DevBuf<int32_t> ekeys;    // [nv][4]
 };
 struct PointsResult {
     int64_t n = 0;
-    double* d_pts = nullptr;
-    double* d_cols = nullptr;
-    int32_t* d_ekeys = nullptr;
-    void release();
+    DevBuf<double> pts;       // [n][3]
+    DevBuf<double> cols;      // [n][3]
+    DevBuf<int32_t> ekeys;    // [n][4]
+};
+// halo pieces packed by otslam_volume_halo_pack: grouped by destination rank, (key, kind) order inside a group
+struct HaloPieces {
+    int64_t n = 0;
+    DevBuf<int32_t> keys;     // [n][4]
+    DevBuf<uint4> planes;     // [n][256]
+    std::vector<int64_t> counts;   // pieces per destination rank
 };
 
 // block hash (hash_table.cuh): the entry index is the handle used by the per-batch work list.  Built whole or not at all
@@ -114,19 +121,15 @@ struct otslam_volume {
     // device-resident list of the allocated blocks sorted by key (extraction order, export, halo selection); rebuilt
     // when `epoch` (bumped by integrate / reset / halo import) has moved past `sorted_epoch`
     uint64_t epoch = 1, sorted_epoch = 0;
-    uint64_t* d_sorted_keys = nullptr;
-    int32_t* d_sorted_slots = nullptr;
+    otslam::DevBuf<uint64_t> sorted_keys;
+    otslam::DevBuf<int32_t> sorted_slots;
     int64_t n_sorted = 0;
 
-    // halo pieces packed by otslam_volume_halo_pack: grouped by destination rank, (key, kind) order inside a group
-    int32_t* d_halo_keys = nullptr;      // [n_halo][4]
-    uint4* d_halo_planes = nullptr;      // [n_halo][256]
-    int64_t n_halo = 0;
-    std::vector<int64_t> halo_counts;    // pieces per destination rank
+    otslam::HaloPieces halo;
 
     otslam::Event ev_ext;                // otslam_volume_wait_stream
 
-    ~otslam_volume();                    // drains the streams, releases the scratch-cache results
+    ~otslam_volume();                    // drains the streams before the members release their memory
 };
 
 namespace otslam {

@@ -107,3 +107,53 @@ def test_profiling(frames):
     ref.integrate_batch(d[2:], c[2:], seq.fxfycxcy, seq.extrinsic[2:])
     assert got == state(ref)
     ref.close()
+
+
+def test_failed_extraction_leaves_no_result(frames):
+    """An extraction releases the old mesh / points first and keeps a new one only when it completes.  On an arena with no
+    object selected it fails after that release: sampling then finds no triangles, the copies copy nothing, and the next
+    good extraction gives what a fresh arena gives."""
+    from otslam_b200 import _lib
+    from otslam_b200.volume import TSDFVolume
+    seq = frames["large"]
+    d, c = seq.numpy()
+
+    def arena():
+        a = TSDFVolume(VL, 4 * VL)
+        a.set_objects(2)
+        a.integrate_batch(d, c, seq.fxfycxcy, seq.extrinsic, object_ids=np.ones(len(seq), np.int32))
+        a.select_object(1)
+        return a
+
+    def results(a):
+        mesh = a.extract_triangle_mesh()
+        sample = a.mesh_sample(4096, 11, colors=True, normals=True)
+        return [x.tobytes() for x in mesh + sample + a.extract_point_cloud(normals=True)]
+
+    v = arena()
+    nv, nf = v.extract_mesh_resident()
+    n_pts = len(v.extract_point_cloud()[0])
+    assert nv > 0 and nf > 0 and n_pts > 0
+    v.select_object(-1)
+    with pytest.raises(RuntimeError, match="select_object"):
+        v.extract_mesh_resident()
+    with pytest.raises(RuntimeError, match="select_object"):
+        v.extract_point_cloud()
+    with pytest.raises(RuntimeError, match="no triangles"):
+        v.mesh_sample(4096, 11)
+    mesh = [np.full((nv, 3), 7.0), np.full((nv, 3), 7.0), np.full((nv, 3), 7.0), np.full((nf, 3), 7, np.int32),
+            np.full((nv, 4), 7, np.int32)]
+    points = [np.full((n_pts, 3), 7.0), np.full((n_pts, 3), 7.0), np.full((n_pts, 4), 7, np.int32)]
+    normals = np.full((n_pts, 3), 7.0)
+    _lib.check(_lib.lib.otslam_volume_mesh_copy(v._h, *(_lib.ptr(a) for a in mesh)))
+    _lib.check(_lib.lib.otslam_volume_points_copy(v._h, *(_lib.ptr(a) for a in points)))
+    _lib.check(_lib.lib.otslam_volume_points_normals(v._h, _lib.ptr(normals)))
+    for a in mesh + points + [normals]:
+        assert (a == 7).all()
+    v.select_object(1)
+    got = results(v)
+    v.close()
+    ref = arena()
+    want = results(ref)
+    ref.close()
+    assert got == want
